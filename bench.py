@@ -2,6 +2,7 @@
 """bench.py — throughput of the vox_box hot path on B200 (BASELINE.json metric: "LPC+formant and pitch frames/sec").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config all|c1|c2|c3|c4|c5] [--utts U]
+                    [--dump-outputs DIR]
 
 The headline record (the keys at the top level of the ONE JSON line rank 0 prints) is C3 = BASELINE.json configs[2], the
 config the metric is quoted on: LPC-12 + formant extraction (Hann -> autocorrelate(13) -> Levinson -> Laguerre roots ->
@@ -25,6 +26,11 @@ kernels), `roofline_hbm` against MEASURED_PEAKS.json's copy bandwidth; `cpu_base
 Rust reference — no Rust toolchain in this image) on this box's host cores, single-threaded as shipped and on all threads.
 `--impl reference` times that CPU port alone on the same configs.  Audio is synthesised on the device (vbx_synth_speech:
 every utterance distinct); the CPU legs of the GPU arm read those very samples back.
+
+--steps K sets the timed steps behind `value` / `ms_per_step` of every config (and C1's repetitions); the sustained leg runs
+the same loop for >= 2 s and the end-to-end legs their own small count, each reported next to its value.  The seeded synthesis
+gives every run with the same arguments the same inputs, so --dump-outputs DIR (what the last timed step computed, see
+dump_outputs) lets two builds be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -381,8 +387,7 @@ def host_corpus(cfg, n_utts, first=0):
 def c1_record(args, reps=None):
     """BASELINE configs[0]: examples/pitch_detection.rs as shipped, timed on the CPU oracle (one thread, as shipped)."""
     import oracle
-    oracle.build()
-    reps = reps or max(3, min(args.steps if args.steps is not None else 20, 20))   # no --steps: 20 repetitions
+    reps = reps or (args.steps if args.steps is not None else 20)
     out = {"metric": C1["metric"], "unit": "frames/s", "higher_is_better": True, "dtype": "f64", "data": "synthetic sine + tests/fixtures/short_sample.wav",
            "config": {"workload": C1["workload"]}, "impl_note": "CPU oracle (C++ f64 port of the Rust reference), 1 thread, as shipped"}
     cases = {}
@@ -457,8 +462,6 @@ def reference_record(args, key, cfg, world):
 def run_reference(args, keys, rank, world):
     if rank != 0:
         return
-    import oracle
-    oracle.build()
     head = keys[0]
     line = reference_record(args, head, CONFIGS[head], world)
     subs = {}
@@ -476,8 +479,6 @@ def run_reference(args, keys, rank, world):
 def cpu_baseline(cfg, rows, J):
     """Bounded CPU sample on rank 0 (N=1 only): oracle port, single thread as shipped + all threads, on the very samples the
     GPU processed (copied device -> host)."""
-    import oracle
-    oracle.build()
     threads = host_threads()
     n_all = min(cpu_sample_utts(cfg, J, threads, 0.6), len(rows))
     n_one = max(1, min(n_all, cpu_sample_utts(cfg, J, 1, 1.0)))
@@ -571,6 +572,7 @@ class Workload:
             p = cfg["p"]
             d_r, d_ac = ctx.empty((F, p + 1), np.float32), ctx.empty((F, p + 1), np.float32)
             self.step = lambda: ctx._check(L.vbx_lpc(h, C.byref(fr), p, d_r.ptr, d_ac.ptr, None, vb.F32), "vbx_lpc")
+            self.outputs = lambda: {"r": d_r.to_host(), "lpc": d_ac.to_host()}
             self._keep = (d_r, d_ac)
             if want_host:
                 h_r, h_ac = pinned((F, p + 1), np.float32), pinned((F, p + 1), np.float32)
@@ -592,6 +594,7 @@ class Workload:
                                                vb.F32), "vbx_find_formants")
 
             self.step = step
+            self.outputs = lambda: {"tracks": d_trk.to_host(), "estimates": d_est.to_host()}
             self._keep = (d_est0, d_est, d_trk, est0)
             if want_host:
                 h_trk, h_est = pinned((F, 8), np.float32), pinned((U, 8), np.float32)
@@ -611,6 +614,7 @@ class Workload:
             K = 16
             d_c, d_n, d_s = ctx.empty((F, K, 2), np.float32), ctx.empty((F,), np.int32), ctx.empty((F,), np.uint8)
             self.step = lambda: ctx._check(L.vbx_pitch(h, C.byref(fr), fsd, 0.45, 75.0, 600.0, K, d_c.ptr, d_n.ptr, d_s.ptr, vb.F32), "vbx_pitch")
+            self.outputs = lambda: {"candidates": d_c.to_host(), "n_cand": d_n.to_host(), "status": d_s.to_host()}
             self._keep = (d_c, d_n, d_s)
             if want_host:
                 h_c, h_n, h_s = pinned((F, K * 2), np.float32), pinned((F,), np.int32), pinned((F,), np.uint8)
@@ -621,6 +625,7 @@ class Workload:
         elif kind == "mfcc":
             d_o = ctx.empty((F, 13), np.float32)
             self.step = lambda: ctx._check(L.vbx_mfcc(h, C.byref(fr), 40, 13, 133.0, 6855.0, fsd, d_o.ptr, None, vb.F32), "vbx_mfcc")
+            self.outputs = lambda: {"mfcc": d_o.to_host()}
             self._keep = (d_o,)
             if want_host:
                 h_o = pinned((F, 13), np.float32)
@@ -630,7 +635,7 @@ class Workload:
                 self.check = lambda: float(np.sum(h_o.a[::max(1, F // 1000), 0], dtype=np.float64))
 
     def free(self):
-        self.step = self.e2e_step = self.check = None
+        self.step = self.e2e_step = self.check = self.outputs = None
         for b in self._pinned:
             b.free()
         for d in (self.d_audio,) + tuple(x for x in self._keep if hasattr(x, "free")):
@@ -722,13 +727,27 @@ class Workload:
         return roof, roof_hbm, kernels
 
 
+DUMP_ROWS = 1 << 16  # rows kept per array by --dump-outputs: every config together stays below 64 MB
+
+
+def dump_outputs(out_dir, key, arrays):
+    """--dump-outputs: writes each output of the last timed step as out_dir/<config>_<name>.npy in float32 (float64 stays
+    float64).  An array with more than DUMP_ROWS rows (frames or utterances) keeps a fixed, seeded sample of its rows in
+    ascending order, and out_dir/<config>_<name>_rows.npy lists their indices, so that runs of two builds on the same
+    arguments compare output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if a.shape[0] > DUMP_ROWS:
+            rows = np.sort(np.random.default_rng(SEED).choice(a.shape[0], DUMP_ROWS, replace=False))
+            a = a[rows]
+            np.save(os.path.join(out_dir, f"{key}_{name}_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(out_dir, f"{key}_{name}.npy"), a if a.dtype == np.float64 else a.astype(np.float32))
+
+
 def gpu_record(ctx, vb, key, cfg, args, comm, clocks, peaks):
     """All legs of one config on this rank's GPU; returns the record on rank 0 (None elsewhere)."""
     rank, world = comm.rank, comm.world
     steps = args.steps if args.steps is not None else DEFAULT_STEPS[cfg["kind"]]
-    if args.steps is not None and key != args.head:
-        # the driver's --steps is sized for the headline; keep the sub-records' timed regions comparable in length
-        steps = max(args.steps, DEFAULT_STEPS[cfg["kind"]])
     warmup = max(args.warmup, 3)
     wl = Workload(ctx, vb, cfg, first_utt=rank * cfg["utts"], want_host=not args.device_only)
     F = wl.F
@@ -749,6 +768,8 @@ def gpu_record(ctx, vb, key, cfg, args, comm, clocks, peaks):
     counters = ctx.profile_counters()
     launches = ctx.kernel_launches - l0
     t_b = time.perf_counter()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, key, wl.outputs())
     comm.barrier()
     ms = comm.max(ms)
     rec = None
@@ -950,7 +971,8 @@ def run_ours(args, keys, rank, world, local_rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=None)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps of every config (default: a count per config, DEFAULT_STEPS)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="all", choices=["all", "c1"] + sorted(CONFIGS),
@@ -960,7 +982,12 @@ def main():
     ap.add_argument("--no-multi", action="store_true", help="skip the in-library multi-GPU leg at N > 1")
     ap.add_argument("--device-only", action="store_true",
                     help="device-resident steps only (no e2e / cpu legs): the command the ncu launch lists under profiles/ are taken with")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<config>_<name>.npy (rank 0's GPU; "
+                         "a fixed, seeded sample of the rows of a larger output)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.config == "c1"):
+        ap.error("--dump-outputs writes the outputs of the GPU path: it needs --impl ours and a GPU config")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
