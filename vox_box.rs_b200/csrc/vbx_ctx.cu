@@ -69,6 +69,23 @@ int vbx_arena_reserve(vbx_ctx* ctx, size_t bytes) {
     return VBX_OK;
 }
 
+int vbx_hard_list_reserve(vbx_ctx* ctx, int64_t n) {
+    if (n <= ctx->hard_cap) return VBX_OK;
+    // grow-only; a fix-up launch of an earlier call may still read the list from the side stream
+    if (ctx->s_side) VBX_CUDA(ctx, cudaStreamSynchronize(ctx->s_side));
+    VBX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (ctx->hard_list) cudaFree(ctx->hard_list);
+    ctx->hard_list = nullptr;
+    ctx->hard_cap = 0;
+    const cudaError_t e = cudaMalloc(&ctx->hard_list, (size_t)n * sizeof(int));
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return vbx_fail(ctx, VBX_ERR_NOMEM, "roots fix-up list: cudaMalloc(%zu) failed: %s", (size_t)n * sizeof(int), cudaGetErrorString(e));
+    }
+    ctx->hard_cap = n;
+    return VBX_OK;
+}
+
 int vbx_scratch_get(vbx_ctx* ctx, size_t bytes, void** out) {
     if (ctx->sub_scratch) {
         if (bytes > ctx->sub_scratch_bytes)
@@ -273,7 +290,6 @@ int vbx_ctx_create(int device, vbx_ctx** out) {
             return VBX_ERR_CUDA;
         }
     if (cudaMalloc(&ctx->tile_counter, 256) != cudaSuccess) { delete ctx; return VBX_ERR_CUDA; }
-    if (cudaMalloc(&ctx->hard_list, vbx_ctx::kHardCap * sizeof(int)) != cudaSuccess) { delete ctx; return VBX_ERR_CUDA; }
     {
         // the tracker's CTAs should be dispatched ahead of the queued LPC / roots grids: highest priority
         int lo = 0, hi = 0;

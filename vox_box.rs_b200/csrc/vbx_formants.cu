@@ -254,14 +254,15 @@ int launch_burg(vbx_ctx* ctx, const vbx_frames* fr, int p, void* coeffs_out, uin
 // =============================================================================================
 using namespace vbx_roots;
 
-// The f64 fix-up launch behind lpc_roots_pair_kernel (see there): redoes the frames of ctx->hard_list with the reference's own
-// algorithm.  Covers the list's capacity; CTAs beyond the list's length return at once (an empty list costs a few µs, a flagged
-// frame ~0.25 ms of single-thread latency — which is why vbx_find_formants puts this launch on its side stream).
+// The f64 fix-up launch behind lpc_roots_pair_kernel (see there): redoes the frames of the pair kernel's list (Q.hard_list /
+// Q.hard_count if the caller chose one, else ctx->hard_list) with the reference's own algorithm.  One CTA per SM at most walks
+// the list (an empty list costs a few µs, a flagged frame ~0.25 ms of single-thread latency — which is why vbx_find_formants puts
+// this launch on its side stream).
 int launch_roots_fixup(vbx_ctx* ctx, const RootsParams& Q, int p, cudaStream_t stream) {
     RootsParams Q2 = Q;
-    Q2.frame_list = ctx->hard_list;
-    Q2.frame_count = ctx->tile_counter + 1;
-    Q2.hard_cap = vbx_ctx::kHardCap;
+    Q2.frame_list = Q.hard_list ? Q.hard_list : ctx->hard_list;
+    Q2.frame_count = Q.hard_list ? Q.hard_count : ctx->tile_counter + 1;
+    Q2.hard_cap = Q.hard_list ? Q.hard_cap : (int)ctx->hard_cap;
     Q2.hard_list = nullptr;
     Q2.hard_count = nullptr;
     Q2.work = nullptr;
@@ -269,7 +270,10 @@ int launch_roots_fixup(vbx_ctx* ctx, const RootsParams& Q, int p, cudaStream_t s
     VBX_CUDA(ctx, cudaFuncSetAttribute(lpc_roots_rt_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_fix));
     const bool side = (stream != ctx->stream);
     const int slot = side ? vbx_prof_range_begin(ctx, "lpc_roots_rt_kernel<double> (fix-up launch)", stream) : -1;
-    lpc_roots_rt_kernel<double><<<vbx_ctx::kHardCap / kRootsThreads, kRootsThreads, smem_fix, stream>>>(Q2, p);
+    // one CTA per SM at most: enough for the few frames speech flags; a batch that flags most of its frames (tonal input) walks
+    // the list at low occupancy, a latency not measured (DESIGN.md K3+K4)
+    const int64_t grid = std::min<int64_t>((Q.n_frames + kRootsThreads - 1) / kRootsThreads, ctx->sm_count);
+    lpc_roots_rt_kernel<double><<<(unsigned)grid, kRootsThreads, smem_fix, stream>>>(Q2, p);
     if (side) {
         vbx_prof_range_end(ctx, slot, stream);
         const cudaError_t e = cudaGetLastError();
@@ -286,8 +290,8 @@ int launch_roots_fixup(vbx_ctx* ctx, const RootsParams& Q, int p, cudaStream_t s
 int launch_lpc_roots(vbx_ctx* ctx, const RootsParams& Q, int p, int precision /*0 fast f32+polish, 1 f64*/, bool* defer_fixup = nullptr) {
     if (defer_fixup) *defer_fixup = false;
     VBX_REQUIRE(ctx, p >= 2 && p <= kMaxRootsOrder, "LPC order for root finding must be in 2..%d", kMaxRootsOrder);
+    VBX_REQUIRE(ctx, Q.n_frames <= 0x7fffffffLL, "too many frames for one launch");  // frame indices of the fix-up list are int
     const int64_t grid = (Q.n_frames + kRootsThreads - 1) / kRootsThreads;
-    VBX_REQUIRE(ctx, grid <= 0x7fffffffLL, "too many frames for one launch");
     const bool f32 = (precision != 1);
     // fp32 path without a request for the roots themselves: conjugate-pair deflation (vbx_roots_kernel.cuh); VBX_ROOTS_PAIR=0
     // keeps the reference's one-root-at-a-time order for A/B runs
@@ -307,9 +311,13 @@ int launch_lpc_roots(vbx_ctx* ctx, const RootsParams& Q, int p, int precision /*
         const int64_t grid_pair = (Q.n_frames + rthreads - 1) / rthreads;
         RootsParams Q1 = Q;
         Q1.work = vbx_work_ptr(ctx);
-        Q1.hard_list = ctx->hard_list;
-        Q1.hard_count = ctx->tile_counter + 1;
-        Q1.hard_cap = vbx_ctx::kHardCap;
+        if (!Q.hard_list) {  // the caller's own list holds at least n_frames entries (vbx_find_formants), else the context's
+            const int st = vbx_hard_list_reserve(ctx, Q.n_frames);
+            if (st != VBX_OK) return st;
+            Q1.hard_list = ctx->hard_list;
+            Q1.hard_count = ctx->tile_counter + 1;
+            Q1.hard_cap = (int)ctx->hard_cap;
+        }
         if (const char* e = getenv("VBX_ROOTS_FORCE_HARD")) Q1.hard_mod = atoi(e);
         VBX_CUDA(ctx, cudaMemsetAsync(Q1.hard_count, 0, sizeof(unsigned), ctx->stream));
         if (rthreads == 96) lpc_roots_pair_kernel<96><<<(unsigned)grid_pair, 96, smem_pair, ctx->stream>>>(Q1, p);
@@ -935,7 +943,8 @@ static int lpc_to_resonances_impl(vbx_ctx* ctx, const void* lpc, int32_t lpc_dty
                                   int32_t lpc_has_leading_one, double sample_rate, int32_t strict_im, const uint8_t* status_in,
                                   void* res_out, int32_t res_slots, int32_t* nres_out, void* roots_out, uint8_t* status_out,
                                   int32_t out_dtype, int32_t precision, int64_t in_J, int64_t out_J, int64_t out_j0,
-                                  RootsParams* q_out = nullptr, bool* defer_fixup = nullptr) {
+                                  RootsParams* q_out = nullptr, bool* defer_fixup = nullptr, int* hard_list = nullptr,
+                                  unsigned* hard_count = nullptr, int hard_cap = 0) {
     if (!ctx) return VBX_ERR_BADARG;
     VBX_REQUIRE(ctx, lpc_dtype == VBX_F32 || lpc_dtype == VBX_F64, "lpc_dtype must be VBX_F32 or VBX_F64");
     VBX_REQUIRE(ctx, out_dtype == VBX_F32 || out_dtype == VBX_F64, "out_dtype must be VBX_F32 or VBX_F64");
@@ -954,7 +963,7 @@ static int lpc_to_resonances_impl(vbx_ctx* ctx, const void* lpc, int32_t lpc_dty
     if (const char* e = getenv("VBX_ROOTS_POLISH")) Q.polish_steps = atoi(e);  // A/B runs
     Q.work = vbx_work_ptr(ctx);
     Q.in_J = in_J; Q.out_J = out_J; Q.out_j0 = out_j0;
-    Q.hard_list = nullptr; Q.hard_count = nullptr; Q.hard_cap = 0; Q.hard_mod = 0; Q.frame_list = nullptr; Q.frame_count = nullptr;
+    Q.hard_list = hard_list; Q.hard_count = hard_count; Q.hard_cap = hard_cap; Q.hard_mod = 0; Q.frame_list = nullptr; Q.frame_count = nullptr;
     if (q_out) *q_out = Q;
     return launch_lpc_roots(ctx, Q, p, precision < 0 ? root_precision_default() : precision, defer_fixup);
 }
@@ -1196,8 +1205,12 @@ int vbx_find_formants(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
     };
     int64_t Jc_max = 1;
     for (int c = 0; c < K; ++c) Jc_max = std::max<int64_t>(Jc_max, chunk_begin(c + 1) - chunk_begin(c));
-    // scratch: lpc [segs·Jc_max][p+1] f64 | lpc status [segs·Jc_max] | status [F] | resonances [F][p] pairs | nres [F]
-    // (the last three only when the caller does not ask for them)
+    // With overlap, chunk c's roots fix-up runs on the side stream and reads the chunk-local LPC rows, LPC status and fix-up
+    // list; chunk c + 1 works on a second set of them, and chunk c + 2 waits for that fix-up before it reuses the first.
+    const bool overlap = track && K > 1 && side_stream != ctx->stream;
+    const int nbuf = overlap ? 2 : 1;
+    // scratch: nbuf × (lpc [segs·Jc_max][p+1] f64) | nbuf × (lpc status [segs·Jc_max]) | status [F] | resonances [F][p] pairs |
+    // nres [F] (the last three only when the caller does not ask for them)
     auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
     const int64_t Fc_max = segs * Jc_max;
     const size_t lpc_bytes = al((size_t)Fc_max * (p + 1) * sizeof(double));
@@ -1214,8 +1227,11 @@ int vbx_find_formants(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
     cfr.n_frames = Fc_max;
     cfr.frames_per_segment = Jc_max;
     const size_t sub_bytes = al(lpc_method == VBX_LPC_BURG ? vbx_burg_scratch_bytes(ctx, &cfr) : vbx_lpc_scratch_bytes(ctx, &cfr, p + 1));
-    const size_t own_bytes = lpc_bytes + stl_bytes + st_bytes + res_bytes + nres_bytes;
+    const size_t lst_bytes = nbuf * (lpc_bytes + stl_bytes);
+    const size_t own_bytes = lst_bytes + st_bytes + res_bytes + nres_bytes;
     st = vbx_arena_reserve(ctx, own_bytes + sub_bytes);
+    if (st != VBX_OK) return st;
+    st = vbx_hard_list_reserve(ctx, nbuf * Fc_max);  // fix-up list(s): Fc_max entries each, counts in tile_counter[1 + b]
     if (st != VBX_OK) return st;
     char* base = (char*)ctx->arena;
     struct SubScratch {  // scoped: the callees of this call see the sub-range, nobody else does
@@ -1223,16 +1239,25 @@ int vbx_find_formants(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
         SubScratch(vbx_ctx* c_, void* p_, size_t b_) : c(c_) { c->sub_scratch = b_ ? p_ : nullptr; c->sub_scratch_bytes = b_; }
         ~SubScratch() { c->sub_scratch = nullptr; c->sub_scratch_bytes = 0; }
     };
-    double* d_lpc = (double*)base;
-    uint8_t* d_st_lpc = (uint8_t*)(base + lpc_bytes);
-    uint8_t* d_st = status_out ? status_out : (uint8_t*)(base + lpc_bytes + stl_bytes);
-    void* d_res = own_res ? (void*)(base + lpc_bytes + stl_bytes + st_bytes) : resonances_out;
-    int32_t* d_nres = nres_out ? nres_out : (int32_t*)(base + lpc_bytes + stl_bytes + st_bytes + res_bytes);
+    uint8_t* d_st = status_out ? status_out : (uint8_t*)(base + lst_bytes);
+    void* d_res = own_res ? (void*)(base + lst_bytes + st_bytes) : resonances_out;
+    int32_t* d_nres = nres_out ? nres_out : (int32_t*)(base + lst_bytes + st_bytes + res_bytes);
+    bool fixup_queued[2] = {false, false};  // a fix-up launch reads buffer set b (its completion: ev_side[2 + b])
     const size_t es = vbx_dtype_size(frames->dtype);
     const int64_t seg_stride = frames->frames_per_segment > 0 ? frames->segment_stride : 0;
     for (int c = 0; c < K; ++c) {
         const int64_t j0 = chunk_begin(c), j1 = chunk_begin(c + 1), Jc = j1 - j0;
         if (Jc <= 0) continue;
+        const int b = c % nbuf;  // buffer set of this chunk
+        double* d_lpc = (double*)(base + b * lpc_bytes);
+        uint8_t* d_st_lpc = (uint8_t*)(base + nbuf * lpc_bytes + b * stl_bytes);
+        if (fixup_queued[b]) {  // chunk c − 2's fix-up still reads this set
+            fixup_queued[b] = false;
+            if (cudaStreamWaitEvent(ctx->stream, ctx->ev_side[2 + b], 0) != cudaSuccess) {
+                st = vbx_fail(ctx, VBX_ERR_CUDA, "find_formants: wait for the roots fix-up failed: %s", cudaGetErrorString(cudaGetLastError()));
+                break;
+            }
+        }
         vbx_frames sub = *frames;
         sub.base = (const char*)frames->base + (size_t)j0 * frames->frame_stride * es;
         sub.n_frames = segs * Jc;
@@ -1258,12 +1283,12 @@ int vbx_find_formants(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
             }
         }
         if (st != VBX_OK) break;
-        const bool overlap = track && K > 1 && side_stream != ctx->stream;
         RootsParams Qc;
         bool fixup_pending = false;
         st = lpc_to_resonances_impl(ctx, d_lpc, VBX_F64, sub.n_frames, lpc_stride, p, has_one, sample_rate, /*strict_im=*/1, lpc_status,
                                     d_res, R, d_nres, nullptr, d_st, dtype, -1, K > 1 ? Jc : 0, K > 1 ? J : 0, K > 1 ? j0 : 0, &Qc,
-                                    overlap ? &fixup_pending : nullptr);
+                                    overlap ? &fixup_pending : nullptr, ctx->hard_list + b * Fc_max, ctx->tile_counter + 1 + b,
+                                    (int)Fc_max);
         if (st != VBX_OK) break;
         if (!track) continue;
         if (K == 1) {
@@ -1288,6 +1313,11 @@ int vbx_find_formants(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
         if (fixup_pending) {  // the roots fix-up (rarely any work, but ~0.25 ms of latency when there is) rides the side stream too
             st = launch_roots_fixup(ctx, Qc, p, side_stream);
             if (st != VBX_OK) break;
+            if (cudaEventRecord(ctx->ev_side[2 + b], ctx->s_side) != cudaSuccess) {
+                st = vbx_fail(ctx, VBX_ERR_CUDA, "find_formants: fix-up event failed: %s", cudaGetErrorString(cudaGetLastError()));
+                break;
+            }
+            fixup_queued[b] = true;
         }
         st = estimate_formants_impl(ctx, d_res, dtype, R, VBX_MAX_RESONANCES, segs, J, d_st, est_inout, n_formants, tracks_out, dtype,
                                     d_nres, j0, Jc, side_stream, /*packed=*/c + 1 < K);

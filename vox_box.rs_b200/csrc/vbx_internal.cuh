@@ -41,7 +41,8 @@ struct vbx_ctx {
     void* pipe = nullptr;
     size_t pipe_bytes = 0;
     // side stream of vbx_find_formants (the latency-bound tracker of frame chunk c runs there while the main stream computes
-    // the LPC / roots of chunk c + 1); ev_side: [0..1] chunk c's resonances ready, [2..3] chunk c's tracker done, by chunk parity
+    // the LPC / roots of chunk c + 1); ev_side: [0..1] chunk c's resonances ready, [2..3] the roots fix-up of the chunk that
+    // used buffer set 0 / 1 done (the set may be reused); [2] also the join after the last chunk's tracker
     cudaStream_t s_side = nullptr;
     cudaEvent_t ev_side[4] = {nullptr, nullptr, nullptr, nullptr};
     // window tables (device, f64), keyed by (kind << 32 | n)
@@ -60,9 +61,9 @@ struct vbx_ctx {
     unsigned long long* work_counters = nullptr;
     int reserve_sms = 0;               // SMs the persistent kernels leave free for a co-running side-stream kernel
     bool roots_small = false;          // lpc_roots_pair_kernel in 96-thread CTAs (they fit beside a persistent LPC CTA)
-    unsigned* tile_counter = nullptr;  // device: [0] the persistent kernels' dynamic tile cursor, [1] length of hard_list
+    unsigned* tile_counter = nullptr;  // device: [0] the persistent kernels' dynamic tile cursor, [1..2] lengths of fix-up lists
     int* hard_list = nullptr;          // device: frames the pair-deflation roots kernel hands to the f64 fix-up launch
-    static constexpr int kHardCap = 4096;
+    int64_t hard_cap = 0;              // entries of hard_list (vbx_hard_list_reserve: as many as a roots launch has frames)
     vbx_mfcc_cache* mfcc_cache = nullptr;
     bool mfcc_fft_f32 = false;  // MFCC transform precision (default fp64)
 };
@@ -78,6 +79,7 @@ int vbx_prof_range_begin(vbx_ctx* ctx, const char* name, cudaStream_t stream);
 void vbx_prof_range_end(vbx_ctx* ctx, int slot, cudaStream_t stream);
 int vbx_arena_reserve(vbx_ctx* ctx, size_t bytes);         // ensures ctx->arena has >= bytes
 int vbx_pinned_reserve(vbx_ctx* ctx, size_t bytes);        // ensures ctx->pinned has >= bytes
+int vbx_hard_list_reserve(vbx_ctx* ctx, int64_t n);        // ensures ctx->hard_list has >= n entries
 // scratch for a kernel launcher: the caller-provided sub-range if one is set (see vbx_ctx::sub_scratch), else the arena
 int vbx_scratch_get(vbx_ctx* ctx, size_t bytes, void** out);
 // scratch the LPC stage of vbx_find_formants may ask for through vbx_scratch_get (0 when the fused kernels apply)

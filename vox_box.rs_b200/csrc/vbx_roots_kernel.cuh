@@ -48,8 +48,9 @@ struct RootsParams {
     // output row (f / in_J)·out_J + out_j0 + f % in_J of the caller's [utterance][frame] layout.  out_J == 0: identity.
     int64_t in_J, out_J, out_j0;
     // Frames on which a solve of the pair kernel ran into its 20-iteration cap WITHOUT converging are appended here (capacity
-    // hard_cap); the fix-up launch of the f64 reference-order kernel then redoes exactly those frames (frame_list / frame_count
-    // set: thread i works on frame frame_list[i]).  hard_mod > 0 (tests): every hard_mod-th frame is treated as hard.
+    // hard_cap, at least the launch's frame count: no frame is dropped); the fix-up launch of the f64 reference-order kernel then
+    // redoes exactly those frames (frame_list / frame_count set: list entry i is frame frame_list[i]).  hard_mod > 0 (tests):
+    // every hard_mod-th frame is treated as hard.
     int* hard_list;
     unsigned* hard_count;
     int hard_cap, hard_mod;
@@ -130,8 +131,9 @@ __device__ __forceinline__ vcx<TR> laguerre_step(vcx<TR> a0, vcx<TR> a1, vcx<TR>
     }
 }
 
+// One frame of lpc_roots_rt_kernel: list entry `item` of n_items (the frame itself, or the fix-up list's item-th frame).
 template <typename TR>
-__global__ void __launch_bounds__(kRootsThreads) lpc_roots_rt_kernel(const RootsParams Q, const int P) {
+__device__ __forceinline__ void lpc_roots_rt_frame(const RootsParams& Q, const int P, const int64_t item, const int64_t n_items) {
     extern __shared__ __align__(16) unsigned char roots_smem[];
     constexpr int T = kRootsThreads;
     const unsigned FULL = 0xffffffffu;
@@ -139,14 +141,8 @@ __global__ void __launch_bounds__(kRootsThreads) lpc_roots_rt_kernel(const Roots
     vcx<TR>* c_s = reinterpret_cast<vcx<TR>*>(a_s + (size_t)(P + 1) * T);   // [P+1][T] working polynomial
     vcx<TR>* r_s = c_s + (size_t)(P + 1) * T;                               // [P][T]   roots in find_roots order
     const int tid = threadIdx.x;
-    int64_t f_raw = (int64_t)blockIdx.x * T + tid;
-    bool in_range = f_raw < Q.n_frames;
-    if (Q.frame_list) {  // fix-up launch: the frames the pair kernel flagged
-        const unsigned cnt = min(*Q.frame_count, (unsigned)Q.hard_cap);
-        if ((unsigned)blockIdx.x * T >= cnt) return;  // CTA-uniform
-        in_range = f_raw < (int64_t)cnt;
-        f_raw = Q.frame_list[in_range ? f_raw : 0];
-    }
+    const bool in_range = item < n_items;
+    const int64_t f_raw = Q.frame_list ? (int64_t)Q.frame_list[in_range ? item : 0] : item;
     const int64_t f = in_range ? f_raw : Q.n_frames - 1;
     const int64_t fo = Q.out_J ? (f / Q.in_J) * Q.out_J + Q.out_j0 + (f % Q.in_J) : f;  // output row  // out-of-range lanes shadow the last frame (no stores): warp-wide ops stay full
     const int R = Q.R;
@@ -317,6 +313,16 @@ __global__ void __launch_bounds__(kRootsThreads) lpc_roots_rt_kernel(const Roots
         }
         for (int s = cnt; s < R; ++s) write_res(s, 0.0, 0.0);
     }
+}
+
+// A plain launch covers its frames with its grid (one trip of the loop).  The fix-up launch (frame_list set) walks the list of
+// frames the pair kernel flagged with a grid-stride loop, so a grid of any size covers a list of any length.
+template <typename TR>
+__global__ void __launch_bounds__(kRootsThreads) lpc_roots_rt_kernel(const RootsParams Q, const int P) {
+    const int64_t n_items = Q.frame_list ? (int64_t)min(*Q.frame_count, (unsigned)Q.hard_cap) : Q.n_frames;
+#pragma unroll 1
+    for (int64_t i0 = (int64_t)blockIdx.x * kRootsThreads; i0 < n_items; i0 += (int64_t)gridDim.x * kRootsThreads)  // CTA-uniform
+        lpc_roots_rt_frame<TR>(Q, P, i0 + threadIdx.x, n_items);
 }
 
 // ---------------------------------------------------------------------------------------------
