@@ -260,7 +260,8 @@ VBX_API int vbx_find_formants_host(vbx_ctx* ctx, const vbx_frames* frames, doubl
 /* ---- periodic.rs:356-456  Pitched::pitch::<Hanning> (+ LocalMaxima :362-375, Pitch :306-318) --------------------- */
 /* Boersma autocorrelation pitch candidates for every frame of the view (the frame is windowed by frames->window as
  * the reference's callers do, Windower::hanning => HANN_SYMMETRIC; the lag window is HanningLag, the only LagType).
- * The reference ignores its local_peak / global_peak arguments (periodic.rs:396), so they are not parameters.
+ * The reference ignores its local_peak / global_peak arguments (periodic.rs:396), so they are not parameters (the opt-in
+ * vbx_pitch_with_peaks below honours them).
  * cand_out: [F][max_candidates] (frequency, strength) pairs of out_dtype, sorted by strength descending exactly as
  * the returned Vec (stable; the unvoiced candidate {0, threshold} is always part of it), zero padded;
  * n_cand_out[f] (optional) = length of the reference's Vec (may exceed max_candidates: the list is truncated);
@@ -273,6 +274,35 @@ VBX_API int vbx_pitch(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
 VBX_API int vbx_pitch_host(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate, double threshold, double min_hz,
                            double max_hz, int32_t max_candidates, void* cand_out, int32_t* n_cand_out,
                            uint8_t* status_out, int32_t out_dtype);
+/* Opt-in extension: the reference's local_peak / global_peak honoured (periodic.rs:357 takes them, :396 ignores them).  In
+ * Boersma (1993), the algorithm vbx_pitch implements, they make a quiet frame unvoiced: every frame is normalised (periodic.rs:404),
+ * so without them a faint periodic component scores as high as loud speech.
+ *  - local peak of frame f: max |x| over its frame_len samples as loaded (VBX_I16 scaled by 1/32767), before frames->window.
+ *    NaN samples are ignored (a NaN never wins the max, as in max_amplitude, waves.rs:45-58); an all-NaN frame has peak 0.
+ *  - global peak of segment u: the same max over every sample its frames span, [u*segment_stride, u*segment_stride +
+ *    (J-1)*frame_stride + frame_len) (with hop > frame_len this includes the samples between frames); for a single-segment view,
+ *    the whole extent of the view.
+ *  - unvoiced strength, a = threshold, b = silence_threshold: ratio = min(local / global, 1), ratio = 0 where global <= 0 or is
+ *    NaN; b > 0: R_f = a + max(0, 2 - ratio * (1 + a) / b) (Boersma 1993; Praat's voiceless strength); b == 0: R_f = a, i.e.
+ *    exactly vbx_pitch (no peaks are read or computed); b < 0: VBX_ERR_BADARG.  A NaN ratio (a NaN local peak) gives R_f = a.
+ * The candidate list is vbx_pitch's with the unvoiced entry's strength replaced by R_f, placed by the same stable descending
+ * sort before truncation to max_candidates: it still goes after voiced candidates of equal strength, n_cand_out is unchanged,
+ * and VBX_ERR_PITCH frames stay unsorted.  Praat's subtraction of the local mean and its centre-only local-peak region are not
+ * implemented.
+ * local_peaks [F] / global_peaks [n_segments] (device pointers for vbx_pitch_with_peaks, host pointers for the _host twins) may
+ * each be NULL = computed as above from the view.  The reference takes them per call: a caller that analyses one recording over
+ * several calls passes the recording-wide global peak.  The _host and _multi_host twins equal the device call bit for bit. */
+VBX_API int vbx_frame_peaks(vbx_ctx* ctx, const vbx_frames* frames, double* local_out /* [F] or NULL */,
+                            double* global_out /* [n_segments] or NULL */);
+VBX_API int vbx_pitch_with_peaks(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate, double threshold,
+                                 double silence_threshold, const double* local_peaks /* [F] or NULL = computed */,
+                                 const double* global_peaks /* [n_segments] or NULL = computed */, double min_hz,
+                                 double max_hz, int32_t max_candidates, void* cand_out, int32_t* n_cand_out, uint8_t* status_out,
+                                 int32_t out_dtype);
+VBX_API int vbx_pitch_with_peaks_host(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate, double threshold,
+                                      double silence_threshold, const double* local_peaks, const double* global_peaks,
+                                      double min_hz, double max_hz, int32_t max_candidates, void* cand_out, int32_t* n_cand_out,
+                                      uint8_t* status_out, int32_t out_dtype);
 /* periodic.rs:403-408: the lag function the candidates are read from (`self_lag`: autocorrelate(N) of the windowed frame,
  * normalize(), divided by the HanningLag window) for every frame of the view: lag_out [F][frame_len] f64 (device).  The reference
  * zero-extends it to 2N (:411) before interpolating. */
@@ -378,6 +408,10 @@ VBX_API int vbx_multi_find_formants_host(vbx_multi* m, const vbx_frames* frames,
 VBX_API int vbx_multi_pitch_host(vbx_multi* m, const vbx_frames* frames, double sample_rate, double threshold, double min_hz,
                                  double max_hz, int32_t max_candidates, void* cand_out, int32_t* n_cand_out,
                                  uint8_t* status_out, int32_t out_dtype);
+VBX_API int vbx_multi_pitch_with_peaks_host(vbx_multi* m, const vbx_frames* frames, double sample_rate, double threshold,
+                                            double silence_threshold, const double* local_peaks, const double* global_peaks,
+                                            double min_hz, double max_hz, int32_t max_candidates, void* cand_out,
+                                            int32_t* n_cand_out, uint8_t* status_out, int32_t out_dtype);
 VBX_API int vbx_multi_mfcc_host(vbx_multi* m, const vbx_frames* frames, int32_t num_coeffs, int32_t n_keep, double freq_lo,
                                 double freq_hi, double sample_rate, void* out, int32_t out_dtype);
 /* Host->device copy bandwidth (GB/s per device, gbs_out[n_devices]) with the first n_active devices copying concurrently from

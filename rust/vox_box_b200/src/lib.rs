@@ -161,6 +161,15 @@ pub mod ffi {
                               max_hz: f64, max_candidates: i32, cand_out: *mut c_void, n_cand_out: *mut i32, status_out: *mut u8,
                               out_dtype: i32) -> c_int;
         pub fn vbx_pitch_lag_function(ctx: *mut vbx_ctx, frames: *const vbx_frames, lag_out: *mut f64) -> c_int;
+        pub fn vbx_frame_peaks(ctx: *mut vbx_ctx, frames: *const vbx_frames, local_out: *mut f64, global_out: *mut f64) -> c_int;
+        pub fn vbx_pitch_with_peaks(ctx: *mut vbx_ctx, frames: *const vbx_frames, sample_rate: f64, threshold: f64,
+                                    silence_threshold: f64, local_peaks: *const f64, global_peaks: *const f64, min_hz: f64,
+                                    max_hz: f64, max_candidates: i32, cand_out: *mut c_void, n_cand_out: *mut i32,
+                                    status_out: *mut u8, out_dtype: i32) -> c_int;
+        pub fn vbx_pitch_with_peaks_host(ctx: *mut vbx_ctx, frames: *const vbx_frames, sample_rate: f64, threshold: f64,
+                                         silence_threshold: f64, local_peaks: *const f64, global_peaks: *const f64, min_hz: f64,
+                                         max_hz: f64, max_candidates: i32, cand_out: *mut c_void, n_cand_out: *mut i32,
+                                         status_out: *mut u8, out_dtype: i32) -> c_int;
         pub fn vbx_pitch_extract(ctx: *mut vbx_ctx, cand: *const c_void, dtype: i32, n_frames: i64, max_candidates: i32,
                                  out: *mut c_void) -> c_int;
         pub fn vbx_pitch_viterbi(ctx: *mut vbx_ctx, cand: *const c_void, dtype: i32, n_cand: *const i32, n_segments: i64,
@@ -204,6 +213,10 @@ pub mod ffi {
         pub fn vbx_multi_pitch_host(m: *mut vbx_multi, frames: *const vbx_frames, sample_rate: f64, threshold: f64, min_hz: f64,
                                     max_hz: f64, max_candidates: i32, cand_out: *mut c_void, n_cand_out: *mut i32,
                                     status_out: *mut u8, out_dtype: i32) -> c_int;
+        pub fn vbx_multi_pitch_with_peaks_host(m: *mut vbx_multi, frames: *const vbx_frames, sample_rate: f64, threshold: f64,
+                                               silence_threshold: f64, local_peaks: *const f64, global_peaks: *const f64,
+                                               min_hz: f64, max_hz: f64, max_candidates: i32, cand_out: *mut c_void,
+                                               n_cand_out: *mut i32, status_out: *mut u8, out_dtype: i32) -> c_int;
         pub fn vbx_multi_mfcc_host(m: *mut vbx_multi, frames: *const vbx_frames, num_coeffs: i32, n_keep: i32, freq_lo: f64,
                                    freq_hi: f64, sample_rate: f64, out: *mut c_void, out_dtype: i32) -> c_int;
         pub fn vbx_multi_h2d_bandwidth(m: *mut vbx_multi, bytes_per_device: usize, reps: i32, n_active: i32, gbs_out: *mut f64) -> c_int;
@@ -600,6 +613,32 @@ pub mod periodic {
                 cand
             })
         }
+    }
+
+    /// Opt-in extension of `Pitched::pitch` that honours `local_peak` / `global_peak` (the reference takes them and ignores
+    /// them, periodic.rs:396): the unvoiced candidate's strength is Boersma's (1993) voiceless strength
+    /// `threshold + max(0, 2 − min(local_peak / global_peak, 1)·(1 + threshold) / silence_threshold)` instead of `threshold`,
+    /// so quiet frames rank it first.  `silence_threshold == 0` is exactly `pitch()` (Praat's default is 0.03 with a voicing
+    /// threshold of 0.45).  The peaks are max |x| of the frame and of the whole recording, as the reference's driver computes
+    /// them (examples/pitch_detection.rs:48); see `vbx_pitch_with_peaks` in include/voxbox_b200.h.  A free function rather than a
+    /// method, so that the `Pitched` trait keeps the reference's surface.
+    pub fn pitch_with_peaks<W: LagType, S: Elem, T: Elem>(samples: &[S], sample_rate: T, threshold: T, silence_threshold: T,
+                                                          local_peak: S, global_peak: S, min: T, max: T) -> Vec<Pitch<T>> {
+        with_context(|ctx| {
+            let fr = one_frame(samples, ffi::VBX_WINDOW_NONE);
+            let cap = samples.len() / 4 + 2; // as pitch(): every other lag below N/2 a maximum, plus the unvoiced candidate
+            let mut cand = vec![Pitch::<T>::default(); cap];
+            let (mut n, mut st) = ([0i32; 1], [0u8; 1]);
+            let (local, global) = ([local_peak.to_f64()], [global_peak.to_f64()]);
+            ctx.check(unsafe {
+                ffi::vbx_pitch_with_peaks_host(ctx.raw(), &fr, sample_rate.to_f64(), threshold.to_f64(), silence_threshold.to_f64(),
+                                               local.as_ptr(), global.as_ptr(), min.to_f64(), max.to_f64(), cap as i32,
+                                               cand.as_mut_ptr() as *mut c_void, n.as_mut_ptr(), st.as_mut_ptr(), T::DTYPE)
+            }).expect("pitch_with_peaks");
+            assert!(st[0] == 0, "pitch_with_peaks: a candidate strength is NaN (the reference's sort panics here)");
+            cand.truncate(n[0] as usize);
+            cand
+        })
     }
 
     /// periodic.rs:29-87

@@ -86,6 +86,10 @@ int vbx_scratch_get(vbx_ctx* ctx, size_t bytes, void** out);
 size_t vbx_lpc_scratch_bytes(vbx_ctx* ctx, const vbx_frames* fr, int n_lags);
 size_t vbx_burg_scratch_bytes(vbx_ctx* ctx, const vbx_frames* fr);
 int vbx_pipe_reserve(vbx_ctx* ctx, size_t bytes);          // ensures ctx->pipe has >= bytes
+// vbx_peaks.cu: per-frame (local_out [F]) and per-segment (global_out [n_segments]) max |x| of a device view, either may be
+// null; and the same max over the whole extent of a host view (the global peak of a single-segment view)
+int vbx_launch_frame_peaks(vbx_ctx* ctx, const vbx_frames* fr, double* local_out, double* global_out);
+double vbx_host_peak(const vbx_frames* fr);
 // cached device table (ones for NONE).  sample_dtype == VBX_I16 folds the PCM scale into the table: w[i] / 32767
 // (tests/lib.rs:17-19 scale every sample by 1/(i32::MAX >> 16) before any arithmetic).
 int vbx_get_window(vbx_ctx* ctx, int kind, int n, const double** dev_out, int sample_dtype = VBX_F32);

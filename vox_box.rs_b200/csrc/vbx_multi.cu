@@ -272,6 +272,33 @@ int vbx_multi_pitch_host(vbx_multi* m, const vbx_frames* frames, double sample_r
     });
 }
 
+// A single-segment view is split into frame ranges, so its missing global peak is taken over the whole view first, as
+// vbx_pitch_with_peaks_host does for its chunks; every device then reads the same value.
+int vbx_multi_pitch_with_peaks_host(vbx_multi* m, const vbx_frames* frames, double sample_rate, double threshold,
+                                    double silence_threshold, const double* local_peaks, const double* global_peaks, double min_hz,
+                                    double max_hz, int32_t max_candidates, void* cand_out, int32_t* n_cand_out, uint8_t* status_out,
+                                    int32_t out_dtype) {
+    if (!m || !frames) return VBX_ERR_BADARG;
+    const size_t pair = (out_dtype == VBX_F64) ? 16 : 8;
+    const bool segmented = frames->frames_per_segment > 0;
+    double whole = 0.0;
+    const double* global = global_peaks;
+    if (silence_threshold > 0.0 && !global && !segmented && frames->n_frames > 0 && frames->base && frames->frame_len >= 1 &&
+        frames->frame_stride >= 1 && (frames->dtype == VBX_F32 || frames->dtype == VBX_I16 || frames->dtype == VBX_F64)) {
+        whole = vbx_host_peak(frames);
+        global = &whole;
+    }
+    return run_all(m, [=](int i, vbx_ctx* ctx) -> int {
+        const Shard s = shard_of(frames, m->n, i, true);
+        if (s.fr.n_frames == 0) return VBX_OK;
+        return vbx_pitch_with_peaks_host(ctx, &s.fr, sample_rate, threshold, silence_threshold,
+                                         local_peaks ? local_peaks + s.frame0 : nullptr,
+                                         global ? global + (segmented ? s.seg0 : 0) : nullptr, min_hz, max_hz, max_candidates,
+                                         row(cand_out, s.frame0, (size_t)max_candidates * pair), (int32_t*)row(n_cand_out, s.frame0, 4),
+                                         (uint8_t*)row(status_out, s.frame0, 1), out_dtype);
+    });
+}
+
 int vbx_multi_mfcc_host(vbx_multi* m, const vbx_frames* frames, int32_t num_coeffs, int32_t n_keep, double freq_lo, double freq_hi,
                         double sample_rate, void* out, int32_t out_dtype) {
     if (!m || !frames) return VBX_ERR_BADARG;

@@ -23,7 +23,9 @@
 //                         minimiser (uniform control flow) with the 2(D+1)-term windowed-sinc sum
 //                         split over the lanes, all in fp64.
 //   pitch_finalize_kernel a warp per frame appends the unvoiced candidate, checks for NaN
-//                         strengths and rank-sorts by strength (stable, descending).
+//                         strengths and rank-sorts by strength (stable, descending).  With peaks
+//                         (vbx_pitch_with_peaks) the unvoiced candidate's strength is Boersma's voiceless
+//                         strength of the frame instead of the fixed threshold.
 #include <cmath>
 #include <type_traits>
 
@@ -58,7 +60,24 @@ struct PitchParams {
     int xs_words;           // shared-memory words per frame
     int ixmax;              // floor(N/2)
     double fs, fmin, fmax, threshold;
+    // vbx_pitch_with_peaks: local peak per frame of the batch, global peak per segment (both null for vbx_pitch)
+    const double* local_peak;
+    const double* global_peak;
+    double silence;         // silence threshold b > 0 of voiceless_strength
 };
+
+// Boersma (1993) / Praat's voiceless strength of a frame: a + max(0, 2 − ratio·(1 + a)/b), ratio = min(local/global, 1),
+// ratio = 0 where global <= 0 or is NaN; a NaN ratio (a NaN local peak) leaves a.  a = voicing threshold, b = silence
+// threshold > 0.  The test reference (tests/test_gpu_pitch_peaks.py) evaluates the same expression in the same order.
+__device__ __forceinline__ double voiceless_strength(double local, double global, double a, double b) {
+    double ratio = 0.0;
+    if (global > 0.0) {
+        ratio = local / global;
+        if (ratio > 1.0) ratio = 1.0;
+    }
+    const double v = 2.0 - ratio * (1.0 + a) / b;
+    return a + (v > 0.0 ? v : 0.0);
+}
 
 __device__ __forceinline__ int chunk_addr(int k) {  // word address of 8-word chunk k: 8k + 4·(8k/16)
     return 8 * k + 4 * (k >> 1);
@@ -882,7 +901,7 @@ __global__ void __launch_bounds__(128, VBX_REFINE_MINB) pitch_refine8q_kernel(co
     }
 }
 
-// K8: append the unvoiced candidate, NaN check, stable sort by strength descending (periodic.rs:452-453)
+// K8: append the unvoiced candidate ({0, threshold}, or {0, voiceless strength} with peaks), NaN check, stable sort by strength descending (periodic.rs:452-453)
 __global__ void __launch_bounds__(128) pitch_finalize_kernel(const PitchParams P, void* cand_out, int max_cand, int32_t* n_cand_out,
                                                              uint8_t* status_out, int out_f64) {
     const int lane = threadIdx.x & 31;
@@ -893,7 +912,9 @@ __global__ void __launch_bounds__(128) pitch_finalize_kernel(const PitchParams P
     const double2* it = P.refined + rg.x;
     const int cnt = rg.y, total = cnt + 1;
     const unsigned FULL = 0xffffffffu;
-    auto item = [&](int i) -> double2 { return i < cnt ? it[i] : make_double2(0.0, P.threshold); };
+    double unvoiced = P.threshold;
+    if (P.local_peak) unvoiced = voiceless_strength(P.local_peak[f], P.global_peak[f / P.seg_frames], P.threshold, P.silence);
+    auto item = [&](int i) -> double2 { return i < cnt ? it[i] : make_double2(0.0, unvoiced); };
     bool has_nan = false;
     for (int i = lane; i < total; i += 32) {
         const double s = item(i).y;
@@ -1040,9 +1061,17 @@ __global__ void __launch_bounds__(128) pitch_viterbi_kernel(const T* __restrict_
 
 constexpr int kMaxPitchFrameLen = 16384;
 
+// Peak inputs of vbx_pitch_with_peaks: silence > 0 turns them on; a null local / global array is computed on the device.
+struct PitchPeaks {
+    double silence = 0.0;
+    const double* local = nullptr;   // [F]
+    const double* global = nullptr;  // [n_segments]
+};
+
 template <typename TIn>
 int launch_pitch(vbx_ctx* ctx, const vbx_frames* fr, double fs, double threshold, double fmin, double fmax, int max_cand,
-                 void* cand_out, int32_t* n_cand_out, uint8_t* status_out, int out_dtype, double* lag_out = nullptr) {
+                 void* cand_out, int32_t* n_cand_out, uint8_t* status_out, int out_dtype, double* lag_out = nullptr,
+                 const PitchPeaks& peaks = PitchPeaks()) {
     const int n = fr->frame_len;
     const double* win = nullptr;
     const double* lagwin = nullptr;
@@ -1108,15 +1137,29 @@ int launch_pitch(vbx_ctx* ctx, const vbx_frames* fr, double fs, double threshold
     if (slab > fr->n_frames) slab = fr->n_frames;
     const size_t y_bytes = al((size_t)slab * n * 8), list_bytes = al((size_t)slab * cap * sizeof(PitchCand)),
                  ref_bytes = al((size_t)slab * cap * sizeof(double2)), range_bytes = al((size_t)slab * sizeof(int2));
-    st = vbx_arena_reserve(ctx, y_bytes + list_bytes + ref_bytes + range_bytes + 256);
+    // peaks the caller did not pass are computed once for the whole batch (the finalize kernel of every slab reads them)
+    const bool with_peaks = peaks.silence > 0.0;
+    const int64_t n_segs = fr->n_frames / P.seg_frames;
+    const size_t local_bytes = (with_peaks && !peaks.local) ? al((size_t)fr->n_frames * sizeof(double)) : 0;
+    const size_t global_bytes = (with_peaks && !peaks.global) ? al((size_t)n_segs * sizeof(double)) : 0;
+    st = vbx_arena_reserve(ctx, y_bytes + list_bytes + ref_bytes + range_bytes + 256 + local_bytes + global_bytes);
     if (st != VBX_OK) return st;
     char* ptr = (char*)ctx->arena;
     P.y = (double*)ptr; ptr += y_bytes;
     P.list = (PitchCand*)ptr; ptr += list_bytes;
     P.refined = (double2*)ptr; ptr += ref_bytes;
     P.range = (int2*)ptr; ptr += range_bytes;
-    P.counter = (unsigned long long*)ptr;
+    P.counter = (unsigned long long*)ptr; ptr += 256;
     VBX_REQUIRE(ctx, (int64_t)slab * cap < 0x7fffffffLL, "pitch slab too large");
+    if (with_peaks) {
+        double* local = local_bytes ? (double*)ptr : nullptr;
+        double* global = global_bytes ? (double*)(ptr + local_bytes) : nullptr;
+        st = vbx_launch_frame_peaks(ctx, fr, local, global);
+        if (st != VBX_OK) return st;
+        P.local_peak = peaks.local ? peaks.local : local;
+        P.global_peak = peaks.global ? peaks.global : global;
+        P.silence = peaks.silence;
+    }
 
     const char* rv = getenv("VBX_PITCH_REFINE");
     const bool refine_v0 = rv && rv[0] == 'v' && rv[1] == '0';  // the first (warp per candidate) version, kept for A/B runs
@@ -1211,6 +1254,83 @@ int vbx_pitch(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate, double
                                     status_out, out_dtype);
     return launch_pitch<float>(ctx, frames, sample_rate, threshold, min_hz, max_hz, max_candidates, cand_out, n_cand_out,
                                status_out, out_dtype);
+}
+
+// vbx_pitch with the reference's local_peak / global_peak honoured (periodic.rs:357; Boersma 1993): the unvoiced candidate's
+// strength is voiceless_strength(local peak of the frame, global peak of its segment) instead of the threshold.
+// silence_threshold == 0 is vbx_pitch itself (no peaks are read or computed).
+int vbx_pitch_with_peaks(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate, double threshold, double silence_threshold,
+                         const double* local_peaks, const double* global_peaks, double min_hz, double max_hz, int32_t max_candidates,
+                         void* cand_out, int32_t* n_cand_out, uint8_t* status_out, int32_t out_dtype) {
+    if (!ctx) return VBX_ERR_BADARG;
+    int st = pitch_check(ctx, frames, max_candidates, cand_out, out_dtype);
+    if (st != VBX_OK) return st;
+    VBX_REQUIRE(ctx, silence_threshold >= 0.0, "silence_threshold must be >= 0");
+    if (frames->n_frames == 0) return VBX_OK;
+    cudaSetDevice(ctx->device);
+    PitchPeaks pk;
+    if (silence_threshold > 0.0) {
+        pk.silence = silence_threshold;
+        pk.local = local_peaks;
+        pk.global = global_peaks;
+    }
+    if (frames->dtype == VBX_I16)
+        return launch_pitch<int16_t>(ctx, frames, sample_rate, threshold, min_hz, max_hz, max_candidates, cand_out, n_cand_out,
+                                     status_out, out_dtype, nullptr, pk);
+    if (frames->dtype == VBX_F64)
+        return launch_pitch<double>(ctx, frames, sample_rate, threshold, min_hz, max_hz, max_candidates, cand_out, n_cand_out,
+                                    status_out, out_dtype, nullptr, pk);
+    return launch_pitch<float>(ctx, frames, sample_rate, threshold, min_hz, max_hz, max_candidates, cand_out, n_cand_out,
+                               status_out, out_dtype, nullptr, pk);
+}
+
+// The host pipeline cuts a segmented view into whole segments, so every chunk computes its segments' global peaks itself.  It
+// cuts a single-segment view into frame ranges, so there the global peak of the whole view is taken here, on the host, before
+// the pipeline starts.  Caller-supplied peaks are uploaded once and every chunk reads its rows.
+int vbx_pitch_with_peaks_host(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate, double threshold, double silence_threshold,
+                              const double* local_peaks, const double* global_peaks, double min_hz, double max_hz,
+                              int32_t max_candidates, void* cand_out, int32_t* n_cand_out, uint8_t* status_out, int32_t out_dtype) {
+    if (!ctx) return VBX_ERR_BADARG;
+    int st = pitch_check(ctx, frames, max_candidates, cand_out, out_dtype);
+    if (st != VBX_OK) return st;
+    VBX_REQUIRE(ctx, silence_threshold >= 0.0, "silence_threshold must be >= 0");
+    if (frames->n_frames == 0) return VBX_OK;
+    cudaSetDevice(ctx->device);
+    const bool with_peaks = silence_threshold > 0.0;
+    const bool segmented = frames->frames_per_segment > 0;
+    const int64_t F = frames->n_frames, n_segs = F / vbx_frames_per_segment(frames);
+    double whole = 0.0;
+    const double* global_src = with_peaks ? global_peaks : nullptr;
+    if (with_peaks && !global_peaks && !segmented) {
+        whole = vbx_host_peak(frames);
+        global_src = &whole;
+    }
+    const double* local_src = with_peaks ? local_peaks : nullptr;
+    const size_t n_local = local_src ? (size_t)F : 0, n_global = global_src ? (size_t)n_segs : 0;
+    double* dev = nullptr;
+    if (n_local + n_global > 0) {
+        VBX_CUDA(ctx, cudaMalloc(&dev, (n_local + n_global) * sizeof(double)));
+        cudaError_t e = cudaSuccess;
+        if (n_local) e = cudaMemcpyAsync(dev, local_src, n_local * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
+        if (e == cudaSuccess && n_global)
+            e = cudaMemcpyAsync(dev + n_local, global_src, n_global * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
+        if (e != cudaSuccess) {
+            cudaStreamSynchronize(ctx->stream);
+            cudaFree(dev);
+            return vbx_fail(ctx, VBX_ERR_CUDA, "peak upload failed: %s", cudaGetErrorString(e));
+        }
+    }
+    const double* d_local = n_local ? dev : nullptr;
+    const double* d_global = n_global ? dev + n_local : nullptr;
+    const size_t pair = (out_dtype == VBX_F64) ? 16 : 8;
+    vbx_host_out outs[3] = {{cand_out, (size_t)max_candidates * pair, nullptr}, {n_cand_out, 4, nullptr}, {status_out, 1, nullptr}};
+    const int rc = vbx_run_chunked(ctx, frames, outs, 3, [&](const vbx_frames* dfr, int64_t f0, int64_t u0, vbx_host_out* o) -> int {
+        return vbx_pitch_with_peaks(ctx, dfr, sample_rate, threshold, silence_threshold, d_local ? d_local + f0 : nullptr,
+                                    d_global ? d_global + u0 : nullptr, min_hz, max_hz, max_candidates, o[0].dev, (int32_t*)o[1].dev,
+                                    (uint8_t*)o[2].dev, out_dtype);
+    }, 0, (size_t)96 << 20);  // the chunking of vbx_pitch_host
+    if (dev) cudaFree(dev);  // the pipeline has drained the stream
+    return rc;
 }
 
 // periodic.rs:403-408: the lag function `self_lag` the candidates are read from — autocorrelate(N), normalize, divide by the

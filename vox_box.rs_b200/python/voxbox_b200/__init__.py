@@ -114,6 +114,9 @@ def _declare(L):
     sig("vbx_pitch", C.c_int, _vp, _frp, _d, _d, _d, _d, _i32, _vp, _vp, _vp, _i32)
     sig("vbx_pitch_host", C.c_int, _vp, _frp, _d, _d, _d, _d, _i32, _vp, _vp, _vp, _i32)
     sig("vbx_pitch_lag_function", C.c_int, _vp, _frp, _vp)
+    sig("vbx_frame_peaks", C.c_int, _vp, _frp, _vp, _vp)
+    sig("vbx_pitch_with_peaks", C.c_int, _vp, _frp, _d, _d, _d, _vp, _vp, _d, _d, _i32, _vp, _vp, _vp, _i32)
+    sig("vbx_pitch_with_peaks_host", C.c_int, _vp, _frp, _d, _d, _d, _vp, _vp, _d, _d, _i32, _vp, _vp, _vp, _i32)
     sig("vbx_pitch_extract", C.c_int, _vp, _vp, _i32, _i64, _i32, _vp)
     sig("vbx_pitch_viterbi", C.c_int, _vp, _vp, _i32, _vp, _i64, _i64, _i32, _d, _d, _d, _d, _vp, _vp)
     sig("vbx_interpolate_sinc", C.c_int, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _i64, _i64, _vp)
@@ -140,6 +143,7 @@ def _declare(L):
     sig("vbx_multi_lpc_host", C.c_int, _vp, _frp, _i32, _vp, _vp, _vp, _i32)
     sig("vbx_multi_find_formants_host", C.c_int, _vp, _frp, C.c_double, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _i32)
     sig("vbx_multi_pitch_host", C.c_int, _vp, _frp, _d, _d, _d, _d, _i32, _vp, _vp, _vp, _i32)
+    sig("vbx_multi_pitch_with_peaks_host", C.c_int, _vp, _frp, _d, _d, _d, _vp, _vp, _d, _d, _i32, _vp, _vp, _vp, _i32)
     sig("vbx_multi_mfcc_host", C.c_int, _vp, _frp, _i32, _i32, _d, _d, _d, _vp, _i32)
     sig("vbx_multi_h2d_bandwidth", C.c_int, _vp, _sz, _i32, _i32, C.POINTER(_d))
 
@@ -527,7 +531,76 @@ def _pitch_lag_function(self, frames):
     return out
 
 
+def _n_segments(n_frames, frames_per_segment):
+    return n_frames // frames_per_segment if frames_per_segment else 1
+
+
+def _host_audio(audio):
+    """Host samples and their vbx dtype: int16 PCM, float64, or anything else as float32."""
+    audio = np.asarray(audio)
+    if audio.dtype == np.int16:
+        return np.ascontiguousarray(audio), I16
+    if audio.dtype == np.float64:
+        return np.ascontiguousarray(audio), F64
+    return np.ascontiguousarray(audio, dtype=np.float32), F32
+
+
+def _host_peaks(a, n):
+    """Caller-supplied peaks for a `_host` twin: None, or a contiguous float64 array of n values."""
+    if a is None:
+        return None
+    a = np.ascontiguousarray(a, dtype=np.float64).reshape(-1)
+    assert a.size == n, (a.size, n)
+    return a
+
+
+def _frame_peaks(self, frames):
+    """Local peak per frame [F] and global peak per segment [n_segments] (max |x| before the window; vbx_frame_peaks) →
+    (local, global) device arrays of float64."""
+    local = self.empty((frames.n_frames,), np.float64)
+    glob = self.empty((_n_segments(frames.n_frames, frames.frames_per_segment),), np.float64)
+    self._check(self.lib.vbx_frame_peaks(self.h, C.byref(frames), local.ptr, glob.ptr), "vbx_frame_peaks")
+    return local, glob
+
+
+def _pitch_with_peaks(self, frames, fs, threshold, silence_threshold, fmin, fmax, max_cand=16, out_dtype=F64, local_peaks=None,
+                      global_peaks=None):
+    """vbx_pitch with Boersma's voiceless strength as the unvoiced candidate's strength (vbx_pitch_with_peaks).  local_peaks [F] /
+    global_peaks [n_segments]: float64 device arrays, or None = computed from the view.  → dict of device arrays as pitch()."""
+    F = frames.n_frames
+    cand = self.empty((F, max_cand, 2), _NP[out_dtype])
+    n = self.empty((F,), np.int32)
+    st = self.empty((F,), np.uint8)
+    self._check(self.lib.vbx_pitch_with_peaks(self.h, C.byref(frames), fs, threshold, silence_threshold,
+                                              local_peaks.ptr if local_peaks is not None else None,
+                                              global_peaks.ptr if global_peaks is not None else None, fmin, fmax, max_cand,
+                                              cand.ptr, n.ptr, st.ptr, out_dtype), "vbx_pitch_with_peaks")
+    return dict(candidates=cand, n_cand=n, status=st)
+
+
+def _pitch_with_peaks_host(self, audio, n_frames, frame_len, stride, window, fs, threshold, silence_threshold, fmin, fmax,
+                           max_cand=16, out_dtype=F64, frames_per_segment=0, segment_stride=0, local_peaks=None,
+                           global_peaks=None):
+    """Host twin of pitch_with_peaks: audio int16 / float32 / float64 samples, peaks host arrays or None."""
+    audio, dt = _host_audio(audio)
+    fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, dt, frames_per_segment, segment_stride)
+    lp = _host_peaks(local_peaks, n_frames)
+    gp = _host_peaks(global_peaks, _n_segments(n_frames, frames_per_segment))
+    cand = np.zeros((n_frames, max_cand, 2), dtype=_NP[out_dtype])
+    n = np.zeros(n_frames, dtype=np.int32)
+    st = np.zeros(n_frames, dtype=np.uint8)
+    self._check(self.lib.vbx_pitch_with_peaks_host(self.h, C.byref(fr), fs, threshold, silence_threshold,
+                                                   lp.ctypes.data if lp is not None else None,
+                                                   gp.ctypes.data if gp is not None else None, fmin, fmax, max_cand,
+                                                   cand.ctypes.data, n.ctypes.data, st.ctypes.data, out_dtype),
+                "vbx_pitch_with_peaks_host")
+    return dict(candidates=cand, n_cand=n, status=st)
+
+
 Context.pitch = _pitch
+Context.frame_peaks = _frame_peaks
+Context.pitch_with_peaks = _pitch_with_peaks
+Context.pitch_with_peaks_host = _pitch_with_peaks_host
 Context.pitch_lag_function = _pitch_lag_function
 Context.pitch_host = _pitch_host
 Context.pitch_extract = _pitch_extract
@@ -784,6 +857,24 @@ class Multi:
         st = np.zeros(n_frames, dtype=np.uint8)
         self._check(self.lib.vbx_multi_pitch_host(self.h, C.byref(fr), fs, threshold, fmin, fmax, max_cand, cand.ctypes.data,
                                                   n.ctypes.data, st.ctypes.data, out_dtype), "vbx_multi_pitch_host")
+        return dict(candidates=cand, n_cand=n, status=st)
+
+    def pitch_with_peaks_host(self, audio, n_frames, frame_len, stride, window, fs, threshold, silence_threshold, fmin, fmax,
+                              max_cand=16, out_dtype=F64, frames_per_segment=0, segment_stride=0, local_peaks=None,
+                              global_peaks=None):
+        """Context.pitch_with_peaks_host sharded over the devices (vbx_multi_pitch_with_peaks_host)."""
+        audio, dt = _host_audio(audio)
+        fr = Context.frames(audio.ctypes.data, n_frames, frame_len, stride, window, dt, frames_per_segment, segment_stride)
+        lp = _host_peaks(local_peaks, n_frames)
+        gp = _host_peaks(global_peaks, _n_segments(n_frames, frames_per_segment))
+        cand = np.zeros((n_frames, max_cand, 2), dtype=_NP[out_dtype])
+        n = np.zeros(n_frames, dtype=np.int32)
+        st = np.zeros(n_frames, dtype=np.uint8)
+        self._check(self.lib.vbx_multi_pitch_with_peaks_host(self.h, C.byref(fr), fs, threshold, silence_threshold,
+                                                             lp.ctypes.data if lp is not None else None,
+                                                             gp.ctypes.data if gp is not None else None, fmin, fmax, max_cand,
+                                                             cand.ctypes.data, n.ctypes.data, st.ctypes.data, out_dtype),
+                    "vbx_multi_pitch_with_peaks_host")
         return dict(candidates=cand, n_cand=n, status=st)
 
     def mfcc_host(self, audio, n_frames, frame_len, stride, window, num_coeffs, f_lo, f_hi, fs, n_keep=None, out_dtype=F64,
