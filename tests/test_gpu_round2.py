@@ -44,22 +44,6 @@ def test_pitch_full_list_parity_10k_frames(oracle):
     assert ds.max() < 1e-6, ds.max()
 
 
-def test_pitch_f32_sweep_still_selectable(oracle, monkeypatch):
-    c = ctx()
-    fs, N, hop = 16000, 640, 160
-    audio = synth.utterance(3, fs, seconds=1.0)
-    d = c.to_device(audio)
-    F = c.n_frames_of(audio.size, N, hop)
-    fr = c.frames(d.ptr, F, N, hop, vb.WINDOW_HANN_SYMMETRIC)
-    a = c.pitch(fr, float(fs), 0.45, 75.0, 600.0, 16)["candidates"].to_host()
-    monkeypatch.setenv("VBX_PITCH_LAG", "f32")
-    c.profile_begin()
-    b = c.pitch(fr, float(fs), 0.45, 75.0, 600.0, 16)["candidates"].to_host()
-    names = c.profile_end()
-    assert "pitch_lag_kernel" in names and "pitch_lag64_kernel" not in names
-    assert np.max(np.abs(a[:, 0, 0] - b[:, 0, 0])) < 0.1
-
-
 # ------------------------------------------------------------------------------------- f64 samples
 def test_f64_samples_every_path(oracle):
     """A frame the caller windowed in f64 (what `for frame in Windower::hanning(..)` yields in the reference) goes in as

@@ -293,10 +293,8 @@ int launch_lpc_roots(vbx_ctx* ctx, const RootsParams& Q, int p, int precision /*
     VBX_REQUIRE(ctx, Q.n_frames <= 0x7fffffffLL, "too many frames for one launch");  // frame indices of the fix-up list are int
     const int64_t grid = (Q.n_frames + kRootsThreads - 1) / kRootsThreads;
     const bool f32 = (precision != 1);
-    // fp32 path without a request for the roots themselves: conjugate-pair deflation (vbx_roots_kernel.cuh); VBX_ROOTS_PAIR=0
-    // keeps the reference's one-root-at-a-time order for A/B runs
-    const char* pe = getenv("VBX_ROOTS_PAIR");
-    if (f32 && !Q.roots_out && !(pe && pe[0] == '0')) {
+    // fp32 path without a request for the roots themselves: conjugate-pair deflation (vbx_roots_kernel.cuh)
+    if (f32 && !Q.roots_out) {
         // 96-thread CTAs (24 KB at order 12) fit next to the persistent LPC kernel's CTA on an SM: ctx->roots_small
         int rthreads = ctx->roots_small ? 96 : kRootsThreads;
         if (const char* e = getenv("VBX_ROOTS_THREADS")) rthreads = atoi(e) == 96 ? 96 : kRootsThreads;
@@ -960,7 +958,6 @@ static int lpc_to_resonances_impl(vbx_ctx* ctx, const void* lpc, int32_t lpc_dty
     Q.status_out = status_out; Q.n_frames = n_frames; Q.fs = sample_rate; Q.lpc_stride = lpc_stride;
     Q.lpc_has_one = lpc_has_leading_one ? 1 : 0; Q.lpc_f64 = (lpc_dtype == VBX_F64); Q.out_f64 = (out_dtype == VBX_F64);
     Q.R = res_slots; Q.strict_im = strict_im ? 1 : 0; Q.polish_steps = 2;
-    if (const char* e = getenv("VBX_ROOTS_POLISH")) Q.polish_steps = atoi(e);  // A/B runs
     Q.work = vbx_work_ptr(ctx);
     Q.in_J = in_J; Q.out_J = out_J; Q.out_j0 = out_j0;
     Q.hard_list = hard_list; Q.hard_count = hard_count; Q.hard_cap = hard_cap; Q.hard_mod = 0; Q.frame_list = nullptr; Q.frame_count = nullptr;
@@ -1078,11 +1075,10 @@ static int estimate_formants_impl(vbx_ctx* ctx, const void* resonances, int32_t 
     T.j_begin = j_begin; T.j_count = j_count;
     const bool side = (stream != ctx->stream);  // side-stream launches are timed as explicit event pairs
     // fused path (per-frame counts known, rows sorted and zero padded): the index-based thread-per-utterance kernel,
-    // when the rows can be staged with 16-byte cp.async chunks.  Arbitrary caller resonances (vbx_estimate_formants),
-    // odd fp32 row lengths, or VBX_TRACKER=warp (A/B runs): the value-based warp-per-utterance kernel.
+    // when the rows can be staged with 16-byte cp.async chunks.  Arbitrary caller resonances (vbx_estimate_formants) or
+    // odd fp32 row lengths: the value-based warp-per-utterance kernel.
     const size_t pair_bytes = (res_dtype == VBX_F64) ? 16 : 8;
     const size_t row_bytes = (size_t)res_slots * pair_bytes;
-    const char* tv = getenv("VBX_TRACKER");
     const bool aligned = (row_bytes % 16 == 0) && ((reinterpret_cast<uintptr_t>(resonances) & 15) == 0);
     const int chunks = (int)(row_bytes / 16);
     // On vbx_find_formants' side stream the tracker runs next to the LPC / roots grids of the following frame chunk.  Spread as
@@ -1099,7 +1095,7 @@ static int estimate_formants_impl(vbx_ctx* ctx, const void* resonances, int32_t 
     }
     while (trk_threads > 32 && (size_t)2 * chunks * trk_threads * 16 > ctx->smem_optin) trk_threads >>= 1;
     const size_t smem = (size_t)2 * chunks * trk_threads * 16;
-    if (nres && aligned && smem <= ctx->smem_optin && !(tv && tv[0] == 'w')) {
+    if (nres && aligned && smem <= ctx->smem_optin) {
         const int64_t grid = (n_segments + trk_threads - 1) / trk_threads;
         VBX_REQUIRE(ctx, grid <= 0x7fffffffLL, "too many segments for one launch");
         if (res_dtype == VBX_F64) {
@@ -1182,13 +1178,10 @@ int vbx_find_formants(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
         if (K > J) K = (int)J;
         if (K < 1) K = 1;
     }
-    cudaStream_t side_stream = ctx->s_side;
-    if (const char* e = getenv("VBX_FORMANT_SIDE"))
-        if (e[0] == '0') side_stream = ctx->stream;
     // chunk boundaries on multiples of 32 frames (the LPC kernels' tile): only an utterance's last tile is partial
     // The last chunk's tracker is the only one nobody overlaps, so the last two chunks are shorter than the others (3/4 and
     // 1/2 of a share): the exposed tail shrinks with the chunk, the chunks before it grow by 10 %.
-    const bool taper = (K >= 4) && !getenv("VBX_FORMANT_UNIFORM");
+    const bool taper = K >= 4;
     auto chunk_begin = [&](int c) -> int64_t {
         if (c <= 0) return 0;
         if (c >= K) return J;
@@ -1207,7 +1200,7 @@ int vbx_find_formants(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
     for (int c = 0; c < K; ++c) Jc_max = std::max<int64_t>(Jc_max, chunk_begin(c + 1) - chunk_begin(c));
     // With overlap, chunk c's roots fix-up runs on the side stream and reads the chunk-local LPC rows, LPC status and fix-up
     // list; chunk c + 1 works on a second set of them, and chunk c + 2 waits for that fix-up before it reuses the first.
-    const bool overlap = track && K > 1 && side_stream != ctx->stream;
+    const bool overlap = track && K > 1;
     const int nbuf = overlap ? 2 : 1;
     // scratch: nbuf × (lpc [segs·Jc_max][p+1] f64) | nbuf × (lpc status [segs·Jc_max]) | status [F] | resonances [F][p] pairs |
     // nres [F] (the last three only when the caller does not ask for them)
@@ -1274,7 +1267,7 @@ int vbx_find_formants(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
                 has_one = 0;
             } else {
                 // the persistent LPC kernel leaves SMs for the co-running tracker: 16 of its warps (512 utterances) per SM
-                ctx->reserve_sms = (track && K > 1 && side_stream != ctx->stream) ? (int)((segs + kTrkThreadsPacked - 1) / kTrkThreadsPacked) : 0;
+                ctx->reserve_sms = overlap ? (int)((segs + kTrkThreadsPacked - 1) / kTrkThreadsPacked) : 0;
                 if (const char* e = getenv("VBX_FORMANT_RESERVE_SMS")) ctx->reserve_sms = atoi(e);
                 st = vbx_lpc(ctx, &sub, p, nullptr, d_lpc, nullptr, VBX_F64);
                 ctx->reserve_sms = 0;
@@ -1297,12 +1290,6 @@ int vbx_find_formants(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
             if (st != VBX_OK) break;
             continue;
         }
-        if (side_stream == ctx->stream) {  // VBX_FORMANT_SIDE=0 (A/B runs): chunks without overlap
-            st = estimate_formants_impl(ctx, d_res, dtype, R, VBX_MAX_RESONANCES, segs, J, d_st, est_inout, n_formants, tracks_out, dtype,
-                                        d_nres, j0, Jc);
-            if (st != VBX_OK) break;
-            continue;
-        }
         // chunk c's resonances are ready -> its tracker steps on the side stream (after chunk c − 1's: same stream)
         cudaEvent_t ready = ctx->ev_side[c & 1];
         if (cudaEventRecord(ready, ctx->stream) != cudaSuccess || cudaStreamWaitEvent(ctx->s_side, ready, 0) != cudaSuccess) {
@@ -1311,7 +1298,7 @@ int vbx_find_formants(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
         }
         // (the last chunk's tracker has the device to itself: small CTAs over all SMs, 0.27 ms instead of 0.69)
         if (fixup_pending) {  // the roots fix-up (rarely any work, but ~0.25 ms of latency when there is) rides the side stream too
-            st = launch_roots_fixup(ctx, Qc, p, side_stream);
+            st = launch_roots_fixup(ctx, Qc, p, ctx->s_side);
             if (st != VBX_OK) break;
             if (cudaEventRecord(ctx->ev_side[2 + b], ctx->s_side) != cudaSuccess) {
                 st = vbx_fail(ctx, VBX_ERR_CUDA, "find_formants: fix-up event failed: %s", cudaGetErrorString(cudaGetLastError()));
@@ -1320,10 +1307,10 @@ int vbx_find_formants(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
             fixup_queued[b] = true;
         }
         st = estimate_formants_impl(ctx, d_res, dtype, R, VBX_MAX_RESONANCES, segs, J, d_st, est_inout, n_formants, tracks_out, dtype,
-                                    d_nres, j0, Jc, side_stream, /*packed=*/c + 1 < K);
+                                    d_nres, j0, Jc, ctx->s_side, /*packed=*/c + 1 < K);
         if (st != VBX_OK) break;
     }
-    if (track && K > 1 && side_stream != ctx->stream) {
+    if (overlap) {
         // join: whatever follows on the context's stream (and vbx_sync) sees the tracks and the final state.  Done on the
         // error path too, so the side stream never runs behind the caller's back.
         cudaEvent_t done = ctx->ev_side[2];

@@ -463,8 +463,7 @@ int launch_mfcc(vbx_ctx* ctx, const vbx_frames* fr, int num_coeffs, int n_keep, 
     }
     // transform precision: fp64 by default (parity first: a band whose sum is ~1 sits on the log10 clamp and an
     // fp32 FFT's ~1e-6 relative error then exceeds the 1e-5 norm-wise bound on quiet frames); fp32 is opt-in
-    bool f32 = ctx->mfcc_fft_f32;
-    if (const char* e = getenv("VBX_MFCC_FFT")) f32 = (e[0] == 'f' && e[1] == '3');
+    const bool f32 = ctx->mfcc_fft_f32;
     // (f64 samples — single windowed frames from the Rust shim's trait calls — take the generic kernel)
     // 400-sample frames, fp64 transform, sample pairs loadable as one word: five lanes per frame (vbx_mfcc_lane5.cuh)
     if constexpr (!std::is_same<TIn, double>::value) {

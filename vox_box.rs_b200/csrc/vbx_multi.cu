@@ -261,15 +261,8 @@ int vbx_multi_find_formants_host(vbx_multi* m, const vbx_frames* frames, double 
 
 int vbx_multi_pitch_host(vbx_multi* m, const vbx_frames* frames, double sample_rate, double threshold, double min_hz, double max_hz,
                          int32_t max_candidates, void* cand_out, int32_t* n_cand_out, uint8_t* status_out, int32_t out_dtype) {
-    if (!m || !frames) return VBX_ERR_BADARG;
-    const size_t pair = (out_dtype == VBX_F64) ? 16 : 8;
-    return run_all(m, [=](int i, vbx_ctx* ctx) -> int {
-        const Shard s = shard_of(frames, m->n, i, true);
-        if (s.fr.n_frames == 0) return VBX_OK;
-        return vbx_pitch_host(ctx, &s.fr, sample_rate, threshold, min_hz, max_hz, max_candidates,
-                              row(cand_out, s.frame0, (size_t)max_candidates * pair), (int32_t*)row(n_cand_out, s.frame0, 4),
-                              (uint8_t*)row(status_out, s.frame0, 1), out_dtype);
-    });
+    return vbx_multi_pitch_with_peaks_host(m, frames, sample_rate, threshold, 0.0, nullptr, nullptr, min_hz, max_hz, max_candidates,
+                                           cand_out, n_cand_out, status_out, out_dtype);
 }
 
 // A single-segment view is split into frame ranges, so its missing global peak is taken over the whole view first, as

@@ -10,24 +10,21 @@
 //   periodic.rs:306-354          Pitch, PitchExtractor               (arg-max: candidates[f][0])
 //
 // Kernel shapes (DESIGN.md §K6/K7):
-//   pitch_lag_kernel      a CTA stages the windowed frames of `fpc` frames in shared memory (fp32,
-//                         4 pad words per 16 so that 8-word chunks at 16-word lane strides are
-//                         bank-conflict free) and computes ALL N lags on the FP32 FMA pipe: a lane
-//                         owns a 16-lag group and walks the frame in 8-sample steps (128 FFMA per 4
-//                         LDS.128), the triangle is balanced by pairing group g with group G-1-g on
-//                         the same lane; fp32 partial sums are folded into fp64 every 8 steps.  A warp
-//                         per frame then normalises (÷ max|r|), divides by the lag window, finds the
-//                         strict local maxima below N/2, interpolates them parabolically, applies the
-//                         (min, max) filter and appends the survivors to a global work list.
-//   pitch_refine_kernel   persistent warps; one warp per candidate runs the reference's Brent
-//                         minimiser (uniform control flow) with the 2(D+1)-term windowed-sinc sum
-//                         split over the lanes, all in fp64.
+//   pitch_lag64_kernel    a CTA stages the windowed frames of `fpc` frames in shared memory as exact
+//                         f64 products x·w and computes ALL N lags on the FP64 pipe: a lane owns a
+//                         16-lag group and walks the frame in 8-sample steps, the triangle is balanced
+//                         by pairing group g with group G-1-g on the same lane (vbx_pitch_lag64.cuh).
+//                         A warp per frame then normalises (÷ max|r|), divides by the lag window, finds
+//                         the strict local maxima below N/2, interpolates them parabolically, applies
+//                         the (min, max) filter and appends the survivors to a global work list.
+//   pitch_refine8q_kernel slots of two lanes run the reference's Brent minimiser over the windowed-sinc
+//                         interpolant, all in fp64; a CTA takes tiles of the work list, sorts each by
+//                         interpolation depth and its slots draw candidates from that order.
 //   pitch_finalize_kernel a warp per frame appends the unvoiced candidate, checks for NaN
 //                         strengths and rank-sorts by strength (stable, descending).  With peaks
 //                         (vbx_pitch_with_peaks) the unvoiced candidate's strength is Boersma's voiceless
 //                         strength of the frame instead of the fixed threshold.
 #include <cmath>
-#include <type_traits>
 
 #include "vbx_internal.cuh"
 #include "vbx_pipeline.cuh"
@@ -79,17 +76,12 @@ __device__ __forceinline__ double voiceless_strength(double local, double global
     return a + (v > 0.0 ? v : 0.0);
 }
 
-__device__ __forceinline__ int chunk_addr(int k) {  // word address of 8-word chunk k: 8k + 4·(8k/16)
-    return 8 * k + 4 * (k >> 1);
-}
-__device__ __forceinline__ int word_addr(int w) { return w + 4 * (w >> 4); }
-
 __device__ __forceinline__ int lag_steps(int n, int g) {  // 8-sample steps lag group g needs
     const int len = n - 16 * g;
     return len > 0 ? (len + 7) >> 3 : 0;
 }
 
-// Per frame (one warp), shared by the fp32 and fp64 sweeps: normalise, ÷ lag window, local maxima, parabolic, filter.
+// Per frame (one warp), after the lag sweep: normalise, ÷ lag window, local maxima, parabolic, filter.
 // `smem` = the CTA's frame buffers (dead after the sweep), `frame_bytes` apart.
 __device__ __forceinline__ void pitch_lag_post(const PitchParams& P, unsigned char* smem, size_t frame_bytes, int64_t f_first, int nf) {
     const int tid = threadIdx.x, nthreads = blockDim.x;
@@ -157,120 +149,7 @@ __device__ __forceinline__ void pitch_lag_post(const PitchParams& P, unsigned ch
     }
 }
 
-// -------------------------------------------------------------------------------------------
 // K6: windowed frame → all-lag autocorrelation → y = (r / max|r|) / lag window → candidates
-// -------------------------------------------------------------------------------------------
-template <typename TIn>
-__global__ void __launch_bounds__(512) pitch_lag_kernel(const PitchParams P) {
-    extern __shared__ __align__(16) float xs_all[];
-    const int tid = threadIdx.x, nthreads = blockDim.x;
-    const int n = P.n;
-    const int64_t f_first = (int64_t)blockIdx.x * P.fpc;                  // slab-local frame index
-    const int nf = (int)min((int64_t)P.fpc, P.n_frames - f_first);
-
-    // ---- stage: xs[q][word_addr(i)] = fp32(x[i]·w[i]) for i < N, zeros up to n16 + 48 -----------------------
-    const int span = P.n16 + 48;
-    for (int q = 0; q < nf; ++q) {
-        const int64_t f = P.frame0 + f_first + q;
-        const int64_t seg = f / P.seg_frames;
-        const TIn* __restrict__ x = reinterpret_cast<const TIn*>(P.base) + seg * P.seg_stride + (f - seg * P.seg_frames) * P.stride;
-        float* xs = xs_all + (size_t)q * P.xs_words;
-        for (int i = tid; i < span; i += nthreads) {
-            float v = 0.f;
-            if (i < n) v = (float)((double)vbx_load_sample<TIn>(x + i) * __ldg(P.win + i));
-            xs[word_addr(i)] = v;
-        }
-    }
-    __syncthreads();
-
-    // ---- lag sweep ------------------------------------------------------------------------------------------
-    const int q = tid / P.lpf, p = tid - q * P.lpf;
-    if (q < nf) {
-        const float* xs = xs_all + (size_t)q * P.xs_words;
-        double* yrow = P.y + (size_t)(f_first + q) * n;
-        const int gA = p, gB = P.G - 1 - p;
-        const int nA = lag_steps(n, gA), nB = (gB > gA) ? lag_steps(n, gB) : 0;
-        const float x0f = xs[0];
-        const double x0d = (double)x0f;  // == the windowed sample 0 rounded to fp32
-        // exact fp64 value of the windowed sample 0 for the reference's fold seed (periodic.rs:284)
-        double x0_exact;
-        {
-            const int64_t f = P.frame0 + f_first + q;
-            const int64_t seg = f / P.seg_frames;
-            const TIn* x = reinterpret_cast<const TIn*>(P.base) + seg * P.seg_stride + (f - seg * P.seg_frames) * P.stride;
-            x0_exact = (double)vbx_load_sample<TIn>(x) * __ldg(P.win);
-        }
-        float acc[16];
-        double racc[16];
-        float4 b0l, b0h, b1l, b1h;
-        int g = gA, left = nA, c = 0, cstep = 1, phase = 0;
-        auto reset = [&]() {
-#pragma unroll
-            for (int j = 0; j < 16; ++j) { acc[j] = 0.f; racc[j] = 0.0; }
-        };
-        auto load_chunk = [&](int k, float4& lo, float4& hi) {
-            const float4* ptr = reinterpret_cast<const float4*>(xs + chunk_addr(k));
-            lo = ptr[0];
-            hi = ptr[1];
-        };
-        auto fold = [&]() {
-#pragma unroll
-            for (int j = 0; j < 16; ++j) { racc[j] += (double)acc[j]; acc[j] = 0.f; }
-        };
-        auto store_group = [&]() {
-            fold();
-#pragma unroll
-            for (int j = 0; j < 16; ++j) {
-                const int lag = 16 * g + j;
-                if (lag < n) {
-                    double r = racc[j];
-                    // r_ref[lag] = x0 + Σ_{i>=1}: remove the i = 0 product, add the seed
-                    if (x0f != 0.f || x0_exact != 0.0) r = r - x0d * (double)xs[word_addr(lag)] + x0_exact;
-                    yrow[lag] = r;
-                }
-            }
-        };
-        reset();
-        if (left == 0) { phase = 2; }
-        load_chunk(c + 2 * g, b0l, b0h);
-        load_chunk(c + 2 * g + 1, b1l, b1h);
-        const int zero_chunk = (P.n16 + 16) >> 3;  // a chunk of zeros (words n16+16 .. n16+23)
-        for (int s = 0; s < P.T; ++s) {
-            if (left == 0 && phase < 2) {
-                store_group();
-                if (phase == 0 && nB > 0) {
-                    phase = 1; g = gB; left = nB; c = 0;
-                    reset();
-                    load_chunk(2 * g, b0l, b0h);
-                    load_chunk(2 * g + 1, b1l, b1h);
-                } else {
-                    phase = 2;
-                }
-            }
-            if (phase == 2) { c = zero_chunk; cstep = 0; g = 0; left = 0x3fffffff; }
-            float4 al, ah, b2l, b2h;
-            load_chunk(c, al, ah);
-            load_chunk(c + 2 * g + 2, b2l, b2h);
-            const float a[8] = {al.x, al.y, al.z, al.w, ah.x, ah.y, ah.z, ah.w};
-            const float bw[24] = {b0l.x, b0l.y, b0l.z, b0l.w, b0h.x, b0h.y, b0h.z, b0h.w, b1l.x, b1l.y, b1l.z, b1l.w,
-                                  b1h.x, b1h.y, b1h.z, b1h.w, b2l.x, b2l.y, b2l.z, b2l.w, b2h.x, b2h.y, b2h.z, b2h.w};
-#pragma unroll
-            for (int ii = 0; ii < 8; ++ii) {
-#pragma unroll
-                for (int jj = 0; jj < 16; ++jj) acc[jj] = fmaf(a[ii], bw[ii + jj], acc[jj]);
-            }
-            b0l = b1l; b0h = b1h; b1l = b2l; b1h = b2h;
-            c += cstep;
-            --left;
-            if ((s & 7) == 7) fold();
-        }
-        if (phase < 2) store_group();
-    }
-    __syncthreads();
-
-    pitch_lag_post(P, reinterpret_cast<unsigned char*>(xs_all), (size_t)P.xs_words * sizeof(float), f_first, nf);
-}
-
 #include "vbx_pitch_lag64.cuh"
 
 // -------------------------------------------------------------------------------------------
@@ -402,261 +281,39 @@ __device__ void improve_extremum_warp(const double* __restrict__ y, long long y_
     *ymid = fx;
 }
 
-// K7: persistent warps over the work list
-__global__ void __launch_bounds__(256) pitch_refine_kernel(const PitchParams P) {
-    const int lane = threadIdx.x & 31;
-    const long long warp_global = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
-    const long long total = (long long)*P.counter;
-    const long long offset = -(long long)P.ixmax - 1;
-    const long long nx = (long long)P.ixmax - offset;
-    for (long long e = warp_global; e < total; e += n_warps) {
-        const PitchCand c = P.list[e];
-        const double* y = P.y + (size_t)c.frame * P.n;
-        double xmid, ymid;
-        improve_extremum_warp(y, 2LL * P.n, P.n, offset, nx, c.n, 2, 1200, true, &xmid, &ymid, lane);
-        xmid += (double)offset;
-        if (ymid > 1.) ymid = 1. / ymid;
-        if (lane == 0) P.refined[e] = make_double2(P.fs / xmid, ymid);
-    }
-}
-
-// K7 (v1): four candidates per warp, 8 lanes each, in lockstep.
-//
-// Lane ℓ8 of a slot owns the terms n ≡ ℓ8 (mod 8) of both sides of interpolate_sinc's sum, so that per term
-//   * (−1)ⁿ is a per-lane constant (stride 8 is even),
-//   * the Hann factor ½ + ½cos(π(φ+n)/(φ+D)) advances by a three-term recurrence in cos 8δ, δ = π/(φ+D),
-//   * the two sides share one reciprocal: y_l·h_l/t_l + y_r·h_r/t_r = (y_l·h_l·t_r + y_r·h_r·t_l)/(t_l·t_r).
-// The four slots of a warp hold consecutive work-list entries (same frame, ascending lag, hence similar depth D)
-// and run Brent in lockstep; the term loop runs to the largest D of the four, shorter slots are masked.
-// Brent's state is replicated in the 8 lanes of a slot (identical arithmetic ⇒ identical values), the only
-// cross-lane traffic is the 3-step butterfly that sums the 8 partial sums.
 __device__ __forceinline__ double rcp_pos(double x) {  // 1/x for normal positive x: MUFU seed + one third-order step
     double r;
     asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(x));
     const double e = fma(-x, r, 1.0);   // seed error, <= 1e-6 relative (tools/cuda/rcp_test.cu)
     return fma(r, fma(e, e, e), r);     // r·(1 + e + e²): error e³, i.e. below one ulp
 }
-
 // (A single Newton step would leave 1e-12 relative error and that already moves some weak candidates' Brent paths by
 // > 0.1 Hz in tests/test_gpu_pitch.py; the third-order step costs the same three DFMAs as one-and-a-half Newton steps.)
-constexpr int kRefineTile = 256;
 
-__global__ void __launch_bounds__(128) pitch_refine8_kernel(const PitchParams P) {
-    const unsigned FULL = 0xffffffffu;
-    const int lane = threadIdx.x & 31, sub = lane >> 3, l8 = lane & 7;
-    const int warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
-    const long long total = (long long)*P.counter;
-    const int N = P.n;
-    // A CTA takes tiles of kRefineTile consecutive work-list entries (about ten frames) and walks each tile in order of
-    // the start abscissa, i.e. of the interpolation depth D: the four slots of a warp then run term loops of nearly the
-    // same length (the list order — ascending lag inside a frame — leaves 19 % of the lanes of the term loop idle, a
-    // sorted tile 3 %).  Results do not depend on the grouping: every slot's arithmetic is its own.
-    __shared__ float s_key[kRefineTile];
-    __shared__ unsigned short s_ord[kRefineTile];
-    const int offset = -P.ixmax - 1;
-    const int nx = P.ixmax - offset;
-    const int ylen = 2 * N;
-    const double golden = 1. - 0.6180339887498948482045868343656381177203091798057628621;
-    const double EPS = 2.220446049250313e-16, sqrt_epsilon = 1.4901161193847656e-08, tol = 1e-10;
-    const double sgn = (l8 & 1) ? -1.0 : 1.0;
-    const double qnan = __longlong_as_double(0x7ff8000000000000LL);
-
-    for (long long tile0 = (long long)blockIdx.x * kRefineTile; tile0 < total; tile0 += (long long)gridDim.x * kRefineTile) {
-    const int tcnt = (int)min((long long)kRefineTile, total - tile0);
-    __syncthreads();  // the previous tile's order is no longer read
-    for (int i = threadIdx.x; i < tcnt; i += blockDim.x) s_key[i] = (float)P.list[tile0 + i].n;
-    __syncthreads();
-    for (int i = threadIdx.x; i < tcnt; i += blockDim.x) {
-        const float ki = s_key[i];
-        int rank = 0;
-        for (int j = 0; j < tcnt; ++j) {
-            const float kj = s_key[j];
-            rank += (kj < ki || (kj == ki && j < i)) ? 1 : 0;
-        }
-        s_ord[rank] = (unsigned short)i;
-    }
-    __syncthreads();
-    for (int g = warp; 4 * g < tcnt; g += nwarps) {
-        const int slot = 4 * g + sub;
-        const bool valid = slot < tcnt;
-        const long long e = tile0 + (valid ? (int)s_ord[slot] : 0);
-        PitchCand cd;
-        cd.frame = 0; cd.k = 0; cd.n = 0.0;
-        if (valid) cd = P.list[e];
-        const double* __restrict__ y = P.y + (size_t)cd.frame * N;
-        auto yat = [&](int idx) -> double { return (idx >= 0 && idx < N) ? __ldg(y + idx) : 0.0; };  // zero-extended to 2N
-        // improve_extremum's early returns (periodic.rs:193-194)
-        bool done = !valid;
-        double rx = 0., ry = 0.;
-        const double ixmid = cd.n;
-        if (valid) {
-            if (ixmid == 0.) { rx = 0.; ry = yat(0); done = true; }
-            else if (ixmid >= (double)nx) { rx = (double)nx; ry = yat(nx - 1); done = true; }
-        }
-        // brent_maximize(f, (ixmid−1, ixmid+1), tol = 1e-10)
-        double a = ixmid - 1., b = ixmid + 1.;
-        double v = a + golden * (b - a), w = v, x = v, fv = 0., fw = 0., fx = 0.;
-        double t = v;
-        int iter = 0;  // 0: the initial evaluation is pending
-        while (!__all_sync(FULL, done)) {
-            // ---- interpolate_sinc(y, offset, nx, t, 1200): per-slot setup ----------------------------------------
-            const double fl = floor(t);
-            const int nl = (fl > 0.0) ? (int)fmin(fl, 1.0e9) : 0;
-            const int nr = nl + 1;
-            const double phil = t - (double)nl, phir = 1. - phil;
-            bool special = done;
-            double sval = 0.;
-            int D = -1;
-            if (!done) {
-                if (t > (double)nx) { special = true; const int i = offset + nx - 1; sval = (i < 0 || i >= ylen) ? qnan : yat(i); }
-                else if (t < 0.) { special = true; sval = yat(0); }
-                else if (fabs(t - (double)nl) < 1.0e-10) { special = true; const int i = offset + nl; sval = (i < 0 || i >= ylen) ? qnan : yat(i); }
-                else if (fabs(t - (double)nr) < 1.0e-10) { special = true; const int i = offset + nr; sval = (i < 0 || i >= ylen) ? qnan : yat(i); }
-                else {
-                    int md = 1200;
-                    if (offset + nr < md) md = (offset + nr < 0) ? 0 : offset + nr;
-                    if (offset + nl + md >= nx) md = nx - offset + nl - 1;
-                    D = md;
-                }
-            }
-            const bool act = !special;
-            const double pl = act ? phil : 0.5, pr = act ? phir : 0.5;
-            const double Dd = (double)(D < 0 ? 0 : D);
-            const double inv_l = rcp_pos(pl + Dd), inv_r = rcp_pos(pr + Dd);
-            // the three slot-uniform trigonometric values share ONE sincospi call: lane 0 of the slot takes πφ (→ sin πφ),
-            // lane 1 takes 8δ_l, lane 2 takes 8δ_r; five shuffles hand the results to the other lanes of the slot
-            double su, cu;
-            sincospi(l8 == 0 ? pl : (l8 == 1 ? 8.0 * inv_l : (l8 == 2 ? 8.0 * inv_r : 0.0)), &su, &cu);
-            const int sb = lane & 24;
-            const double s0 = __shfl_sync(FULL, su, sb);
-            const double S8l = __shfl_sync(FULL, su, sb + 1), C8l = __shfl_sync(FULL, cu, sb + 1);
-            const double S8r = __shfl_sync(FULL, su, sb + 2), C8r = __shfl_sync(FULL, cu, sb + 2);
-            double sl, cl, sr, cr;
-            double tl = pl + (double)l8, tr = pr + (double)l8;
-            sincospi(tl * inv_l, &sl, &cl);
-            sincospi(tr * inv_r, &sr, &cr);
-            // Hann factor h_j = ½ + ½cos(θ0 + 8δ·j) by the three-term recurrence h_{j+1} = K·h_j − h_{j−1} + (1 − K/2),
-            // K = 2cos 8δ (error growth ~j²·ε, j <= 150), started from h_0 and h_{−1} = ½ + ½cos(θ0 − 8δ)
-            double hl = fma(0.5, cl, 0.5), hlp = fma(0.5, fma(cl, C8l, sl * S8l), 0.5);
-            double hr = fma(0.5, cr, 0.5), hrp = fma(0.5, fma(cr, C8r, sr * S8r), 0.5);
-            const double Kl = 2.0 * C8l, Kr = 2.0 * C8r, Cl = 1.0 - C8l, Cr = 1.0 - C8r;
-            const int L = offset + nr, R = offset + nl;
-            const int Dmax = __reduce_max_sync(FULL, D);
-            double acc = 0.;
-            // Left terms read y[L − n] (>= 0 because D <= L), right terms y[R + n]; beyond N the zero extension
-            // contributes nothing.  When every active slot has 0 <= R and L < N (always, for candidates at positive
-            // lags) the bounds collapse into one per-side depth and the loads walk two pointers.
-            const bool plain = !act || (R >= 0 && L < N);
-            if (__all_sync(FULL, plain)) {
-                const int Dl = D, Dr = min(D, N - 1 - R);
-                const double* __restrict__ ql = y + (act ? L - l8 : 0);
-                const double* __restrict__ qr = y + (act ? R + l8 : 0);
-                for (int n = l8; n <= Dmax; n += 8) {
-                    const double yl = (n <= Dl) ? __ldg(ql) : 0.0;
-                    const double yr = (n <= Dr) ? __ldg(qr) : 0.0;
-                    ql -= 8;
-                    qr += 8;
-                    const double num = fma(yl * hl, tr, (yr * hr) * tl);
-                    acc = fma(num, rcp_pos(tl * tr), acc);
-                    const double nhl = fma(Kl, hl, Cl - hlp), nhr = fma(Kr, hr, Cr - hrp);
-                    hlp = hl; hl = nhl; hrp = hr; hr = nhr;
-                    tl += 8.0; tr += 8.0;
-                }
-            } else {
-                for (int n = l8; n <= Dmax; n += 8) {
-                    const bool on = (n <= D);
-                    int il = L - n;
-                    il = il < 0 ? 0 : il;
-                    int ir = R + n;
-                    ir = ir < 0 ? 0 : ir;
-                    const double yl = (on && il < N) ? __ldg(y + il) : 0.0;
-                    const double yr = (on && ir < N) ? __ldg(y + ir) : 0.0;
-                    const double num = fma(yl * hl, tr, (yr * hr) * tl);
-                    acc = fma(num, rcp_pos(tl * tr), acc);
-                    // advance: t += 8, Hann factors one recurrence step
-                    const double nhl = fma(Kl, hl, Cl - hlp), nhr = fma(Kr, hr, Cr - hrp);
-                    hlp = hl; hl = nhl; hrp = hr; hr = nhr;
-                    tl += 8.0; tr += 8.0;
-                }
-            }
-            acc *= sgn;
-            acc += __shfl_xor_sync(FULL, acc, 1);
-            acc += __shfl_xor_sync(FULL, acc, 2);
-            acc += __shfl_xor_sync(FULL, acc, 4);
-            const double ft = special ? sval : acc * (s0 * (1.0 / kPi));
-            // ---- Brent update (periodic.rs:121-186) ---------------------------------------------------------------------
-            if (!done) {
-                if (iter == 0) {
-                    fv = ft; fx = ft; fw = ft;
-                    iter = 1;
-                } else {
-                    if (ft <= fx) {
-                        if (t < x) b = x; else a = x;
-                        v = w; w = x; x = t;
-                        fv = fw; fw = fx; fx = ft;
-                    } else {
-                        if (t < x) a = t; else b = t;
-                        if (ft <= fw || fabs(w - x) < EPS) {
-                            v = w; w = t;
-                            fv = fw; fw = ft;
-                        } else if (ft <= fv || fabs(v - x) < EPS || fabs(v - w) < EPS) {
-                            v = t;
-                            fv = ft;
-                        }
-                    }
-                    ++iter;
-                }
-                if (iter > 60) {
-                    done = true; rx = x; ry = fx;
-                } else {
-                    const double range = b - a, middle_range = (a + b) * 0.5;
-                    const double tol_act = sqrt_epsilon * fabs(x) + tol / 3.;
-                    if (fabs(x - middle_range) + range * 0.5 <= 2. * tol_act) {
-                        done = true; rx = x; ry = fx;
-                    } else {
-                        double new_step = (x < middle_range) ? golden * (b - x) : golden * (a - x);
-                        if (fabs(x - w) >= tol_act) {
-                            const double tt = (x - w) * (fx - fv);
-                            double q = (x - v) * (fx - fw);
-                            double p = (x - v) * q - (x - w) * tt;
-                            q = 2. * q - tt;
-                            if (q > 0.) p = -p; else q = -q;
-                            if (fabs(p) < fabs(new_step * q) && p > q * (a - x + 2. * tol_act) && p < q * (b - x - 2. * tol_act))
-                                new_step = p / q;
-                        }
-                        if (fabs(new_step) < tol_act) new_step = (new_step > 0.) ? tol_act : -tol_act;
-                        t = x + new_step;
-                    }
-                }
-            }
-        }
-        if (valid && l8 == 0) {
-            double xmid = rx + (double)offset, ymid = ry;
-            if (ymid > 1.) ymid = 1. / ymid;
-            P.refined[e] = make_double2(P.fs / xmid, ymid);
-        }
-    }
-    }
-}
-
-// K7 (v2): the same slots, fed from a queue.  Brent needs a different number of evaluations for every candidate (about
-// 12 to 40), so in the lockstep version above a warp idles a finished slot until the slowest of its four is done.  Here
-// every slot draws its next candidate from the tile's sorted order (a shared-memory cursor) as soon as it finishes:
-// the warp stays in lockstep only over single evaluations of the interpolant.
-#ifndef VBX_REFINE_MINB
-#define VBX_REFINE_MINB 1
-#endif
-template <int LS, int TILE>  // lanes per slot: 8, 4 or 2 (4, 8 or 16 candidates per warp); TILE = work-list entries per tile
-__global__ void __launch_bounds__(128, VBX_REFINE_MINB) pitch_refine8q_kernel(const PitchParams P) {
-    static_assert(LS == 8 || LS == 4 || LS == 2, "an even term stride keeps (-1)^n a per-lane constant");
+// K7: Brent over the windowed-sinc interpolant, one work-list entry per slot of LS lanes, 32 / LS slots per warp.
+//
+// Lane ℓ of a slot owns the terms n ≡ ℓ (mod LS) of both sides of interpolate_sinc's sum, so that per term
+//   * (−1)ⁿ is a per-lane constant (LS is even),
+//   * the Hann factor ½ + ½cos(π(φ+n)/(φ+D)) advances by a three-term recurrence in cos LS·δ, δ = π/(φ+D),
+//   * the two sides share one reciprocal: y_l·h_l/t_l + y_r·h_r/t_r = (y_l·h_l·t_r + y_r·h_r·t_l)/(t_l·t_r).
+// Brent's state is replicated in the lanes of a slot (identical arithmetic ⇒ identical values); the only cross-lane
+// traffic is the shuffle that sums the partial sums.  Brent needs a different number of evaluations for every candidate
+// (about 12 to 40), so every slot draws its next candidate from the tile's sorted order (a shared-memory cursor) as soon
+// as it finishes: the warp stays in lockstep only over single evaluations of the interpolant.
+__global__ void __launch_bounds__(128, 1) pitch_refine8q_kernel(const PitchParams P) {
+    // Every evaluation of the interpolant pays ~300 instructions of setup (three sincospi, two reciprocals, the Brent
+    // update) whatever the slot width, so narrow slots amortise it best: 8 lanes 5.70e6 frames/s on C4, 4 lanes 6.85e6,
+    // 2 lanes 7.06e6 (results identical: a slot's arithmetic is its own).  Tiles larger than 256 entries were slower for
+    // every width: a tile's ~10 lag-function rows stay in L1, 40 rows do not.
+    constexpr int LS = 2;       // lanes per slot
+    constexpr int TILE = 256;   // work-list entries per tile
     constexpr int SLOT_MASK = 32 - LS;  // lane & SLOT_MASK = the slot's first lane
     const unsigned FULL = 0xffffffffu;
-    const int lane = threadIdx.x & 31, l8 = lane & (LS - 1);
+    const int lane = threadIdx.x & 31, li = lane & (LS - 1);
     const long long total = (long long)*P.counter;
     const int N = P.n;
     // A CTA takes tiles of TILE consecutive work-list entries (about ten frames) and walks each tile in order of
-    // the start abscissa, i.e. of the interpolation depth D: the four slots of a warp then run term loops of nearly the
+    // the start abscissa, i.e. of the interpolation depth D: the slots of a warp then run term loops of nearly the
     // same length (the list order — ascending lag inside a frame — leaves 19 % of the lanes of the term loop idle, a
     // sorted tile 3 %).  Results do not depend on the grouping: every slot's arithmetic is its own.
     __shared__ float s_key[TILE];
@@ -668,7 +325,7 @@ __global__ void __launch_bounds__(128, VBX_REFINE_MINB) pitch_refine8q_kernel(co
     const int ylen = 2 * N;
     const double golden = 1. - 0.6180339887498948482045868343656381177203091798057628621;
     const double EPS = 2.220446049250313e-16, sqrt_epsilon = 1.4901161193847656e-08, tol = 1e-10;
-    const double sgn = (l8 & 1) ? -1.0 : 1.0;
+    const double sgn = (li & 1) ? -1.0 : 1.0;
     const double qnan = __longlong_as_double(0x7ff8000000000000LL);
     unsigned work_terms = 0, work_evals = 0;  // executed term-loop iterations / evaluation rounds of this warp
 
@@ -702,7 +359,7 @@ __global__ void __launch_bounds__(128, VBX_REFINE_MINB) pitch_refine8q_kernel(co
         s_ord[rank] = (unsigned short)i;
     }
     __syncthreads();
-    // slot state (replicated in the 8 lanes of a slot)
+    // slot state (replicated in the lanes of a slot)
     bool have = false, dry = false;     // have: a candidate is being refined; dry: the tile's queue is exhausted
     long long e = 0;
     const double* __restrict__ y = P.y;
@@ -715,7 +372,7 @@ __global__ void __launch_bounds__(128, VBX_REFINE_MINB) pitch_refine8q_kernel(co
             // ---- free slots draw the next candidate of the tile ---------------------------------------------------------
             const bool want = !have && !dry;
             int qi = -1;
-            if (want && l8 == 0) qi = atomicAdd(&s_next, 1);
+            if (want && li == 0) qi = atomicAdd(&s_next, 1);
             qi = __shfl_sync(FULL, qi, lane & SLOT_MASK);
             if (want) {
                 if (qi >= tcnt) {
@@ -727,7 +384,7 @@ __global__ void __launch_bounds__(128, VBX_REFINE_MINB) pitch_refine8q_kernel(co
                     const double ixmid = cd.n;
                     // improve_extremum's early returns (periodic.rs:193-194)
                     if (ixmid == 0. || ixmid >= (double)nx) {
-                        if (l8 == 0) {
+                        if (li == 0) {
                             double ymid = (ixmid == 0.) ? yat(0) : yat(nx - 1);
                             const double xmid = ((ixmid == 0.) ? 0. : (double)nx) + (double)offset;
                             if (ymid > 1.) ymid = 1. / ymid;
@@ -773,29 +430,24 @@ __global__ void __launch_bounds__(128, VBX_REFINE_MINB) pitch_refine8q_kernel(co
             const double pl = act ? phil : 0.5, pr = act ? phir : 0.5;
             const double Dd = (double)(D < 0 ? 0 : D);
             const double inv_l = rcp_pos(pl + Dd), inv_r = rcp_pos(pr + Dd);
-            // the three slot-uniform trigonometric values share ONE sincospi call: lane 0 of the slot takes πφ (→ sin πφ),
-            // lane 1 takes 8δ_l, lane 2 takes 8δ_r; five shuffles hand the results to the other lanes of the slot
+            // two of the three slot-uniform trigonometric values share ONE sincospi call: lane 0 of the slot takes πφ
+            // (→ sin πφ), lane 1 takes LS·δ_l; three shuffles hand the results to the other lane of the slot
             double su, cu;
-            sincospi(l8 == 0 ? pl : (l8 == 1 ? (double)LS * inv_l : (l8 == 2 ? (double)LS * inv_r : 0.0)), &su, &cu);
+            sincospi(li == 0 ? pl : (li == 1 ? (double)LS * inv_l : 0.0), &su, &cu);
             const int sb = lane & SLOT_MASK;
             const double s0 = __shfl_sync(FULL, su, sb);
-            const double S8l = __shfl_sync(FULL, su, sb + 1), C8l = __shfl_sync(FULL, cu, sb + 1);
-            double S8r, C8r;
-            if (LS >= 4) {
-                S8r = __shfl_sync(FULL, su, sb + 2);
-                C8r = __shfl_sync(FULL, cu, sb + 2);
-            } else {  // two lanes per slot: the third slot-uniform angle gets its own call
-                sincospi((double)LS * inv_r, &S8r, &C8r);
-            }
+            const double Sdl = __shfl_sync(FULL, su, sb + 1), Cdl = __shfl_sync(FULL, cu, sb + 1);
+            double Sdr, Cdr;
+            sincospi((double)LS * inv_r, &Sdr, &Cdr);
             double sl, cl, sr, cr;
-            double tl = pl + (double)l8, tr = pr + (double)l8;
+            double tl = pl + (double)li, tr = pr + (double)li;
             sincospi(tl * inv_l, &sl, &cl);
             sincospi(tr * inv_r, &sr, &cr);
-            // Hann factor h_j = ½ + ½cos(θ0 + 8δ·j) by the three-term recurrence h_{j+1} = K·h_j − h_{j−1} + (1 − K/2),
-            // K = 2cos 8δ (error growth ~j²·ε, j <= 150), started from h_0 and h_{−1} = ½ + ½cos(θ0 − 8δ)
-            double hl = fma(0.5, cl, 0.5), hlp = fma(0.5, fma(cl, C8l, sl * S8l), 0.5);
-            double hr = fma(0.5, cr, 0.5), hrp = fma(0.5, fma(cr, C8r, sr * S8r), 0.5);
-            const double Kl = 2.0 * C8l, Kr = 2.0 * C8r, Cl = 1.0 - C8l, Cr = 1.0 - C8r;
+            // Hann factor h_j = ½ + ½cos(θ0 + LS·δ·j) by the three-term recurrence h_{j+1} = K·h_j − h_{j−1} + (1 − K/2),
+            // K = 2cos LS·δ (error growth ~j²·ε, j <= 600), started from h_0 and h_{−1} = ½ + ½cos(θ0 − LS·δ)
+            double hl = fma(0.5, cl, 0.5), hlp = fma(0.5, fma(cl, Cdl, sl * Sdl), 0.5);
+            double hr = fma(0.5, cr, 0.5), hrp = fma(0.5, fma(cr, Cdr, sr * Sdr), 0.5);
+            const double Kl = 2.0 * Cdl, Kr = 2.0 * Cdr, Cl = 1.0 - Cdl, Cr = 1.0 - Cdr;
             const int L = offset + nr, R = offset + nl;
             const int Dmax = __reduce_max_sync(FULL, D);
             work_terms += (unsigned)((Dmax >= 0 ? Dmax : -1) + LS) / LS;
@@ -807,9 +459,9 @@ __global__ void __launch_bounds__(128, VBX_REFINE_MINB) pitch_refine8q_kernel(co
             const bool plain = !act || (R >= 0 && L < N);
             if (__all_sync(FULL, plain)) {
                 const int Dl = D, Dr = min(D, N - 1 - R);
-                const double* __restrict__ ql = y + (act ? L - l8 : 0);
-                const double* __restrict__ qr = y + (act ? R + l8 : 0);
-                for (int n = l8; n <= Dmax; n += LS) {
+                const double* __restrict__ ql = y + (act ? L - li : 0);
+                const double* __restrict__ qr = y + (act ? R + li : 0);
+                for (int n = li; n <= Dmax; n += LS) {
                     const double yl = (n <= Dl) ? __ldg(ql) : 0.0;
                     const double yr = (n <= Dr) ? __ldg(qr) : 0.0;
                     ql -= LS;
@@ -821,7 +473,7 @@ __global__ void __launch_bounds__(128, VBX_REFINE_MINB) pitch_refine8q_kernel(co
                     tl += (double)LS; tr += (double)LS;
                 }
             } else {
-                for (int n = l8; n <= Dmax; n += LS) {
+                for (int n = li; n <= Dmax; n += LS) {
                     const bool on = (n <= D);
                     int il = L - n;
                     il = il < 0 ? 0 : il;
@@ -831,7 +483,7 @@ __global__ void __launch_bounds__(128, VBX_REFINE_MINB) pitch_refine8q_kernel(co
                     const double yr = (on && ir < N) ? __ldg(y + ir) : 0.0;
                     const double num = fma(yl * hl, tr, (yr * hr) * tl);
                     acc = fma(num, rcp_pos(tl * tr), acc);
-                    // advance: t += 8, Hann factors one recurrence step
+                    // advance: t += LS, Hann factors one recurrence step
                     const double nhl = fma(Kl, hl, Cl - hlp), nhr = fma(Kr, hr, Cr - hrp);
                     hlp = hl; hl = nhl; hrp = hr; hr = nhr;
                     tl += (double)LS; tr += (double)LS;
@@ -839,8 +491,6 @@ __global__ void __launch_bounds__(128, VBX_REFINE_MINB) pitch_refine8q_kernel(co
             }
             acc *= sgn;
             acc += __shfl_xor_sync(FULL, acc, 1);
-            if (LS >= 4) acc += __shfl_xor_sync(FULL, acc, 2);
-            if (LS == 8) acc += __shfl_xor_sync(FULL, acc, 4);
             const double ft = special ? sval : acc * (s0 * (1.0 / kPi));
             // ---- Brent update (periodic.rs:121-186) ---------------------------------------------------------------------
             if (!done) {
@@ -889,7 +539,7 @@ __global__ void __launch_bounds__(128, VBX_REFINE_MINB) pitch_refine8q_kernel(co
             }
         }
             if (have && done) {
-                if (l8 == 0) {
+                if (li == 0) {
                     double xmid = rx + (double)offset, ymid = ry;
                     if (ymid > 1.) ymid = 1. / ymid;
                     P.refined[e] = make_double2(P.fs / xmid, ymid);
@@ -1070,8 +720,7 @@ struct PitchPeaks {
 
 template <typename TIn>
 int launch_pitch(vbx_ctx* ctx, const vbx_frames* fr, double fs, double threshold, double fmin, double fmax, int max_cand,
-                 void* cand_out, int32_t* n_cand_out, uint8_t* status_out, int out_dtype, double* lag_out = nullptr,
-                 const PitchPeaks& peaks = PitchPeaks()) {
+                 void* cand_out, int32_t* n_cand_out, uint8_t* status_out, int out_dtype, double* lag_out, const PitchPeaks& peaks) {
     const int n = fr->frame_len;
     const double* win = nullptr;
     const double* lagwin = nullptr;
@@ -1100,31 +749,21 @@ int launch_pitch(vbx_ctx* ctx, const vbx_frames* fr, double fs, double threshold
         if (t > T) T = t;
     }
     P.T = T;
-    // The sweep runs in fp64 (exact x·w products, one DFMA per lag product: vbx_pitch_lag64.cuh); VBX_PITCH_LAG=f32 selects
-    // the fp32-FMA sweep with fp64 folding (≈ 3e-8·r[0] in the lag function: enough for the top candidate, not for the
-    // weak entries of the list) for A/B runs.
-    const char* lv = getenv("VBX_PITCH_LAG");
-    const bool lag_f32 = lv && lv[0] == 'f' && lv[1] == '3' && !std::is_same<TIn, double>::value;
-    // frame buffer: fp32 with 4 pad words per 16, or f64 with 2 pad doubles per 16 (xs_words counts elements)
-    P.xs_words = lag_f32 ? ((P.n16 + 48) * 5) / 4 : ((P.n16 + 48) * 9) / 8;
+    // frame buffer: f64 with 2 pad doubles per 16 (xs_words counts doubles)
+    P.xs_words = ((P.n16 + 48) * 9) / 8;
     // frames per CTA: fill ~160 threads, bounded by shared memory (<= 56 KB so that 4 CTAs fit an SM)
     int fpc = 160 / P.lpf;
     if (fpc < 1) fpc = 1;
-    const size_t frame_bytes = (size_t)P.xs_words * (lag_f32 ? sizeof(float) : sizeof(double));
+    const size_t frame_bytes = (size_t)P.xs_words * sizeof(double);
     while (fpc > 1 && fpc * frame_bytes > 56 * 1024) --fpc;
     P.fpc = fpc;
     int threads = ((fpc * P.lpf + 31) / 32) * 32;
     if (threads < 64) threads = 64;
     const size_t smem = fpc * frame_bytes;
-    VBX_REQUIRE(ctx, smem <= ctx->smem_optin && threads <= (lag_f32 ? 512 : 256), "frame_len %d does not fit the pitch kernel", n);
-    if constexpr (!std::is_same<TIn, double>::value) {
-        if (lag_f32) VBX_CUDA(ctx, cudaFuncSetAttribute(pitch_lag_kernel<TIn>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    }
+    VBX_REQUIRE(ctx, smem <= ctx->smem_optin && threads <= 256, "frame_len %d does not fit the pitch kernel", n);
     const bool lag_small = threads <= 160;
-    if (!lag_f32) {
-        if (lag_small) VBX_CUDA(ctx, cudaFuncSetAttribute(pitch_lag64_kernel<TIn, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        else VBX_CUDA(ctx, cudaFuncSetAttribute(pitch_lag64_kernel<TIn, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    }
+    if (lag_small) VBX_CUDA(ctx, cudaFuncSetAttribute(pitch_lag64_kernel<TIn, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    else VBX_CUDA(ctx, cudaFuncSetAttribute(pitch_lag64_kernel<TIn, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 
     // scratch per frame: y [N] f64 + worst-case candidate capacity (every other lag below N/2 a maximum)
     const int cap = P.ixmax / 2 + 1;
@@ -1161,62 +800,30 @@ int launch_pitch(vbx_ctx* ctx, const vbx_frames* fr, double fs, double threshold
         P.silence = peaks.silence;
     }
 
-    const char* rv = getenv("VBX_PITCH_REFINE");
-    const bool refine_v0 = rv && rv[0] == 'v' && rv[1] == '0';  // the first (warp per candidate) version, kept for A/B runs
-    const bool refine_v1 = rv && rv[0] == 'v' && rv[1] == '1';  // lockstep groups of four (no queue), kept for A/B runs
-    // Lanes per candidate slot of the queue-fed kernel.  Every evaluation of the interpolant pays ~300 instructions of setup (three
-    // sincospi, two reciprocals, the Brent update) whatever the slot width, so narrower slots — more candidates per warp —
-    // amortise it better: 8 lanes 5.70e6 frames/s on C4, 4 lanes 6.85e6, 2 lanes 7.06e6 (results identical: a slot's arithmetic
-    // is its own; 0 of 262 471 list positions off by > 0.1 Hz for each width).
-    int refine_lanes = 2;
-    if (const char* e = getenv("VBX_PITCH_REFINE_LANES")) refine_lanes = atoi(e) == 4 ? 4 : (atoi(e) == 8 ? 8 : 2);
     for (int64_t f0 = 0; f0 < fr->n_frames; f0 += slab) {
         P.frame0 = f0;
         P.n_frames = (fr->n_frames - f0 < slab) ? fr->n_frames - f0 : slab;
         VBX_CUDA(ctx, cudaMemsetAsync(P.counter, 0, 2 * sizeof(unsigned long long), ctx->stream));
         const int64_t grid = (P.n_frames + fpc - 1) / fpc;
         VBX_REQUIRE(ctx, grid <= 0x7fffffffLL, "too many frames for one launch");
-        if constexpr (!std::is_same<TIn, double>::value) {
-            if (lag_f32) pitch_lag_kernel<TIn><<<(unsigned)grid, threads, smem, ctx->stream>>>(P);
-        }
-        if (!lag_f32) {
-            if (lag_small) pitch_lag64_kernel<TIn, true><<<(unsigned)grid, threads, smem, ctx->stream>>>(P);
-            else pitch_lag64_kernel<TIn, false><<<(unsigned)grid, threads, smem, ctx->stream>>>(P);
-        }
-        VBX_CHECK_LAUNCH(ctx, lag_f32 ? "pitch_lag_kernel" : "pitch_lag64_kernel");
+        if (lag_small) pitch_lag64_kernel<TIn, true><<<(unsigned)grid, threads, smem, ctx->stream>>>(P);
+        else pitch_lag64_kernel<TIn, false><<<(unsigned)grid, threads, smem, ctx->stream>>>(P);
+        VBX_CHECK_LAUNCH(ctx, "pitch_lag64_kernel");
         if (lag_out) {  // vbx_pitch_lag_function: hand the lag function out and stop here
             VBX_CUDA(ctx, cudaMemcpyAsync(lag_out + (size_t)f0 * n, P.y, (size_t)P.n_frames * n * sizeof(double), cudaMemcpyDeviceToDevice,
                                           ctx->stream));
             continue;
         }
-        if (refine_v0) {
-            pitch_refine_kernel<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(P);
-        } else if (refine_v1) {
-            pitch_refine8_kernel<<<ctx->sm_count * 16, 128, 0, ctx->stream>>>(P);
-        } else {
-            static const int resident8 = [] {  // CTAs of the queue-fed kernel that fit one SM (computed once, thread-safely)
-                int r = 0;
-                if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&r, pitch_refine8q_kernel<8, 256>, 128, 0) != cudaSuccess || r < 1) {
-                    cudaGetLastError();
-                    r = 4;
-                }
-                return r;
-            }();
-            static const int resident4 = [] {
-                int r = 0;
-                if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&r, pitch_refine8q_kernel<2, 256>, 128, 0) != cudaSuccess || r < 1) {
-                    cudaGetLastError();
-                    r = 4;
-                }
-                return r;
-            }();
-            // (tiles larger than 256 entries were measured slower for every slot width: a tile's ~10 lag-function rows stay
-            // in L1, 40 rows do not)
-            if (refine_lanes == 2) pitch_refine8q_kernel<2, 256><<<ctx->sm_count * resident4, 128, 0, ctx->stream>>>(P);
-            else if (refine_lanes == 4) pitch_refine8q_kernel<4, 256><<<ctx->sm_count * resident4, 128, 0, ctx->stream>>>(P);
-            else pitch_refine8q_kernel<8, 256><<<ctx->sm_count * resident8, 128, 0, ctx->stream>>>(P);
-        }
-        VBX_CHECK_LAUNCH(ctx, refine_v0 ? "pitch_refine_kernel" : (refine_v1 ? "pitch_refine8_kernel" : "pitch_refine8q_kernel"));
+        static const int resident = [] {  // CTAs of the refinement kernel that fit one SM (computed once, thread-safely)
+            int r = 0;
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&r, pitch_refine8q_kernel, 128, 0) != cudaSuccess || r < 1) {
+                cudaGetLastError();
+                r = 4;
+            }
+            return r;
+        }();
+        pitch_refine8q_kernel<<<ctx->sm_count * resident, 128, 0, ctx->stream>>>(P);
+        VBX_CHECK_LAUNCH(ctx, "pitch_refine8q_kernel");
         pitch_finalize_kernel<<<(unsigned)((P.n_frames + 3) / 4), 128, 0, ctx->stream>>>(P, cand_out, max_cand, n_cand_out,
                                                                                         status_out, out_dtype == VBX_F64);
         VBX_CHECK_LAUNCH(ctx, "pitch_finalize_kernel");
@@ -1235,25 +842,27 @@ int pitch_check(vbx_ctx* ctx, const vbx_frames* fr, int max_cand, const void* ca
     return VBX_OK;
 }
 
+// The sample dtype picks the instantiation; every pitch entry point launches through here.
+int launch_pitch_any(vbx_ctx* ctx, const vbx_frames* fr, double fs, double threshold, double fmin, double fmax, int max_cand,
+                     void* cand_out, int32_t* n_cand_out, uint8_t* status_out, int out_dtype, double* lag_out, const PitchPeaks& peaks) {
+    cudaSetDevice(ctx->device);
+    if (fr->dtype == VBX_I16)
+        return launch_pitch<int16_t>(ctx, fr, fs, threshold, fmin, fmax, max_cand, cand_out, n_cand_out, status_out, out_dtype, lag_out,
+                                     peaks);
+    if (fr->dtype == VBX_F64)  // f64 samples (a frame the caller windowed in f64, as the reference's callers do)
+        return launch_pitch<double>(ctx, fr, fs, threshold, fmin, fmax, max_cand, cand_out, n_cand_out, status_out, out_dtype, lag_out,
+                                    peaks);
+    return launch_pitch<float>(ctx, fr, fs, threshold, fmin, fmax, max_cand, cand_out, n_cand_out, status_out, out_dtype, lag_out, peaks);
+}
+
 }  // namespace
 
 extern "C" {
 
 int vbx_pitch(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate, double threshold, double min_hz, double max_hz,
               int32_t max_candidates, void* cand_out, int32_t* n_cand_out, uint8_t* status_out, int32_t out_dtype) {
-    if (!ctx) return VBX_ERR_BADARG;
-    int st = pitch_check(ctx, frames, max_candidates, cand_out, out_dtype);
-    if (st != VBX_OK) return st;
-    if (frames->n_frames == 0) return VBX_OK;
-    cudaSetDevice(ctx->device);
-    if (frames->dtype == VBX_I16)
-        return launch_pitch<int16_t>(ctx, frames, sample_rate, threshold, min_hz, max_hz, max_candidates, cand_out, n_cand_out,
-                                     status_out, out_dtype);
-    if (frames->dtype == VBX_F64)  // f64 samples (a frame the caller windowed in f64, as the reference's callers do)
-        return launch_pitch<double>(ctx, frames, sample_rate, threshold, min_hz, max_hz, max_candidates, cand_out, n_cand_out,
-                                    status_out, out_dtype);
-    return launch_pitch<float>(ctx, frames, sample_rate, threshold, min_hz, max_hz, max_candidates, cand_out, n_cand_out,
-                               status_out, out_dtype);
+    return vbx_pitch_with_peaks(ctx, frames, sample_rate, threshold, 0.0, nullptr, nullptr, min_hz, max_hz, max_candidates, cand_out,
+                                n_cand_out, status_out, out_dtype);
 }
 
 // vbx_pitch with the reference's local_peak / global_peak honoured (periodic.rs:357; Boersma 1993): the unvoiced candidate's
@@ -1267,21 +876,14 @@ int vbx_pitch_with_peaks(vbx_ctx* ctx, const vbx_frames* frames, double sample_r
     if (st != VBX_OK) return st;
     VBX_REQUIRE(ctx, silence_threshold >= 0.0, "silence_threshold must be >= 0");
     if (frames->n_frames == 0) return VBX_OK;
-    cudaSetDevice(ctx->device);
     PitchPeaks pk;
     if (silence_threshold > 0.0) {
         pk.silence = silence_threshold;
         pk.local = local_peaks;
         pk.global = global_peaks;
     }
-    if (frames->dtype == VBX_I16)
-        return launch_pitch<int16_t>(ctx, frames, sample_rate, threshold, min_hz, max_hz, max_candidates, cand_out, n_cand_out,
-                                     status_out, out_dtype, nullptr, pk);
-    if (frames->dtype == VBX_F64)
-        return launch_pitch<double>(ctx, frames, sample_rate, threshold, min_hz, max_hz, max_candidates, cand_out, n_cand_out,
-                                    status_out, out_dtype, nullptr, pk);
-    return launch_pitch<float>(ctx, frames, sample_rate, threshold, min_hz, max_hz, max_candidates, cand_out, n_cand_out,
-                               status_out, out_dtype, nullptr, pk);
+    return launch_pitch_any(ctx, frames, sample_rate, threshold, min_hz, max_hz, max_candidates, cand_out, n_cand_out, status_out,
+                            out_dtype, nullptr, pk);
 }
 
 // The host pipeline cuts a segmented view into whole segments, so every chunk computes its segments' global peaks itself.  It
@@ -1324,11 +926,12 @@ int vbx_pitch_with_peaks_host(vbx_ctx* ctx, const vbx_frames* frames, double sam
     const double* d_global = n_global ? dev + n_local : nullptr;
     const size_t pair = (out_dtype == VBX_F64) ? 16 : 8;
     vbx_host_out outs[3] = {{cand_out, (size_t)max_candidates * pair, nullptr}, {n_cand_out, 4, nullptr}, {status_out, 1, nullptr}};
+    // chunked H2D / kernels / D2H pipeline (vbx_pipeline.cuh); output rows are indexed from the chunk's first frame
     const int rc = vbx_run_chunked(ctx, frames, outs, 3, [&](const vbx_frames* dfr, int64_t f0, int64_t u0, vbx_host_out* o) -> int {
         return vbx_pitch_with_peaks(ctx, dfr, sample_rate, threshold, silence_threshold, d_local ? d_local + f0 : nullptr,
                                     d_global ? d_global + u0 : nullptr, min_hz, max_hz, max_candidates, o[0].dev, (int32_t*)o[1].dev,
                                     (uint8_t*)o[2].dev, out_dtype);
-    }, 0, (size_t)96 << 20);  // the chunking of vbx_pitch_host
+    }, 0, (size_t)96 << 20);  // compute-bound: the copies hide behind the kernels anyway, larger chunks mean fewer kernel tails
     if (dev) cudaFree(dev);  // the pipeline has drained the stream
     return rc;
 }
@@ -1340,26 +943,13 @@ int vbx_pitch_lag_function(vbx_ctx* ctx, const vbx_frames* frames, double* lag_o
     int st = pitch_check(ctx, frames, 1, lag_out, VBX_F64);
     if (st != VBX_OK) return st;
     if (frames->n_frames == 0) return VBX_OK;
-    cudaSetDevice(ctx->device);
-    if (frames->dtype == VBX_I16) return launch_pitch<int16_t>(ctx, frames, 1.0, 0.0, 0.0, 0.0, 1, nullptr, nullptr, nullptr, VBX_F64, lag_out);
-    if (frames->dtype == VBX_F64) return launch_pitch<double>(ctx, frames, 1.0, 0.0, 0.0, 0.0, 1, nullptr, nullptr, nullptr, VBX_F64, lag_out);
-    return launch_pitch<float>(ctx, frames, 1.0, 0.0, 0.0, 0.0, 1, nullptr, nullptr, nullptr, VBX_F64, lag_out);
+    return launch_pitch_any(ctx, frames, 1.0, 0.0, 0.0, 0.0, 1, nullptr, nullptr, nullptr, VBX_F64, lag_out, PitchPeaks());
 }
 
 int vbx_pitch_host(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate, double threshold, double min_hz, double max_hz,
                    int32_t max_candidates, void* cand_out, int32_t* n_cand_out, uint8_t* status_out, int32_t out_dtype) {
-    if (!ctx) return VBX_ERR_BADARG;
-    int st = pitch_check(ctx, frames, max_candidates, cand_out, out_dtype);
-    if (st != VBX_OK) return st;
-    if (frames->n_frames == 0) return VBX_OK;
-    cudaSetDevice(ctx->device);
-    const size_t pair = (out_dtype == VBX_F64) ? 16 : 8;
-    vbx_host_out outs[3] = {{cand_out, (size_t)max_candidates * pair, nullptr}, {n_cand_out, 4, nullptr}, {status_out, 1, nullptr}};
-    // chunked H2D / kernels / D2H pipeline (vbx_pipeline.cuh); output rows are indexed from the chunk's first frame
-    return vbx_run_chunked(ctx, frames, outs, 3, [&](const vbx_frames* dfr, int64_t, int64_t, vbx_host_out* o) -> int {
-        return vbx_pitch(ctx, dfr, sample_rate, threshold, min_hz, max_hz, max_candidates, o[0].dev, (int32_t*)o[1].dev,
-                         (uint8_t*)o[2].dev, out_dtype);
-    }, 0, (size_t)96 << 20);  // compute-bound: the copies hide behind the kernels anyway, larger chunks mean fewer kernel tails
+    return vbx_pitch_with_peaks_host(ctx, frames, sample_rate, threshold, 0.0, nullptr, nullptr, min_hz, max_hz, max_candidates,
+                                     cand_out, n_cand_out, status_out, out_dtype);
 }
 
 int vbx_pitch_extract(vbx_ctx* ctx, const void* cand, int32_t dtype, int64_t n_frames, int32_t max_candidates, void* out) {

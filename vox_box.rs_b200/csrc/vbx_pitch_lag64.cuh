@@ -1,12 +1,12 @@
 // vbx_pitch_lag64.cuh — the all-lag autocorrelation of the pitch path in fp64 (periodic.rs:279-288 with L = N lags,
 // then :403-439).  Included inside the anonymous namespace of vbx_pitch.cu after PitchParams.
 //
-// Same work decomposition as the fp32 pitch_lag_kernel (a lane owns a 16-lag group and walks the frame in 8-sample
-// steps, group g paired with group G−1−g on the same lane so every lane runs the same number of steps), but the
-// windowed samples stay the exact f64 products x·w the reference forms and every lag product is one DFMA into a single
-// f64 accumulator per lag, summed in ascending i like the reference's fold.  What is left against the oracle is the
-// fused-multiply-add rounding (≈ 1e-16·r[0]); the fp32 sweep left ≈ 3e-8·r[0] in the lag function, which Brent on a
-// flat, mirrored interpolant amplified into > 0.1 Hz on 0.3 % of the weak (below-threshold) list entries.
+// A lane owns a 16-lag group and walks the frame in 8-sample steps, group g paired with group G−1−g on the same lane so
+// every lane runs the same number of steps.  The windowed samples stay the exact f64 products x·w the reference forms and
+// every lag product is one DFMA into a single f64 accumulator per lag, summed in ascending i like the reference's fold.
+// What is left against the oracle is the fused-multiply-add rounding (≈ 1e-16·r[0]); an fp32 sweep leaves ≈ 3e-8·r[0]
+// in the lag function, which Brent on a flat, mirrored interpolant amplifies into > 0.1 Hz on 0.3 % of the weak
+// (below-threshold) list entries (DESIGN.md §K6).
 //
 // Shared memory: the frame as doubles with 2 pad doubles per 16 (chunk k of 8 doubles starts at 8k + 2·(k >> 1)), so
 // the lanes of a quarter-warp — consecutive lag groups, 16 doubles apart — read their 16-byte pieces from 8 different
