@@ -209,11 +209,12 @@ def test_lpc_16_aligned_kernel_segments(oracle):
         assert np.max(normwise(ac[u * J:(u + 1) * J], ac_ref)) < 1e-7
 
 
-@pytest.mark.parametrize("ns,dtype", [(16000, "f32"), (16001, "f32"), (16003, "i16"), (24000, "i16")])
+@pytest.mark.parametrize("ns,dtype", [(16000, "f32"), (16001, "f32"), (16003, "i16"), (24000, "i16"), (8000, "f32")])
 def test_lpc_16_aligned_kernel_straddles_utterances(oracle, ns, dtype):
     """CTAs of the 16-aligned kernel take 64 consecutive frames of the batch, so most of them cross from one utterance into
     the next and stage their span as two pieces; an odd utterance length makes the second piece's source unaligned
-    (scalar staging path).  Results must equal the per-utterance oracle, and the per-segment mode (VBX_LPC16_NO_STRADDLE)."""
+    (scalar staging path).  Utterances shorter than one CTA's 64 frames (ns = 8000: 48 frames) take the per-segment mode,
+    one utterance per CTA.  Results must equal the per-utterance oracle in both modes."""
     fs, N, hop, p, U = 16000, 400, 160, 12, 7
     rng = np.random.default_rng(ns)
     audio = (rng.standard_normal((U, ns)) * 0.1).astype(np.float32)
@@ -229,7 +230,9 @@ def test_lpc_16_aligned_kernel_straddles_utterances(oracle, ns, dtype):
         d = c.to_device(audio)
         ref_in, scale = audio, 1.0
         fr = c.frames(d.ptr, U * J, N, hop, vb.WINDOW_HANN_SYMMETRIC, frames_per_segment=J, segment_stride=ns)
+    c.profile_begin()
     r = c.autocorrelate(fr, p + 1, out_dtype=vb.F64).to_host()
+    assert "lpc_fused16_kernel" in c.profile_end()
     for u in range(U):
         r_ref = oracle.batch_autocorrelate(ref_in[u], J, N, hop, oracle.WIN_HANN_SYMMETRIC, p + 1) * scale
         assert np.max(normwise(r[u * J:(u + 1) * J], r_ref)) < 1e-12, u

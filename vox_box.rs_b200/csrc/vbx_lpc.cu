@@ -32,7 +32,7 @@ struct LpcParams {
     void* kc_out;          // [F][L-1] or null
     int64_t n_frames;
     int64_t stride;        // frame stride in samples
-    int64_t seg_frames;    // frames per segment (utterance); CTAs never straddle segments
+    int64_t seg_frames;    // frames per segment (utterance); a CTA's frames lie in one segment unless `straddle`
     int64_t seg_stride;    // samples between segment starts
     int ctas_per_seg;
     int threads;           // CTA size (multiple of 32, <= kMaxThreads)
@@ -321,12 +321,6 @@ __global__ void __launch_bounds__(kMaxThreads, (L <= 13 ? 5 : 1)) lpc_fused_kern
     lpc_finish<L>(P, acc, g < Gc && q == 0, g, Gc, g0, s_out);
 }
 
-// VBX_LPC_FORCE_GENERIC=1 (tests): no fused kernel, the generic autocorrelation + stand-alone Levinson run instead
-bool lpc_force_generic() {
-    const char* e = getenv("VBX_LPC_FORCE_GENERIC");
-    return e && e[0] == '1';
-}
-
 #include "vbx_lpc16.cuh"
 #include "vbx_lpca.cuh"
 
@@ -427,28 +421,19 @@ __global__ void __launch_bounds__(128) levinson_kernel(const void* __restrict__ 
 }
 
 constexpr int kMaxFastLags = 25;  // fused kernel instantiated for 2..25 lags (LPC orders 1..24)
+constexpr int kMaxLevinsonOrder = 32;
 
 typedef void (*lpc_kernel_t)(const LpcParams);
-template <typename TIn, int L> struct LpcTable {
-    static void fill(lpc_kernel_t* t) {
-        t[L] = lpc_fused_kernel<L, TIn>;
-        LpcTable<TIn, L - 1>::fill(t);
-    }
-};
-template <typename TIn> struct LpcTable<TIn, 1> {
-    static void fill(lpc_kernel_t*) {}
-};
-
 typedef void (*lpca_kernel_t)(const LpcParams, const LpcaExtra);
-template <typename TIn, int L> struct LpcaTable {
-    static void fill(lpca_kernel_t* t) {
-        t[L] = lpc_fuseda_kernel<L, TIn>;
-        LpcaTable<TIn, L - 1>::fill(t);
-    }
-};
-template <typename TIn> struct LpcaTable<TIn, 1> {
-    static void fill(lpca_kernel_t*) {}
-};
+typedef void (*lpcp_kernel_t)(const LpcParams, const LpcaExtra, const int, unsigned*);
+typedef void (*lev_kernel_t)(const void*, int, int64_t, int, void*, void*, int);
+
+// Kernel tables indexed by a template argument: t[I] = make(std::integral_constant<int, I>()) for I = Lo..Hi.
+template <int Lo, int Hi, typename T, typename Make>
+void fill_table(T* t, Make make) {
+    t[Lo] = make(std::integral_constant<int, Lo>());
+    if constexpr (Lo < Hi) fill_table<Lo + 1, Hi>(t, make);
+}
 
 // The two shifted window rows of lpc_fuseda_kernel, E = [0, 0, w…, 0…] and O = [0, 0, 0, w…, 0…] ([2][wt] f64), cached per
 // (window kind, n, sample dtype) next to the plain tables.
@@ -479,50 +464,18 @@ int get_window_rows_aligned(vbx_ctx* ctx, int kind, int n, int wt, const double*
     return VBX_OK;
 }
 
-template <typename TIn, int L> struct Lpc16Table {
-    static void fill(lpc_kernel_t* t) {
-        t[L] = lpc_fused16_kernel<L, TIn>;
-        Lpc16Table<TIn, L - 1>::fill(t);
-    }
-};
-template <typename TIn> struct Lpc16Table<TIn, 1> {
-    static void fill(lpc_kernel_t*) {}
-};
-
-typedef void (*lev_kernel_t)(const void*, int, int64_t, int, void*, void*, int);
-template <int P> struct LevTable {
-    static void fill(lev_kernel_t* t) {
-        t[P] = levinson_kernel<P>;
-        LevTable<P - 1>::fill(t);
-    }
-};
-template <> struct LevTable<0> {
-    static void fill(lev_kernel_t*) {}
-};
-constexpr int kMaxLevinsonOrder = 32;
-
-// Choose lanes-per-frame K (and the CTA size): the smallest power of two whose CTA span fits the
+// Choose lanes-per-frame K for a CTA of kMaxThreads: the smallest power of two whose CTA span fits the
 // shared-memory budget, keeping each lane's part >= 2L samples.  Returns false if no fused
-// configuration fits.  VBX_LPC_PLAN="k:threads" overrides the choice (tuning experiments).
+// configuration fits.
 bool plan_fused(const vbx_ctx* ctx, int n, int64_t stride, int L, LpcParams* P, size_t* smem_bytes) {
-    if (lpc_force_generic()) return false;
     const int sv = (int)(stride < (int64_t)n ? stride : n);
     const int pad = ((sv & 1) == 0) ? 1 : 0;
     const size_t budget_soft = 72 * 1024;  // 3 CTAs / SM
     const size_t budget_hard = ctx->smem_optin;
-    int threads = kMaxThreads, force_k = 0;
-    if (const char* e = getenv("VBX_LPC_PLAN")) {
-        int a = 0, b = 0;
-        if (sscanf(e, "%d:%d", &a, &b) == 2 && a >= 1 && a <= 32 && (a & (a - 1)) == 0 && b >= 32 && b <= kMaxThreads && b % 32 == 0) {
-            force_k = a;
-            threads = b;
-        }
-    }
     int best_k = 0;
     size_t best_bytes = 0;
     for (int k = 1; k <= 32; k <<= 1) {
-        if (force_k && k != force_k) continue;
-        const int G = threads / k;
+        const int G = kMaxThreads / k;
         const int part = (n + k - 1) / k;
         if (k > 1 && part < 2 * L) break;
         const int64_t span = (int64_t)(G - 1) * sv + n;
@@ -544,33 +497,29 @@ bool plan_fused(const vbx_ctx* ctx, int n, int64_t stride, int L, LpcParams* P, 
     if (!best_k) return false;
     P->sv = sv;
     P->pad = pad;
-    P->threads = threads;
+    P->threads = kMaxThreads;
     P->sv_magic = sv > 1 ? (unsigned)((1ULL << 32) / (unsigned)sv) + 1u : 0u;
     *smem_bytes = best_bytes;
     return true;
 }
 
-// Plan for lpc_fused16_kernel (vbx_lpc16.cuh): 16-aligned framings with at most 16 lags.  Two lanes per frame;
-// the CTA size is chosen as described in the loop below (C2: 128 threads = 64 frames, 4 CTAs / SM).
-// VBX_LPC16=0 disables the kernel, VBX_LPC16_THREADS=<n> pins the CTA size.
-bool plan_fused16(const vbx_ctx* ctx, int n, int64_t stride, int64_t seg_frames, int L, LpcParams* P, size_t* smem_bytes) {
-    if (L < 2 || L > kChunk || (n % kChunk) != 0 || lpc_force_generic()) return false;
+// Plan for lpc_fused16_kernel (vbx_lpc16.cuh): 16-aligned framings with at most 16 lags.  Two lanes per frame (a pair of
+// warps per 32 frames); the CTA size is chosen as described in the loop below (C2: 128 threads = 64 frames, 4 CTAs / SM).
+// VBX_LPC16=0 disables the kernel.
+bool plan_fused16(const vbx_ctx* ctx, int n, int64_t stride, int L, LpcParams* P, size_t* smem_bytes) {
+    if (L < 2 || L > kChunk || (n % kChunk) != 0) return false;
     const int sv = (int)(stride < (int64_t)n ? stride : n);
     if ((sv % kChunk) != 0) return false;
     if (const char* e = getenv("VBX_LPC16")) {
         if (atoi(e) == 0) return false;
     }
     const int pad = 4;  // sv / 4 is even, so (sv + 4) / 4 is odd: frame starts walk through all 8 bank groups
-    int force_threads = 0, halves = 2;
-    if (const char* e = getenv("VBX_LPC16_THREADS")) force_threads = atoi(e);
-    if (const char* e = getenv("VBX_LPC16_K")) halves = atoi(e) == 1 ? 1 : 2;  // lanes per frame (experiments)
     const size_t sm_bytes = 228 * 1024, cta_overhead = 1024;
     int best_threads = 0, best_score = 0;
     size_t best_bytes = 0;
     int best_words = 0;
-    for (int threads = 32 * halves; threads <= 256; threads += 32 * halves) {
-        if (force_threads && threads != force_threads) continue;
-        const int G = threads / halves;
+    for (int threads = 64; threads <= 256; threads += 64) {
+        const int G = threads / 2;
         const int64_t span = (int64_t)(G - 1) * sv + n;
         if (span * (int64_t)sv >= (1LL << 32)) continue;
         // room for a span staged as two pieces (a CTA that crosses into the next utterance, P.straddle)
@@ -590,7 +539,6 @@ bool plan_fused16(const vbx_ctx* ctx, int n, int64_t stride, int64_t seg_frames,
         const int warps = ctas * threads / 32;
         const int d = threads > 128 ? threads - 128 : 128 - threads;
         const int score = (warps < 16 ? warps : 16) * 1000 + (ctas >= 3 ? 500 : 0) + (256 - d);
-        (void)seg_frames;
         if (score > best_score) {
             best_threads = threads;
             best_score = score;
@@ -599,9 +547,9 @@ bool plan_fused16(const vbx_ctx* ctx, int n, int64_t stride, int64_t seg_frames,
         }
     }
     if (!best_threads) return false;
-    P->k = halves;
+    P->k = 2;
     P->threads = best_threads;
-    P->frames_per_cta = best_threads / halves;
+    P->frames_per_cta = best_threads / 2;
     P->part = 0;
     P->span_words = best_words;
     P->sv = sv;
@@ -611,107 +559,106 @@ bool plan_fused16(const vbx_ctx* ctx, int n, int64_t stride, int64_t seg_frames,
     return true;
 }
 
+enum class LpcKind { fused16, persistent, aligned, general, generic };
+
+struct LpcPlan {
+    LpcKind kind;
+    LpcParams P;   // everything but the window, the outputs and the Levinson flag, which launch_lpc adds
+    LpcaExtra X;   // persistent / aligned: geometry of the window rows (launch_lpc adds the rows themselves)
+    size_t smem;   // dynamic shared memory per CTA
+    int64_t ctas;  // CTAs of the one-shot kernels, tiles of the persistent one
+};
+
+// The one place that picks the LPC kernel for a view.  vbx_lpc_scratch_bytes asks it too, so the scratch that
+// vbx_find_formants reserves for the LPC stage always matches the path launch_lpc takes.  In order of preference:
+// lpc_fused16_kernel (16-aligned framings, <= 16 lags), lpc_fusedp_kernel (fp32, overlapped or packed frames, <= 13 lags,
+// enough tiles for every SM), lpc_fuseda_kernel (the same framings), lpc_fused_kernel (<= 25 lags), and the generic
+// autocorrelation + stand-alone Levinson.  f64 samples (the single-frame trait calls of the Rust shim on [f64]) take the
+// generic kernels: the fused ones stage fp32 / int16 samples.  VBX_LPC_FORCE_GENERIC=1 (tests) sends every view there.
+LpcPlan plan_lpc(const vbx_ctx* ctx, const vbx_frames* fr, int L) {
+    LpcPlan pl{};
+    pl.kind = LpcKind::generic;
+    const char* force = getenv("VBX_LPC_FORCE_GENERIC");
+    if (fr->dtype == VBX_F64 || (force && force[0] == '1')) return pl;
+    const int n = fr->frame_len;
+    const int64_t stride = fr->frame_stride;
+    LpcParams& P = pl.P;
+    if (plan_fused16(ctx, n, stride, L, &P, &pl.smem)) pl.kind = LpcKind::fused16;
+    else if (plan_fusedp(ctx, fr, L, &P, &pl.X, &pl.smem)) pl.kind = LpcKind::persistent;
+    else if (plan_fuseda(ctx, n, stride, L, vbx_dtype_size(fr->dtype), &P, &pl.X, &pl.smem)) pl.kind = LpcKind::aligned;
+    else if (L >= 2 && L <= kMaxFastLags && plan_fused(ctx, n, stride, L, &P, &pl.smem)) pl.kind = LpcKind::general;
+    else return pl;
+    P.base = fr->base;
+    P.n_frames = fr->n_frames;
+    P.stride = stride;
+    P.seg_frames = vbx_frames_per_segment(fr);
+    P.seg_stride = fr->frames_per_segment > 0 ? fr->segment_stride : 0;
+    P.ctas_per_seg = (int)((P.seg_frames + P.frames_per_cta - 1) / P.frames_per_cta);
+    P.n = n;
+    // 16-aligned kernel, several utterances of at least one CTA's worth of overlapped frames: CTAs take G consecutive
+    // frames of the batch (an utterance of 998 frames otherwise leaves 26 of its last CTA's 64 frame slots empty)
+    P.straddle = (pl.kind == LpcKind::fused16 && P.n_frames > P.seg_frames && P.seg_frames >= P.frames_per_cta &&
+                  stride <= (int64_t)n) ? 1 : 0;
+    pl.ctas = P.straddle ? (P.n_frames + P.frames_per_cta - 1) / P.frames_per_cta
+                         : (P.n_frames / P.seg_frames) * P.ctas_per_seg;
+    return pl;
+}
+
+// Launches the fused kernel a plan names.  Instantiated for fp32 and int16 samples: plan_lpc sends f64 samples to the
+// generic kernels.
+template <typename TIn>
+int launch_fused(vbx_ctx* ctx, const vbx_frames* fr, int L, LpcPlan& pl) {
+    // kernel tables: filled once, thread-safely (C++11 static initialisation)
+    struct Tables {
+        lpc_kernel_t chunk16[kChunk + 1] = {nullptr};
+        lpcp_kernel_t persistent[kLpcaMaxLags + 1] = {nullptr};
+        lpca_kernel_t aligned[kLpcaMaxLags + 1] = {nullptr};
+        lpc_kernel_t general[kMaxFastLags + 1] = {nullptr};
+        Tables() {
+            fill_table<2, kChunk>(chunk16, [](auto l) -> lpc_kernel_t { return lpc_fused16_kernel<decltype(l)::value, TIn>; });
+            fill_table<2, kLpcaMaxLags>(persistent, [](auto l) -> lpcp_kernel_t { return lpc_fusedp_kernel<decltype(l)::value>; });
+            fill_table<2, kLpcaMaxLags>(aligned, [](auto l) -> lpca_kernel_t { return lpc_fuseda_kernel<decltype(l)::value, TIn>; });
+            fill_table<2, kMaxFastLags>(general, [](auto l) -> lpc_kernel_t { return lpc_fused_kernel<decltype(l)::value, TIn>; });
+        }
+    };
+    static const Tables tables;
+    auto launch = [&](auto kern, int64_t grid, const char* name, auto... args) -> int {
+        VBX_REQUIRE(ctx, grid <= 0x7fffffffLL, "too many frames for one launch");
+        VBX_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
+        kern<<<(unsigned)grid, pl.P.threads, pl.smem, ctx->stream>>>(args...);
+        VBX_CHECK_LAUNCH(ctx, name);
+        return VBX_OK;
+    };
+    if (pl.kind == LpcKind::fused16) return launch(tables.chunk16[L], pl.ctas, "lpc_fused16_kernel", pl.P);
+    if (pl.kind == LpcKind::general) return launch(tables.general[L], pl.ctas, "lpc_fused_kernel", pl.P);
+    // the aligned-down 16-sample-chunk walk (vbx_lpca.cuh)
+    int st = get_window_rows_aligned(ctx, fr->window, fr->frame_len, pl.X.wt, &pl.X.tabs, fr->dtype);
+    if (st != VBX_OK) return st;
+    if (pl.kind == LpcKind::aligned) return launch(tables.aligned[L], pl.ctas, "lpc_fuseda_kernel", pl.P, pl.X);
+    // enough tiles for every SM: the persistent, TMA-fed, warp-specialised CTA (one per SM)
+    int grid = ctx->sm_count - (ctx->reserve_sms > 0 && ctx->reserve_sms < ctx->sm_count / 2 ? ctx->reserve_sms : 0);
+    if (pl.ctas < grid) grid = (int)pl.ctas;
+    VBX_CUDA(ctx, cudaMemsetAsync(ctx->tile_counter, 0, sizeof(unsigned), ctx->stream));
+    return launch(tables.persistent[L], grid, "lpc_fusedp_kernel", pl.P, pl.X, (int)pl.ctas, ctx->tile_counter);
+}
+
 template <typename TIn>
 int launch_lpc(vbx_ctx* ctx, const vbx_frames* fr, int L, void* r_out, void* ac_out, void* kc_out, int out_dtype,
                bool do_levinson) {
     const double* win = nullptr;
     int st = vbx_get_window(ctx, fr->window, fr->frame_len, &win, fr->dtype);
     if (st != VBX_OK) return st;
-    // f64 samples (the single-frame trait calls of the Rust shim on [f64]) take the generic kernels; the fused kernels
-    // stage fp32 / int16 samples
     if constexpr (!std::is_same<TIn, double>::value) {
-    // kernel tables: filled once, thread-safely (C++11 static initialisation)
-    struct Tables {
-        lpc_kernel_t general[kMaxFastLags + 1] = {nullptr};
-        lpc_kernel_t chunk16[kChunk + 1] = {nullptr};
-        lpca_kernel_t aligned[kLpcaMaxLags + 1] = {nullptr};
-        lpcp_kernel_t persistent[kLpcaMaxLags + 1] = {nullptr};
-        Tables() {
-            LpcTable<TIn, kMaxFastLags>::fill(general);
-            Lpc16Table<TIn, kChunk>::fill(chunk16);
-            LpcaTable<TIn, kLpcaMaxLags>::fill(aligned);
-            if (std::is_same<TIn, float>::value) LpcpTable<kLpcaMaxLags>::fill(persistent);
+        LpcPlan pl = plan_lpc(ctx, fr, L);
+        if (pl.kind != LpcKind::generic) {
+            pl.P.win = win;
+            pl.P.r_out = r_out;
+            pl.P.ac_out = ac_out;
+            pl.P.kc_out = kc_out;
+            pl.P.out_f64 = (out_dtype == VBX_F64);
+            pl.P.do_levinson = do_levinson ? 1 : 0;
+            return launch_fused<TIn>(ctx, fr, L, pl);
         }
-    };
-    static const Tables tables;
-    const lpc_kernel_t* table = tables.general;
-    const lpc_kernel_t* table16 = tables.chunk16;
-
-    LpcParams P;
-    memset(&P, 0, sizeof(P));
-    size_t smem = 0;
-    const bool fused16 = plan_fused16(ctx, fr->frame_len, fr->frame_stride, vbx_frames_per_segment(fr), L, &P, &smem);
-    LpcaExtra X;
-    memset(&X, 0, sizeof(X));
-    int n_tiles = 0;
-    bool persistent = false;
-    if constexpr (std::is_same<TIn, float>::value) persistent = !fused16 && plan_fusedp(ctx, fr, L, &P, &X, &smem, &n_tiles);
-    if (persistent || (!fused16 && plan_fuseda(ctx, fr->frame_len, fr->frame_stride, L, sizeof(TIn), &P, &X, &smem))) {
-        // any other overlapped / packed framing with <= 13 lags: the aligned-down 16-sample-chunk walk (vbx_lpca.cuh)
-        st = get_window_rows_aligned(ctx, fr->window, fr->frame_len, X.wt, &X.tabs, fr->dtype);
-        if (st != VBX_OK) return st;
-        P.base = fr->base;
-        P.win = win;
-        P.r_out = r_out;
-        P.ac_out = ac_out;
-        P.kc_out = kc_out;
-        P.n_frames = fr->n_frames;
-        P.stride = fr->frame_stride;
-        P.seg_frames = vbx_frames_per_segment(fr);
-        P.seg_stride = fr->frames_per_segment > 0 ? fr->segment_stride : 0;
-        P.ctas_per_seg = (int)((P.seg_frames + P.frames_per_cta - 1) / P.frames_per_cta);
-        P.n = fr->frame_len;
-        P.out_f64 = (out_dtype == VBX_F64);
-        P.do_levinson = do_levinson ? 1 : 0;
-        if (persistent) {
-            // enough tiles for every SM: the persistent, TMA-fed, warp-specialised CTA (one per SM)
-            lpcp_kernel_t kern = tables.persistent[L];
-            VBX_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            int grid = ctx->sm_count - (ctx->reserve_sms > 0 && ctx->reserve_sms < ctx->sm_count / 2 ? ctx->reserve_sms : 0);
-            if (n_tiles < grid) grid = n_tiles;
-            VBX_CUDA(ctx, cudaMemsetAsync(ctx->tile_counter, 0, sizeof(unsigned), ctx->stream));
-            kern<<<(unsigned)grid, P.threads, smem, ctx->stream>>>(P, X, n_tiles, ctx->tile_counter);
-            VBX_CHECK_LAUNCH(ctx, "lpc_fusedp_kernel");
-            return VBX_OK;
-        }
-        lpca_kernel_t kern = tables.aligned[L];
-        VBX_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        const int64_t grid = (fr->n_frames / P.seg_frames) * P.ctas_per_seg;
-        VBX_REQUIRE(ctx, grid <= 0x7fffffffLL, "too many frames for one launch");
-        kern<<<(unsigned)grid, P.threads, smem, ctx->stream>>>(P, X);
-        VBX_CHECK_LAUNCH(ctx, "lpc_fuseda_kernel");
-        return VBX_OK;
-    }
-    const bool fused_ok =
-        fused16 || ((L >= 2 && L <= kMaxFastLags) && plan_fused(ctx, fr->frame_len, fr->frame_stride, L, &P, &smem));
-    if (fused_ok) {
-        P.base = fr->base;
-        P.win = win;
-        P.r_out = r_out;
-        P.ac_out = ac_out;
-        P.kc_out = kc_out;
-        P.n_frames = fr->n_frames;
-        P.stride = fr->frame_stride;
-        P.seg_frames = vbx_frames_per_segment(fr);
-        P.seg_stride = fr->frames_per_segment > 0 ? fr->segment_stride : 0;
-        P.ctas_per_seg = (int)((P.seg_frames + P.frames_per_cta - 1) / P.frames_per_cta);
-        P.n = fr->frame_len;
-        P.out_f64 = (out_dtype == VBX_F64);
-        P.do_levinson = do_levinson ? 1 : 0;
-        lpc_kernel_t kern = fused16 ? table16[L] : table[L];
-        VBX_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        // 16-aligned kernel, several utterances of at least one CTA's worth of overlapped frames: CTAs take G consecutive
-        // frames of the batch (an utterance of 998 frames otherwise leaves 26 of its last CTA's 64 frame slots empty)
-        P.straddle = (fused16 && fr->n_frames > P.seg_frames && P.seg_frames >= P.frames_per_cta && P.stride <= (int64_t)P.n &&
-                      !getenv("VBX_LPC16_NO_STRADDLE")) ? 1 : 0;
-        const int64_t grid = P.straddle ? (fr->n_frames + P.frames_per_cta - 1) / P.frames_per_cta
-                                        : (fr->n_frames / P.seg_frames) * P.ctas_per_seg;
-        VBX_REQUIRE(ctx, grid <= 0x7fffffffLL, "too many frames for one launch");
-        kern<<<(unsigned)grid, P.threads, smem, ctx->stream>>>(P);
-        VBX_CHECK_LAUNCH(ctx, fused16 ? "lpc_fused16_kernel" : "lpc_fused_kernel");
-        return VBX_OK;
-    }
-
     }
 
     // fallback: generic autocorrelation (+ stand-alone Levinson through a scratch r buffer)
@@ -746,28 +693,26 @@ int launch_lpc(vbx_ctx* ctx, const vbx_frames* fr, int L, void* r_out, void* ac_
     return VBX_OK;
 }
 
-bool lpc_is_fused(vbx_ctx* ctx, const vbx_frames* fr, int L) {
-    if (fr->dtype == VBX_F64) return false;
-    LpcParams P;
-    memset(&P, 0, sizeof(P));
-    size_t smem = 0;
-    if (plan_fused16(ctx, fr->frame_len, fr->frame_stride, vbx_frames_per_segment(fr), L, &P, &smem)) return true;
-    LpcaExtra X;
-    if (plan_fuseda(ctx, fr->frame_len, fr->frame_stride, L, vbx_dtype_size(fr->dtype), &P, &X, &smem)) return true;
-    return (L >= 2 && L <= kMaxFastLags) && plan_fused(ctx, fr->frame_len, fr->frame_stride, L, &P, &smem);
-}
-
-int lpc_dispatch(vbx_ctx* ctx, const vbx_frames* fr, int n_lags, void* r_out, void* ac_out, void* kc_out, int out_dtype,
-                 bool do_levinson) {
+// Argument checks of the autocorrelation and LPC entry points.  The host twins run them before they size their buffers
+// from n_lags, the device calls before they launch.
+int lpc_check(vbx_ctx* ctx, const vbx_frames* fr, int n_lags, const void* r_out, int out_dtype, bool do_levinson) {
     if (!ctx) return VBX_ERR_BADARG;
     int st = vbx_check_frames(ctx, fr, /*allow_f64=*/true);
     if (st != VBX_OK) return st;
     VBX_REQUIRE(ctx, out_dtype == VBX_F32 || out_dtype == VBX_F64, "out_dtype must be VBX_F32 or VBX_F64");
+    VBX_REQUIRE(ctx, do_levinson || r_out || fr->n_frames == 0, "r_out is NULL");
+    VBX_REQUIRE(ctx, !do_levinson || n_lags >= 2, "LPC order must be >= 1");
     VBX_REQUIRE(ctx, n_lags >= 1, "n_lags must be >= 1");
     VBX_REQUIRE(ctx, n_lags <= fr->frame_len, "n_lags (%d) > frame_len (%d): the reference's `self.len() - lag` underflows",
                 n_lags, fr->frame_len);
     VBX_REQUIRE(ctx, !do_levinson || n_lags - 1 <= kMaxLevinsonOrder, "LPC order > %d not supported", kMaxLevinsonOrder);
-    if (fr->n_frames == 0) return VBX_OK;
+    return VBX_OK;
+}
+
+int lpc_dispatch(vbx_ctx* ctx, const vbx_frames* fr, int n_lags, void* r_out, void* ac_out, void* kc_out, int out_dtype,
+                 bool do_levinson) {
+    int st = lpc_check(ctx, fr, n_lags, r_out, out_dtype, do_levinson);
+    if (st != VBX_OK || fr->n_frames == 0) return st;
     cudaSetDevice(ctx->device);
     if (fr->dtype == VBX_I16)
         return launch_lpc<int16_t>(ctx, fr, n_lags, r_out, ac_out, kc_out, out_dtype, do_levinson);
@@ -779,11 +724,8 @@ int lpc_dispatch(vbx_ctx* ctx, const vbx_frames* fr, int n_lags, void* r_out, vo
 // host twin: chunked H2D / kernels / D2H pipeline (vbx_pipeline.cuh)
 int lpc_host(vbx_ctx* ctx, const vbx_frames* fr, int n_lags, void* r_out, void* ac_out, void* kc_out, int out_dtype,
              bool do_levinson) {
-    if (!ctx) return VBX_ERR_BADARG;
-    int st = vbx_check_frames(ctx, fr, /*allow_f64=*/true);
-    if (st != VBX_OK) return st;
-    VBX_REQUIRE(ctx, out_dtype == VBX_F32 || out_dtype == VBX_F64, "out_dtype must be VBX_F32 or VBX_F64");
-    if (fr->n_frames == 0) return VBX_OK;
+    int st = lpc_check(ctx, fr, n_lags, r_out, out_dtype, do_levinson);
+    if (st != VBX_OK || fr->n_frames == 0) return st;
     cudaSetDevice(ctx->device);
     const size_t os = vbx_dtype_size(out_dtype);
     vbx_host_out outs[3] = {{r_out, (size_t)n_lags * os, nullptr},
@@ -798,19 +740,15 @@ int lpc_host(vbx_ctx* ctx, const vbx_frames* fr, int n_lags, void* r_out, void* 
 
 // scratch launch_lpc asks vbx_scratch_get for when called as vbx_lpc(.., r_out = NULL, ..) (vbx_find_formants' LPC stage)
 size_t vbx_lpc_scratch_bytes(vbx_ctx* ctx, const vbx_frames* fr, int n_lags) {
-    if (lpc_is_fused(ctx, fr, n_lags)) return 0;
-    return (size_t)fr->n_frames * n_lags * sizeof(double);
+    return plan_lpc(ctx, fr, n_lags).kind == LpcKind::generic ? (size_t)fr->n_frames * n_lags * sizeof(double) : 0;
 }
 
 extern "C" {
 
 int vbx_autocorrelate(vbx_ctx* ctx, const vbx_frames* frames, int32_t n_lags, void* r_out, int32_t out_dtype) {
-    if (ctx && !r_out && frames && frames->n_frames > 0) return vbx_fail(ctx, VBX_ERR_BADARG, "r_out is NULL");
     return lpc_dispatch(ctx, frames, n_lags, r_out, nullptr, nullptr, out_dtype, false);
 }
 int vbx_autocorrelate_host(vbx_ctx* ctx, const vbx_frames* frames, int32_t n_lags, void* r_out, int32_t out_dtype) {
-    if (ctx && !r_out && frames && frames->n_frames > 0) return vbx_fail(ctx, VBX_ERR_BADARG, "r_out is NULL");
-    if (ctx && frames && n_lags < 1) return vbx_fail(ctx, VBX_ERR_BADARG, "n_lags must be >= 1");
     return lpc_host(ctx, frames, n_lags, r_out, nullptr, nullptr, out_dtype, false);
 }
 
@@ -842,13 +780,10 @@ int vbx_autocorrelate_ring(vbx_ctx* ctx, const void* rings, int32_t dtype, int64
 }
 
 int vbx_lpc(vbx_ctx* ctx, const vbx_frames* frames, int32_t p, void* r_out, void* ac_out, void* kc_out, int32_t out_dtype) {
-    if (ctx && p < 1) return vbx_fail(ctx, VBX_ERR_BADARG, "LPC order must be >= 1");
     return lpc_dispatch(ctx, frames, p + 1, r_out, ac_out, kc_out, out_dtype, true);
 }
 int vbx_lpc_host(vbx_ctx* ctx, const vbx_frames* frames, int32_t p, void* r_out, void* ac_out, void* kc_out,
                  int32_t out_dtype) {
-    if (ctx && p < 1) return vbx_fail(ctx, VBX_ERR_BADARG, "LPC order must be >= 1");
-    if (ctx && frames && p + 1 > frames->frame_len) return vbx_fail(ctx, VBX_ERR_BADARG, "order + 1 > frame_len");
     return lpc_host(ctx, frames, p + 1, r_out, ac_out, kc_out, out_dtype, true);
 }
 
@@ -857,7 +792,7 @@ int vbx_lpc_levinson(vbx_ctx* ctx, const void* r, int32_t r_dtype, int64_t n_fra
     if (!ctx) return VBX_ERR_BADARG;
     struct Tables {
         lev_kernel_t t[kMaxLevinsonOrder + 1] = {nullptr};
-        Tables() { LevTable<kMaxLevinsonOrder>::fill(t); }
+        Tables() { fill_table<1, kMaxLevinsonOrder>(t, [](auto p) -> lev_kernel_t { return levinson_kernel<decltype(p)::value>; }); }
     };
     static const Tables tables;  // filled once, thread-safely
     const lev_kernel_t* table = tables.t;

@@ -132,11 +132,11 @@ __global__ void __maxnreg__(96) lpc_fused16_kernel(const LpcParams P) {
     if (nB > 0) stage_span16<TIn>(P, base + P.seg_stride, 0, nB, s_span + offB);
     __syncthreads();
 
-    // warp → (32 frames, half): with two halves per frame (P.k == 2) even warps walk the first chunks of their 32
-    // frames and odd warps the rest, so the pre-roll below is warp-uniform; P.k == 1: a lane walks its whole frame
+    // warp → (32 frames, half): even warps walk the first chunks of their 32 frames and odd warps the rest, so the
+    // pre-roll below is warp-uniform
     const int warp = tid >> 5, lane = tid & 31;
-    const int q = (P.k == 2) ? (warp & 1) : 0;
-    const int g = ((P.k == 2) ? (warp >> 1) : warp) * 32 + lane;
+    const int q = warp & 1;
+    const int g = (warp >> 1) * 32 + lane;
     double acc[L], h[kChunk];
 #pragma unroll
     for (int j = 0; j < L; ++j) acc[j] = 0.0;
@@ -144,7 +144,7 @@ __global__ void __maxnreg__(96) lpc_fused16_kernel(const LpcParams P) {
     for (int j = 0; j < kChunk; ++j) h[j] = 0.0;
     if (g < Gc) {
         const int C = n / kChunk;                               // chunks per frame
-        const int nch = (P.k == 2) ? ((C + 2) >> 1) : C;        // chunk passes per lane: ceil((C + 1) / 2)
+        const int nch = (C + 2) >> 1;                           // chunk passes per lane: ceil((C + 1) / 2)
         const int pre = q ? 2 * nch - C : 0;                    // pre-roll passes of the second half (1 or 2): ring fill only
         const int cpb = sv / kChunk;                            // chunks between pad words
         const int c = q ? C - nch : 0;
@@ -209,12 +209,10 @@ __global__ void __maxnreg__(96) lpc_fused16_kernel(const LpcParams P) {
 #pragma unroll
         for (int lag = 0; lag < L; ++lag) s_r[g * L + lag] = acc[lag];
     }
-    if (P.k == 2) {
-        __syncthreads();
-        if (q == 0 && g < Gc) {
+    __syncthreads();
+    if (q == 0 && g < Gc) {
 #pragma unroll
-            for (int lag = 0; lag < L; ++lag) acc[lag] += s_r[g * L + lag];
-        }
+        for (int lag = 0; lag < L; ++lag) acc[lag] += s_r[g * L + lag];
     }
     lpc_finish<L>(P, acc, g < Gc && q == 0, g, Gc, g0, s_out);
 }

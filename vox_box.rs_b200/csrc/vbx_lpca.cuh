@@ -233,9 +233,7 @@ __global__ void __launch_bounds__(256) lpc_fuseda_kernel(const LpcParams P, cons
 
 // Plan for lpc_fuseda_kernel.  Returns false when the shape is not its (gapped frames, too many lags, too long a frame).
 bool plan_fuseda(const vbx_ctx* ctx, int n, int64_t stride, int L, size_t in_size, LpcParams* P, LpcaExtra* X, size_t* smem_bytes) {
-    if (L < 2 || L > kLpcaMaxLags || stride > (int64_t)n || lpc_force_generic()) return false;
-    if (const char* e = getenv("VBX_LPCA"))
-        if (atoi(e) == 0) return false;
+    if (L < 2 || L > kLpcaMaxLags || stride > (int64_t)n) return false;
     const int sv = (int)stride;
     const int C = (n + 3 + kChunk - 1) / kChunk;
     int G = 32, K = 8;
@@ -538,24 +536,11 @@ __global__ void __launch_bounds__(320, 1) lpc_fusedp_kernel(const LpcParams P, c
     }
 }
 
-typedef void (*lpcp_kernel_t)(const LpcParams, const LpcaExtra, const int, unsigned*);
-template <int L> struct LpcpTable {
-    static void fill(lpcp_kernel_t* t) {
-        t[L] = lpc_fusedp_kernel<L>;
-        LpcpTable<L - 1>::fill(t);
-    }
-};
-template <> struct LpcpTable<1> {
-    static void fill(lpcp_kernel_t*) {}
-};
-
 // Plan for lpc_fusedp_kernel: fp32 samples, overlapped or packed frames, <= 13 lags, enough tiles to keep every SM's CTA busy.
-bool plan_fusedp(const vbx_ctx* ctx, const vbx_frames* fr, int L, LpcParams* P, LpcaExtra* X, size_t* smem_bytes, int* n_tiles) {
+bool plan_fusedp(const vbx_ctx* ctx, const vbx_frames* fr, int L, LpcParams* P, LpcaExtra* X, size_t* smem_bytes) {
     const int n = fr->frame_len;
-    if (fr->dtype != VBX_F32 || L < 2 || L > kLpcaMaxLags || fr->frame_stride > (int64_t)n || lpc_force_generic()) return false;
+    if (fr->dtype != VBX_F32 || L < 2 || L > kLpcaMaxLags || fr->frame_stride > (int64_t)n) return false;
     if (const char* e = getenv("VBX_LPCP"))
-        if (atoi(e) == 0) return false;
-    if (const char* e = getenv("VBX_LPCA"))
         if (atoi(e) == 0) return false;
     if ((reinterpret_cast<uintptr_t>(fr->base) & 3) != 0) return false;
     const int sv = (int)fr->frame_stride;
@@ -587,6 +572,5 @@ bool plan_fusedp(const vbx_ctx* ctx, const vbx_frames* fr, int L, LpcParams* P, 
     X->chunks = C;
     X->span_floats = span_floats;
     *smem_bytes = bytes;
-    *n_tiles = (int)tiles;
     return true;
 }
