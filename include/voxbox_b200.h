@@ -266,8 +266,9 @@ VBX_API int vbx_find_formants_host(vbx_ctx* ctx, const vbx_frames* frames, doubl
  * the returned Vec (stable; the unvoiced candidate {0, threshold} is always part of it), zero padded;
  * n_cand_out[f] (optional) = length of the reference's Vec (may exceed max_candidates: the list is truncated);
  * status_out[f] (optional) = VBX_ERR_PITCH where a strength is NaN (the reference panics in its sort) — such frames
- * return their candidates unsorted.  The lag sweep runs on the FP32 FMA pipe (fp64 partial-sum folding), everything
- * after it in fp64.  frame_len <= 16384. */
+ * return their candidates unsorted.  Everything runs in fp64: the sweep over all frame_len lags and the refinement.
+ * 2 <= frame_len <= 16384 (Praat's three periods of the pitch floor: 11 520 samples for 50 Hz at 192 kHz); other lengths
+ * are VBX_ERR_BADARG. */
 VBX_API int vbx_pitch(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate, double threshold, double min_hz,
                       double max_hz, int32_t max_candidates, void* cand_out, int32_t* n_cand_out, uint8_t* status_out,
                       int32_t out_dtype);

@@ -760,10 +760,11 @@ int launch_pitch(vbx_ctx* ctx, const vbx_frames* fr, double fs, double threshold
     int threads = ((fpc * P.lpf + 31) / 32) * 32;
     if (threads < 64) threads = 64;
     const size_t smem = fpc * frame_bytes;
-    VBX_REQUIRE(ctx, smem <= ctx->smem_optin && threads <= 256, "frame_len %d does not fit the pitch kernel", n);
-    const bool lag_small = threads <= 160;
-    if (lag_small) VBX_CUDA(ctx, cudaFuncSetAttribute(pitch_lag64_kernel<TIn, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    else VBX_CUDA(ctx, cudaFuncSetAttribute(pitch_lag64_kernel<TIn, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    VBX_REQUIRE(ctx, smem <= ctx->smem_optin && threads <= 512, "frame_len %d does not fit the pitch kernel", n);
+    void (*lag_kernel)(const PitchParams) = threads <= 160   ? pitch_lag64_kernel<TIn, 160>
+                                            : threads <= 256 ? pitch_lag64_kernel<TIn, 256>
+                                                             : pitch_lag64_kernel<TIn, 512>;
+    VBX_CUDA(ctx, cudaFuncSetAttribute(lag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 
     // scratch per frame: y [N] f64 + worst-case candidate capacity (every other lag below N/2 a maximum)
     const int cap = P.ixmax / 2 + 1;
@@ -806,8 +807,7 @@ int launch_pitch(vbx_ctx* ctx, const vbx_frames* fr, double fs, double threshold
         VBX_CUDA(ctx, cudaMemsetAsync(P.counter, 0, 2 * sizeof(unsigned long long), ctx->stream));
         const int64_t grid = (P.n_frames + fpc - 1) / fpc;
         VBX_REQUIRE(ctx, grid <= 0x7fffffffLL, "too many frames for one launch");
-        if (lag_small) pitch_lag64_kernel<TIn, true><<<(unsigned)grid, threads, smem, ctx->stream>>>(P);
-        else pitch_lag64_kernel<TIn, false><<<(unsigned)grid, threads, smem, ctx->stream>>>(P);
+        lag_kernel<<<(unsigned)grid, threads, smem, ctx->stream>>>(P);
         VBX_CHECK_LAUNCH(ctx, "pitch_lag64_kernel");
         if (lag_out) {  // vbx_pitch_lag_function: hand the lag function out and stop here
             VBX_CUDA(ctx, cudaMemcpyAsync(lag_out + (size_t)f0 * n, P.y, (size_t)P.n_frames * n * sizeof(double), cudaMemcpyDeviceToDevice,

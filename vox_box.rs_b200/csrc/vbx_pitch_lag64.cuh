@@ -39,9 +39,12 @@ __device__ __forceinline__ void lag_step64(double (&acc)[16], const D8& A, const
     }
 }
 
-// SMALL: CTAs of at most 160 threads (every frame length up to 5 120 samples) — four of them per SM (96 registers)
-template <typename TIn, bool SMALL>
-__global__ void __launch_bounds__(SMALL ? 160 : 256, SMALL ? 4 : 1) pitch_lag64_kernel(const PitchParams P) {
+// CTA-size class MAXT, the smallest that holds a CTA's fpc·lpf lanes (launch_pitch picks it from the frame length):
+//   160: frame lengths up to 5 120 samples, four CTAs per SM (96 registers);
+//   256: up to 8 192, one CTA per SM (108 registers);
+//   512: up to 16 384, the longest frame vbx_pitch accepts, one CTA per SM (106 registers).
+template <typename TIn, int MAXT>
+__global__ void __launch_bounds__(MAXT, MAXT == 160 ? 4 : 1) pitch_lag64_kernel(const PitchParams P) {
     extern __shared__ __align__(16) double xd_all[];
     const int tid = threadIdx.x, nthreads = blockDim.x;
     const int n = P.n;
