@@ -51,7 +51,17 @@ typedef enum vbx_status {
     VBX_ERR_NOMEM = 7       /* device or pinned allocation failed                                      */
 } vbx_status;
 
-typedef enum vbx_dtype { VBX_F32 = 0, VBX_F64 = 1, VBX_I16 = 2 } vbx_dtype;
+/* VBX_MULAW8 / VBX_ALAW8: one byte per sample, ITU-T G.711 mu-law / A-law (WAV format tags 7 / 6), accepted wherever
+ * vbx_frames.dtype accepts VBX_I16 (never as out_dtype, nor by the entry points that take plain arrays).  A code decodes to
+ * the 16-bit linear value of G.711 (the g711.c tables; Python's audioop.ulaw2lin / alaw2lin with width 2), range +-32124
+ * (mu-law) / +-32256 (A-law):
+ *   mu-law: u = ~b; t = ((u & 0x0F) << 3) + 0x84; t <<= (u & 0x70) >> 4; v = (u & 0x80) ? 0x84 - t : t - 0x84
+ *   A-law:  a = b ^ 0x55; t = (a & 0x0F) << 4; seg = (a & 0x70) >> 4; t += seg ? 0x108 : 8; if (seg > 1) t <<= seg - 1;
+ *           v = (a & 0x80) ? t : -t
+ * The decode happens as the kernels load the samples; from there on a G.711 sample IS the VBX_I16 sample v (scaled by
+ * 1/32767): every call on a G.711 view returns, bit for bit, what the same call returns on a VBX_I16 view of the decoded
+ * samples. */
+typedef enum vbx_dtype { VBX_F32 = 0, VBX_F64 = 1, VBX_I16 = 2, VBX_MULAW8 = 3, VBX_ALAW8 = 4 } vbx_dtype;
 
 /* Window applied while a frame is loaded (the reference's callers window the
  * frame before calling the trait method):
@@ -74,9 +84,10 @@ typedef enum vbx_window {
  * A batch of equally long utterances is a two-level view: with frames_per_segment = J > 0, frame
  * f = u*J + j starts at base[u*segment_stride + j*frame_stride] (n_frames must be a multiple of J);
  * frames_per_segment == 0 means one segment holds all frames.
- * dtype: VBX_F32 samples, VBX_I16 PCM scaled by 1/32767 on load (tests/lib.rs:17-19), or VBX_F64 samples (what the
- * reference's f64 callers hold, e.g. a frame they windowed themselves: use VBX_WINDOW_NONE; f64 samples run the same
- * arithmetic through the general-purpose kernels, the tuned batch kernels stage fp32 / int16). */
+ * dtype: VBX_F32 samples, VBX_I16 PCM scaled by 1/32767 on load (tests/lib.rs:17-19), VBX_MULAW8 / VBX_ALAW8 G.711 bytes
+ * (decoded to int16 PCM on load, then exactly VBX_I16), or VBX_F64 samples (what the reference's f64 callers hold, e.g. a
+ * frame they windowed themselves: use VBX_WINDOW_NONE; f64 samples run the same arithmetic through the general-purpose
+ * kernels, the tuned batch kernels stage fp32 / int16 / G.711).  Strides are in samples whatever the sample size. */
 typedef struct vbx_frames {
     const void* base;
     int64_t n_frames;
@@ -84,7 +95,7 @@ typedef struct vbx_frames {
     int64_t frames_per_segment; /* J, or 0 */
     int64_t segment_stride;     /* in samples; ignored when frames_per_segment == 0 */
     int32_t frame_len;          /* N */
-    int32_t dtype;        /* vbx_dtype: VBX_F32, VBX_I16 or VBX_F64 */
+    int32_t dtype;        /* vbx_dtype: VBX_F32, VBX_I16, VBX_MULAW8, VBX_ALAW8 or VBX_F64 */
     int32_t window;       /* vbx_window */
     int32_t reserved;     /* must be 0 */
 } vbx_frames;
@@ -278,7 +289,8 @@ VBX_API int vbx_pitch_host(vbx_ctx* ctx, const vbx_frames* frames, double sample
 /* Opt-in extension: the reference's local_peak / global_peak honoured (periodic.rs:357 takes them, :396 ignores them).  In
  * Boersma (1993), the algorithm vbx_pitch implements, they make a quiet frame unvoiced: every frame is normalised (periodic.rs:404),
  * so without them a faint periodic component scores as high as loud speech.
- *  - local peak of frame f: max |x| over its frame_len samples as loaded (VBX_I16 scaled by 1/32767), before frames->window.
+ *  - local peak of frame f: max |x| over its frame_len samples as loaded (VBX_I16 and decoded G.711 scaled by 1/32767), before
+ *    frames->window.
  *    NaN samples are ignored (a NaN never wins the max, as in max_amplitude, waves.rs:45-58); an all-NaN frame has peak 0.
  *  - global peak of segment u: the same max over every sample its frames span, [u*segment_stride, u*segment_stride +
  *    (J-1)*frame_stride + frame_len) (with hop > frame_len this includes the samples between frames); for a single-segment view,
@@ -365,7 +377,7 @@ VBX_API int vbx_preemphasis(vbx_ctx* ctx, void* x_inout, int32_t dtype, int64_t 
 
 /* ---- lib.rs:40-116 find_formants with resample_ratio != 1 (lib.rs:57-61: sample::interpolate::Linear +
  * Converter::scale_sample_hz) ---------------------------------------------------------------------------------------- */
-/* Every frame of the view (VBX_F32, VBX_I16 or VBX_F64 samples, frames->window = VBX_WINDOW_NONE) is resampled linearly to
+/* Every frame of the view (VBX_F32, VBX_I16, G.711 or VBX_F64 samples, frames->window = VBX_WINDOW_NONE) is resampled linearly to
  * ceil(resample_ratio * frame_len) f64 samples, then windowed with the periodic Hann of that length and run through Burg ->
  * roots -> resonances -> McCandless exactly as vbx_find_formants(.., VBX_LPC_BURG, ..).  sample_rate is passed to
  * Resonance::from_root unchanged, as the reference does (callers pass the resampled rate).  The reference analyses its whole
@@ -420,7 +432,9 @@ VBX_API int vbx_multi_mfcc_host(vbx_multi* m, const vbx_frames* frames, int32_t 
 VBX_API int vbx_multi_h2d_bandwidth(vbx_multi* m, size_t bytes_per_device, int32_t reps, int32_t n_active, double* gbs_out);
 
 /* ---- synthetic speech-like audio, generated on the device (bench / parity-at-scale infrastructure; SURVEY 8d) ----------------
- * out: [n_utts][n_samples] of dtype (VBX_F32, or VBX_I16 = the same samples as 16-bit PCM, round(x * 32767)).  Utterance u of the
+ * out: [n_utts][n_samples] of dtype (VBX_F32, or VBX_I16 = the same samples as 16-bit PCM, round(x * 32767), or VBX_MULAW8 /
+ * VBX_ALAW8 = those int16 samples G.711-encoded as audioop.lin2ulaw / lin2alaw(x, 2) do: g711.c's 14-bit mu-law encoder on
+ * x >> 2, its 13-bit A-law encoder on x >> 3).  Utterance u of the
  * call is global utterance first_utt + u: a function of (seed, first_utt + u, sample_rate) only.  Recipe: csrc/vbx_synth.cu. */
 VBX_API int vbx_synth_speech(vbx_ctx* ctx, void* out, int32_t dtype, int64_t n_utts, int64_t n_samples, double sample_rate,
                              uint64_t seed, int64_t first_utt);

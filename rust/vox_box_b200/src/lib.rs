@@ -74,6 +74,9 @@ pub mod ffi {
     pub const VBX_F32: i32 = 0;
     pub const VBX_F64: i32 = 1;
     pub const VBX_I16: i32 = 2;
+    /// G.711 mu-law / A-law bytes, decoded to int16 PCM as the kernels load them (frame views only)
+    pub const VBX_MULAW8: i32 = 3;
+    pub const VBX_ALAW8: i32 = 4;
     pub const VBX_WINDOW_NONE: i32 = 0;
     pub const VBX_WINDOW_HANN_SYMMETRIC: i32 = 1;
     pub const VBX_WINDOW_HANN_PERIODIC: i32 = 2;

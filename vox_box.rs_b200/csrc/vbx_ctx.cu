@@ -164,7 +164,7 @@ void vbx_window_fill_host(int kind, int n, double* out) {
 }
 
 int vbx_get_window(vbx_ctx* ctx, int kind, int n, const double** dev_out, int sample_dtype) {
-    const bool pcm = (sample_dtype == VBX_I16);
+    const bool pcm = vbx_dtype_is_pcm(sample_dtype);
     uint64_t key = ((uint64_t)(uint32_t)(kind | (pcm ? 0x100 : 0)) << 32) | (uint32_t)n;
     auto it = ctx->windows.find(key);
     if (it != ctx->windows.end()) {
@@ -193,8 +193,9 @@ int vbx_check_frames(vbx_ctx* ctx, const vbx_frames* fr, bool allow_f64) {
     VBX_REQUIRE(ctx, fr->n_frames >= 0, "n_frames < 0");
     VBX_REQUIRE(ctx, fr->frame_len >= 1, "frame_len must be >= 1 (the reference indexes self[0])");
     VBX_REQUIRE(ctx, fr->frame_stride >= 1, "frame_stride must be >= 1");
-    VBX_REQUIRE(ctx, fr->dtype == VBX_F32 || fr->dtype == VBX_I16 || (allow_f64 && fr->dtype == VBX_F64),
-                allow_f64 ? "frames dtype must be VBX_F32, VBX_I16 or VBX_F64" : "frames dtype must be VBX_F32 or VBX_I16");
+    VBX_REQUIRE(ctx, fr->dtype == VBX_F32 || vbx_dtype_is_pcm(fr->dtype) || (allow_f64 && fr->dtype == VBX_F64),
+                allow_f64 ? "frames dtype must be VBX_F32, VBX_I16, VBX_MULAW8, VBX_ALAW8 or VBX_F64"
+                          : "frames dtype must be VBX_F32, VBX_I16, VBX_MULAW8 or VBX_ALAW8");
     VBX_REQUIRE(ctx, fr->window >= VBX_WINDOW_NONE && fr->window <= VBX_WINDOW_HANN_PERIODIC, "unknown window kind");
     VBX_REQUIRE(ctx, fr->reserved == 0, "frames.reserved must be 0");
     VBX_REQUIRE(ctx, fr->frames_per_segment >= 0, "frames_per_segment < 0");

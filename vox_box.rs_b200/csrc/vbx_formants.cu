@@ -933,6 +933,8 @@ int vbx_lpc_burg(vbx_ctx* ctx, const vbx_frames* frames, int32_t p, void* coeffs
     VBX_REQUIRE(ctx, coeffs_out != nullptr, "coeffs_out is NULL");
     cudaSetDevice(ctx->device);
     if (frames->dtype == VBX_I16) return launch_burg<int16_t>(ctx, frames, p, coeffs_out, status_out, out_dtype);
+    if (frames->dtype == VBX_MULAW8) return launch_burg<vbx_mulaw8>(ctx, frames, p, coeffs_out, status_out, out_dtype);
+    if (frames->dtype == VBX_ALAW8) return launch_burg<vbx_alaw8>(ctx, frames, p, coeffs_out, status_out, out_dtype);
     if (frames->dtype == VBX_F64) return launch_burg<double>(ctx, frames, p, coeffs_out, status_out, out_dtype);
     return launch_burg<float>(ctx, frames, p, coeffs_out, status_out, out_dtype);
 }
@@ -1401,6 +1403,14 @@ extern "C" int vbx_find_formants_buffered(vbx_ctx* ctx, const vbx_frames* frames
             resample_kernel<int16_t><<<(unsigned)grid, 256, 0, ctx->stream>>>((const int16_t*)frames->base, F, frames->frame_stride, J,
                                                                            seg_stride, n, 1.0 / 32767.0, d_idx, d_w, rlen, wn, row_len,
                                                                            copy_only, d_out);
+        else if (frames->dtype == VBX_MULAW8)
+            resample_kernel<vbx_mulaw8><<<(unsigned)grid, 256, 0, ctx->stream>>>((const vbx_mulaw8*)frames->base, F, frames->frame_stride,
+                                                                              J, seg_stride, n, 1.0 / 32767.0, d_idx, d_w, rlen, wn,
+                                                                              row_len, copy_only, d_out);
+        else if (frames->dtype == VBX_ALAW8)
+            resample_kernel<vbx_alaw8><<<(unsigned)grid, 256, 0, ctx->stream>>>((const vbx_alaw8*)frames->base, F, frames->frame_stride,
+                                                                             J, seg_stride, n, 1.0 / 32767.0, d_idx, d_w, rlen, wn,
+                                                                             row_len, copy_only, d_out);
         else if (frames->dtype == VBX_F64)
             resample_kernel<double><<<(unsigned)grid, 256, 0, ctx->stream>>>((const double*)frames->base, F, frames->frame_stride, J,
                                                                           seg_stride, n, 1.0, d_idx, d_w, rlen, wn, row_len, copy_only, d_out);

@@ -90,8 +90,11 @@ int vbx_pipe_reserve(vbx_ctx* ctx, size_t bytes);          // ensures ctx->pipe 
 // null; and the same max over the whole extent of a host view (the global peak of a single-segment view)
 int vbx_launch_frame_peaks(vbx_ctx* ctx, const vbx_frames* fr, double* local_out, double* global_out);
 double vbx_host_peak(const vbx_frames* fr);
-// cached device table (ones for NONE).  sample_dtype == VBX_I16 folds the PCM scale into the table: w[i] / 32767
-// (tests/lib.rs:17-19 scale every sample by 1/(i32::MAX >> 16) before any arithmetic).
+// sample dtypes whose samples load as integer PCM values (int16, or G.711 decoded to int16): their 1/32767 scale lives in the
+// window table
+static inline bool vbx_dtype_is_pcm(int dt) { return dt == VBX_I16 || dt == VBX_MULAW8 || dt == VBX_ALAW8; }
+// cached device table (ones for NONE).  An integer-PCM sample_dtype folds the PCM scale into the table: w[i] / 32767
+// (tests/lib.rs:17-19 scale every sample by 1/(i32::MAX >> 16) before any arithmetic).  int16 and G.711 views share it.
 int vbx_get_window(vbx_ctx* ctx, int kind, int n, const double** dev_out, int sample_dtype = VBX_F32);
 void vbx_window_fill_host(int kind, int n, double* out);
 
@@ -117,7 +120,9 @@ void vbx_window_fill_host(int kind, int n, double* out);
         if (!(cond)) return vbx_fail((ctx), VBX_ERR_BADARG, __VA_ARGS__);                            \
     } while (0)
 
-static inline size_t vbx_dtype_size(int dt) { return dt == VBX_F64 ? 8 : (dt == VBX_I16 ? 2 : 4); }
+static inline size_t vbx_dtype_size(int dt) {
+    return dt == VBX_F64 ? 8 : (dt == VBX_I16 ? 2 : ((dt == VBX_MULAW8 || dt == VBX_ALAW8) ? 1 : 4));
+}
 
 // validates a vbx_frames descriptor (device or host pointers alike)
 int vbx_check_frames(vbx_ctx* ctx, const vbx_frames* fr, bool allow_f64 = false);
@@ -137,10 +142,78 @@ static inline int64_t vbx_frames_extent(const vbx_frames* fr) {
 #ifdef __CUDACC__
 template <typename T> __device__ __forceinline__ T vbx_ldg(const T* p) { return __ldg(p); }
 
-// sample load with dtype dispatch (F32, or raw I16 PCM: the 1/32767 scale lives in the window table, vbx_get_window)
+// G.711 (VBX_MULAW8 / VBX_ALAW8): one byte per sample.  The tag types give the kernels one instantiation per law.
+struct vbx_mulaw8 { uint8_t code; };
+struct vbx_alaw8 { uint8_t code; };
+
+// code -> the 16-bit linear value of ITU-T G.711 (g711.c's ulaw2linear / alaw2linear).  Arithmetic rather than a table: the
+// 32 lanes of a warp load 32 different codes, which a constant-memory table would serialise.
+__host__ __device__ __forceinline__ int vbx_mulaw_decode(unsigned b) {
+    const unsigned u = ~b & 0xffu;
+    const int t = (int)(((u & 0x0fu) << 3) + 0x84u) << ((u & 0x70u) >> 4);
+    return (u & 0x80u) ? 0x84 - t : t - 0x84;
+}
+__host__ __device__ __forceinline__ int vbx_alaw_decode(unsigned b) {
+    const unsigned a = (b ^ 0x55u) & 0xffu;
+    const unsigned seg = (a & 0x70u) >> 4;
+    int t = (int)((a & 0x0fu) << 4) + (seg ? 0x108 : 8);
+    if (seg > 1) t <<= seg - 1;
+    return (a & 0x80u) ? t : -t;
+}
+// int16 -> code, as audioop.lin2ulaw / lin2alaw(x, 2): g711.c's 14-bit mu-law encoder on x >> 2, 13-bit A-law encoder on x >> 3
+__host__ __device__ __forceinline__ unsigned vbx_mulaw_encode(int x) {
+    int v = x >> 2;
+    unsigned mask = 0xffu;
+    if (v < 0) { v = -v; mask = 0x7fu; }
+    if (v > 8159) v = 8159;
+    v += 0x84 >> 2;
+    int seg = 0;
+    while (seg < 8 && v > (0x40 << seg) - 1) ++seg;  // seg_uend = {0x3F, 0x7F, ..., 0x1FFF}
+    if (seg >= 8) return 0x7fu ^ mask;
+    return (((unsigned)seg << 4) | (((unsigned)v >> (seg + 1)) & 0x0fu)) ^ mask;
+}
+__host__ __device__ __forceinline__ unsigned vbx_alaw_encode(int x) {
+    int v = x >> 3;
+    unsigned mask = 0xd5u;
+    if (v < 0) { v = -v - 1; mask = 0x55u; }
+    int seg = 0;
+    while (seg < 8 && v > (0x20 << seg) - 1) ++seg;  // seg_aend = {0x1F, 0x3F, ..., 0xFFF}
+    if (seg >= 8) return 0x7fu ^ mask;
+    const unsigned q = seg < 2 ? ((unsigned)v >> 1) & 0x0fu : ((unsigned)v >> seg) & 0x0fu;
+    return (((unsigned)seg << 4) | q) ^ mask;
+}
+
+template <typename TIn> struct vbx_g711 { static constexpr bool value = false; };
+template <> struct vbx_g711<vbx_mulaw8> { static constexpr bool value = true; };
+template <> struct vbx_g711<vbx_alaw8> { static constexpr bool value = true; };
+// sample types that load as integer PCM values (the 1/32767 scale lives in the window table)
+template <typename TIn> struct vbx_pcm { static constexpr bool value = vbx_g711<TIn>::value; };
+template <> struct vbx_pcm<int16_t> { static constexpr bool value = true; };
+
+// the value of one G.711 code (the low byte of `code`)
+template <typename TIn> __device__ __forceinline__ float vbx_decode8(unsigned code);
+template <> __device__ __forceinline__ float vbx_decode8<vbx_mulaw8>(unsigned code) { return (float)vbx_mulaw_decode(code & 0xffu); }
+template <> __device__ __forceinline__ float vbx_decode8<vbx_alaw8>(unsigned code) { return (float)vbx_alaw_decode(code & 0xffu); }
+// the 16 samples of one 16-byte load of G.711 codes, in memory order
+template <typename TIn> __device__ __forceinline__ void vbx_decode16(const uint4& v, float (&x)[16]) {
+    const unsigned w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+    for (int h = 0; h < 4; ++h)
+#pragma unroll
+        for (int b = 0; b < 4; ++b) x[4 * h + b] = vbx_decode8<TIn>(w[h] >> (8 * b));
+}
+
+// sample load with dtype dispatch (F32, raw I16 PCM, or G.711 decoded to the int16 value: the 1/32767 scale lives in the
+// window table, vbx_get_window)
 template <typename TIn> __device__ __forceinline__ float vbx_load_sample(const TIn* p);
 template <> __device__ __forceinline__ float vbx_load_sample<float>(const float* p) { return __ldg(p); }
 template <> __device__ __forceinline__ float vbx_load_sample<int16_t>(const int16_t* p) { return (float)__ldg(p); }
+template <> __device__ __forceinline__ float vbx_load_sample<vbx_mulaw8>(const vbx_mulaw8* p) {
+    return vbx_decode8<vbx_mulaw8>(__ldg(reinterpret_cast<const unsigned char*>(p)));
+}
+template <> __device__ __forceinline__ float vbx_load_sample<vbx_alaw8>(const vbx_alaw8* p) {
+    return vbx_decode8<vbx_alaw8>(__ldg(reinterpret_cast<const unsigned char*>(p)));
+}
 // double-valued loader for the paths that also accept f64 samples (Burg / find_formants)
 template <typename TIn> __device__ __forceinline__ double vbx_load_sample_d(const TIn* p) { return (double)vbx_load_sample<TIn>(p); }
 template <> __device__ __forceinline__ double vbx_load_sample_d<double>(const double* p) { return __ldg(p); }

@@ -214,6 +214,32 @@ __global__ void __launch_bounds__(kMaxThreads, (L <= 13 ? 5 : 1)) lpc_fused_kern
             }
             done = n8 << 3;
         }
+        if constexpr (vbx_g711<TIn>::value) {
+            if ((reinterpret_cast<uintptr_t>(src) & 15) == 0) {
+                // G.711: 16-byte loads of 16 codes, 4 in flight per thread, decoded as they land
+                const uint4* src16 = reinterpret_cast<const uint4*>(src);
+                const int n16 = total >> 4;
+                for (int v0 = tid; v0 < n16; v0 += 4 * nthreads) {
+                    uint4 a[4];
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        const int v = v0 + u * nthreads;
+                        if (v < n16) a[u] = __ldg(src16 + v);
+                    }
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        const int v = v0 + u * nthreads;
+                        if (v < n16) {
+                            float x[16];
+                            vbx_decode16<TIn>(a[u], x);
+#pragma unroll
+                            for (int e = 0; e < 16; ++e) s_span[phys(16 * v + e)] = x[e];
+                        }
+                    }
+                }
+                done = n16 << 4;
+            }
+        }
         for (int s0 = done + tid; s0 < total; s0 += 8 * nthreads) {
             float a[8];
 #pragma unroll
@@ -438,7 +464,7 @@ void fill_table(T* t, Make make) {
 // The two shifted window rows of lpc_fuseda_kernel, E = [0, 0, w…, 0…] and O = [0, 0, 0, w…, 0…] ([2][wt] f64), cached per
 // (window kind, n, sample dtype) next to the plain tables.
 int get_window_rows_aligned(vbx_ctx* ctx, int kind, int n, int wt, const double** dev_out, int sample_dtype) {
-    const bool pcm = (sample_dtype == VBX_I16);
+    const bool pcm = vbx_dtype_is_pcm(sample_dtype);
     const uint64_t key = ((uint64_t)(uint32_t)(kind | (pcm ? 0x100 : 0) | 0x200) << 32) | (uint32_t)n;
     auto it = ctx->windows.find(key);
     if (it != ctx->windows.end()) {
@@ -604,7 +630,7 @@ LpcPlan plan_lpc(const vbx_ctx* ctx, const vbx_frames* fr, int L) {
     return pl;
 }
 
-// Launches the fused kernel a plan names.  Instantiated for fp32 and int16 samples: plan_lpc sends f64 samples to the
+// Launches the fused kernel a plan names.  Instantiated for fp32, int16 and G.711 samples: plan_lpc sends f64 samples to the
 // generic kernels.
 template <typename TIn>
 int launch_fused(vbx_ctx* ctx, const vbx_frames* fr, int L, LpcPlan& pl) {
@@ -716,6 +742,10 @@ int lpc_dispatch(vbx_ctx* ctx, const vbx_frames* fr, int n_lags, void* r_out, vo
     cudaSetDevice(ctx->device);
     if (fr->dtype == VBX_I16)
         return launch_lpc<int16_t>(ctx, fr, n_lags, r_out, ac_out, kc_out, out_dtype, do_levinson);
+    if (fr->dtype == VBX_MULAW8)
+        return launch_lpc<vbx_mulaw8>(ctx, fr, n_lags, r_out, ac_out, kc_out, out_dtype, do_levinson);
+    if (fr->dtype == VBX_ALAW8)
+        return launch_lpc<vbx_alaw8>(ctx, fr, n_lags, r_out, ac_out, kc_out, out_dtype, do_levinson);
     if (fr->dtype == VBX_F64)
         return launch_lpc<double>(ctx, fr, n_lags, r_out, ac_out, kc_out, out_dtype, do_levinson);
     return launch_lpc<float>(ctx, fr, n_lags, r_out, ac_out, kc_out, out_dtype, do_levinson);

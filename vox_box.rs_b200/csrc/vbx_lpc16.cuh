@@ -69,6 +69,33 @@ __device__ __forceinline__ void stage_span16(const LpcParams& P, const TIn* __re
             }
             done = n8 << 3;
         }
+        if constexpr (vbx_g711<TIn>::value) {
+            if ((reinterpret_cast<uintptr_t>(src) & 15) == 0) {
+                // G.711: 16-byte loads of 16 codes, decoded as they land (never straddling a pad: sv % 16 == 0)
+                const uint4* src16 = reinterpret_cast<const uint4*>(src);
+                const int n16 = total >> 4;
+                for (int v0 = tid; v0 < n16; v0 += 4 * nthreads) {
+                    uint4 a[4];
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        const int v = v0 + u * nthreads;
+                        if (v < n16) a[u] = __ldg(src16 + v);
+                    }
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        const int v = v0 + u * nthreads;
+                        if (v < n16) {
+                            float x[16];
+                            vbx_decode16<TIn>(a[u], x);
+                            float4* dst = reinterpret_cast<float4*>(s_span + phys(16 * v));
+#pragma unroll
+                            for (int e = 0; e < 4; ++e) dst[e] = make_float4(x[4 * e], x[4 * e + 1], x[4 * e + 2], x[4 * e + 3]);
+                        }
+                    }
+                }
+                done = n16 << 4;
+            }
+        }
         for (int s0 = done + tid; s0 < total; s0 += 8 * nthreads) {  // unaligned base pointer
             float a[8];
 #pragma unroll

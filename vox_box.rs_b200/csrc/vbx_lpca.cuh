@@ -91,7 +91,7 @@ __global__ void __launch_bounds__(256) lpc_fuseda_kernel(const LpcParams P, cons
     const int64_t g0 = seg * P.seg_frames + j0;                            // ... and in the batch (output row)
     const int Gc = (int)min((int64_t)G, P.seg_frames - j0);
     const TIn* __restrict__ src = reinterpret_cast<const TIn*>(P.base) + seg * P.seg_stride + j0 * P.stride;
-    constexpr int A = 16 / (int)sizeof(TIn);                               // samples per 16-byte load (4 or 8)
+    constexpr int A = 16 / (int)sizeof(TIn);                               // samples per 16-byte load (4, 8 or 16)
     const int mis = (int)((reinterpret_cast<uintptr_t>(src) / sizeof(TIn)) & (A - 1));
     const TIn* __restrict__ src_al = src - mis;                            // 16-byte aligned
 
@@ -102,7 +102,7 @@ __global__ void __launch_bounds__(256) lpc_fuseda_kernel(const LpcParams P, cons
         for (int i = tid; i < X.wt; i += nthreads) d2[i] = __ldg(t2 + i);   // 2·wt doubles = wt double2
     }
     const int first = mis, last = mis + (Gc - 1) * sv + n;                  // real samples are words [first, last)
-    const int total = X.span_floats;                                        // multiple of 8
+    const int total = X.span_floats;                                        // multiple of max(A, 8)
     bool bad = false;
     if (sizeof(TIn) == 4) {
         const int nv = total >> 2;
@@ -133,6 +133,35 @@ __global__ void __launch_bounds__(256) lpc_fuseda_kernel(const LpcParams P, cons
                     const unsigned m = 0x7f800000u;
                     bad = bad || ((e0 & m) == m) || ((e1 & m) == m) || ((e2 & m) == m) || ((e3 & m) == m);
                 }
+            }
+        }
+    } else if constexpr (vbx_g711<TIn>::value) {
+        // G.711: 16-byte loads of 16 codes, decoded as they land (always finite); two loads in flight per thread hold as many
+        // samples as the four of int16 (four spill registers at 10 / 11 lags)
+        const int nv = total >> 4;
+        for (int v0 = tid; v0 < nv; v0 += 2 * nthreads) {
+            uint4 a[2];
+            bool whole[2];
+#pragma unroll
+            for (int u = 0; u < 2; ++u) {
+                const int v = v0 + u * nthreads, s = 16 * v;
+                whole[u] = (v < nv) && (s >= first && s + 16 <= last);
+                if (whole[u]) a[u] = __ldg(reinterpret_cast<const uint4*>(src_al) + v);
+            }
+#pragma unroll
+            for (int u = 0; u < 2; ++u) {
+                const int v = v0 + u * nthreads, s = 16 * v;
+                if (v >= nv) continue;
+                float e[16];
+                if (whole[u]) {
+                    vbx_decode16<TIn>(a[u], e);
+                } else {
+#pragma unroll
+                    for (int k = 0; k < 16; ++k) e[k] = (s + k >= first && s + k < last) ? vbx_load_sample<TIn>(src_al + s + k) : 0.f;
+                }
+                float4* dst = reinterpret_cast<float4*>(s_span + s);
+#pragma unroll
+                for (int k = 0; k < 4; ++k) dst[k] = make_float4(e[4 * k], e[4 * k + 1], e[4 * k + 2], e[4 * k + 3]);
             }
         }
     } else {
@@ -246,9 +275,10 @@ bool plan_fuseda(const vbx_ctx* ctx, int n, int64_t stride, int L, size_t in_siz
     }
     while (K > 1 && C / K < 2) K >>= 1;  // every part at least two chunks
     if ((G * K) % 32 != 0) return false;
-    const int A = 16 / (int)in_size;
+    const int A = 16 / (int)in_size;  // samples per 16-byte load: the staging pass copies whole loads
     const int64_t span = (int64_t)(A - 1) + (int64_t)(G - 1) * sv + (int64_t)C * kChunk + 3;
-    const int span_floats = (int)((span + 7) & ~(int64_t)7);
+    const int64_t round = A > 8 ? A : 8;
+    const int span_floats = (int)((span + round - 1) & ~(round - 1));
     const int wt = C * kChunk + 4;
     const size_t stage_bytes = (size_t)G * ((3 * L - 1) + (size_t)(K - 1) * L) * sizeof(double);
     size_t span_bytes = (size_t)span_floats * sizeof(float);

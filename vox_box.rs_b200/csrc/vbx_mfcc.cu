@@ -560,6 +560,10 @@ int vbx_mfcc(vbx_ctx* ctx, const vbx_frames* frames, int32_t num_coeffs, int32_t
     cudaSetDevice(ctx->device);
     if (frames->dtype == VBX_I16)
         return launch_mfcc<int16_t>(ctx, frames, num_coeffs, n_keep, freq_lo, freq_hi, sample_rate, out, energies_out, out_dtype);
+    if (frames->dtype == VBX_MULAW8)
+        return launch_mfcc<vbx_mulaw8>(ctx, frames, num_coeffs, n_keep, freq_lo, freq_hi, sample_rate, out, energies_out, out_dtype);
+    if (frames->dtype == VBX_ALAW8)
+        return launch_mfcc<vbx_alaw8>(ctx, frames, num_coeffs, n_keep, freq_lo, freq_hi, sample_rate, out, energies_out, out_dtype);
     if (frames->dtype == VBX_F64)
         return launch_mfcc<double>(ctx, frames, num_coeffs, n_keep, freq_lo, freq_hi, sample_rate, out, energies_out, out_dtype);
     return launch_mfcc<float>(ctx, frames, num_coeffs, n_keep, freq_lo, freq_hi, sample_rate, out, energies_out, out_dtype);

@@ -79,8 +79,15 @@ typedef cxt<double> C;
 template <typename TIn> struct RawPair;
 template <> struct RawPair<float> { typedef float2 type; };
 template <> struct RawPair<int16_t> { typedef short2 type; };
+template <> struct RawPair<vbx_mulaw8> { typedef float2 type; };
+template <> struct RawPair<vbx_alaw8> { typedef float2 type; };
 template <typename TIn> __device__ __forceinline__ typename RawPair<TIn>::type load_raw(const TIn* p) {
-    return __ldg(reinterpret_cast<const typename RawPair<TIn>::type*>(p));
+    if constexpr (vbx_g711<TIn>::value) {  // one 2-byte load of a code pair, decoded
+        const uchar2 c = __ldg(reinterpret_cast<const uchar2*>(p));
+        return make_float2(vbx_decode8<TIn>(c.x), vbx_decode8<TIn>(c.y));
+    } else {
+        return __ldg(reinterpret_cast<const typename RawPair<TIn>::type*>(p));
+    }
 }
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 

@@ -277,7 +277,7 @@ int vbx_multi_pitch_with_peaks_host(vbx_multi* m, const vbx_frames* frames, doub
     double whole = 0.0;
     const double* global = global_peaks;
     if (silence_threshold > 0.0 && !global && !segmented && frames->n_frames > 0 && frames->base && frames->frame_len >= 1 &&
-        frames->frame_stride >= 1 && (frames->dtype == VBX_F32 || frames->dtype == VBX_I16 || frames->dtype == VBX_F64)) {
+        frames->frame_stride >= 1 && (frames->dtype == VBX_F32 || vbx_dtype_is_pcm(frames->dtype) || frames->dtype == VBX_F64)) {
         whole = vbx_host_peak(frames);
         global = &whole;
     }

@@ -1,6 +1,7 @@
 // vbx_peaks.cu — per-frame and per-segment peak amplitudes of a vbx_frames view (vbx_frame_peaks).
 //
-// The local peak of frame f is max |x| over its frame_len samples as loaded (I16 scaled by 1/32767), before any window.
+// The local peak of frame f is max |x| over its frame_len samples as loaded (I16 and decoded G.711 scaled by 1/32767), before
+// any window.
 // The global peak of segment u is the same max over every sample its frames span,
 // [u·segment_stride, u·segment_stride + (J−1)·frame_stride + frame_len): with hop > frame_len that includes the gaps
 // between frames.  NaN samples are skipped (a fold from 0 with `>`, so a NaN never wins; an all-NaN frame has peak 0).
@@ -52,7 +53,7 @@ __global__ void __launch_bounds__(32 * kPeakWarps) frame_peaks_kernel(const TIn*
             if (o > loc) loc = o;
             if (g > glo) glo = g;
         }
-        if constexpr (std::is_same<TIn, int16_t>::value) {  // monotone, so max(|v| / 32767) = max|v| / 32767 exactly
+        if constexpr (vbx_pcm<TIn>::value) {  // monotone, so max(|v| / 32767) = max|v| / 32767 exactly
             loc = loc / 32767.0;
             glo = glo / 32767.0;
         }
@@ -87,6 +88,12 @@ int vbx_launch_frame_peaks(vbx_ctx* ctx, const vbx_frames* fr, double* local_out
     if (fr->dtype == VBX_I16)
         frame_peaks_kernel<int16_t><<<(unsigned)grid, 32 * kPeakWarps, 0, ctx->stream>>>(
             (const int16_t*)fr->base, fr->n_frames, fr->frame_stride, J, seg_stride, fr->frame_len, local_out, g);
+    else if (fr->dtype == VBX_MULAW8)
+        frame_peaks_kernel<vbx_mulaw8><<<(unsigned)grid, 32 * kPeakWarps, 0, ctx->stream>>>(
+            (const vbx_mulaw8*)fr->base, fr->n_frames, fr->frame_stride, J, seg_stride, fr->frame_len, local_out, g);
+    else if (fr->dtype == VBX_ALAW8)
+        frame_peaks_kernel<vbx_alaw8><<<(unsigned)grid, 32 * kPeakWarps, 0, ctx->stream>>>(
+            (const vbx_alaw8*)fr->base, fr->n_frames, fr->frame_stride, J, seg_stride, fr->frame_len, local_out, g);
     else if (fr->dtype == VBX_F64)
         frame_peaks_kernel<double><<<(unsigned)grid, 32 * kPeakWarps, 0, ctx->stream>>>(
             (const double*)fr->base, fr->n_frames, fr->frame_stride, J, seg_stride, fr->frame_len, local_out, g);
@@ -100,11 +107,14 @@ int vbx_launch_frame_peaks(vbx_ctx* ctx, const vbx_frames* fr, double* local_out
 double vbx_host_peak(const vbx_frames* fr) {
     const int64_t extent = vbx_frames_extent(fr);
     double m = 0.0;
-    if (fr->dtype == VBX_I16) {
-        const int16_t* x = (const int16_t*)fr->base;
+    if (vbx_dtype_is_pcm(fr->dtype)) {
         int a = 0;
         for (int64_t i = 0; i < extent; ++i) {
-            const int v = x[i] < 0 ? -(int)x[i] : (int)x[i];
+            int v;
+            if (fr->dtype == VBX_I16) v = ((const int16_t*)fr->base)[i];
+            else if (fr->dtype == VBX_MULAW8) v = vbx_mulaw_decode(((const uint8_t*)fr->base)[i]);
+            else v = vbx_alaw_decode(((const uint8_t*)fr->base)[i]);
+            if (v < 0) v = -v;
             if (v > a) a = v;
         }
         m = (double)a / 32767.0;

@@ -846,6 +846,12 @@ int pitch_check(vbx_ctx* ctx, const vbx_frames* fr, int max_cand, const void* ca
 int launch_pitch_any(vbx_ctx* ctx, const vbx_frames* fr, double fs, double threshold, double fmin, double fmax, int max_cand,
                      void* cand_out, int32_t* n_cand_out, uint8_t* status_out, int out_dtype, double* lag_out, const PitchPeaks& peaks) {
     cudaSetDevice(ctx->device);
+    if (fr->dtype == VBX_MULAW8)
+        return launch_pitch<vbx_mulaw8>(ctx, fr, fs, threshold, fmin, fmax, max_cand, cand_out, n_cand_out, status_out, out_dtype,
+                                        lag_out, peaks);
+    if (fr->dtype == VBX_ALAW8)
+        return launch_pitch<vbx_alaw8>(ctx, fr, fs, threshold, fmin, fmax, max_cand, cand_out, n_cand_out, status_out, out_dtype,
+                                       lag_out, peaks);
     if (fr->dtype == VBX_I16)
         return launch_pitch<int16_t>(ctx, fr, fs, threshold, fmin, fmax, max_cand, cand_out, n_cand_out, status_out, out_dtype, lag_out,
                                      peaks);

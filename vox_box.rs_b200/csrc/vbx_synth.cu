@@ -12,8 +12,10 @@
 // [4200,5500] Hz, bandwidths uniform 50–300 Hz, fixed per utterance, fp64 filter state); the result is scaled to peak 0.5
 // and white noise at −40 dB re peak is added (mandatory: without a noise floor LPC is ill-posed even in f64, SURVEY §7.3).
 // One thread per utterance, counter-based RNG (splitmix64 finaliser over (seed, utterance, stream, index)); two passes:
-// the first finds the peak, the second regenerates the same samples and writes them scaled (fp32, or int16 PCM ·32767).
+// the first finds the peak, the second regenerates the same samples and writes them scaled (fp32, or int16 PCM ·32767, or
+// that int16 PCM G.711-encoded).
 #include <cmath>
+#include <type_traits>
 
 #include "vbx_internal.cuh"
 
@@ -84,12 +86,14 @@ __device__ __forceinline__ double synth_pass(uint64_t seed, uint64_t u, int64_t 
         }
         if (WRITE) {
             const double v = x * scale + 0.005 * (double)rng_normal(seed, u, STREAM_FLOOR, (uint64_t)i);  // −40 dB re the 0.5 peak
-            if (sizeof(TOut) == 2) {
+            if constexpr (std::is_same<TOut, float>::value) {
+                out[i] = v;
+            } else {
                 double q = rint(v * 32767.0);
                 q = q < -32768.0 ? -32768.0 : (q > 32767.0 ? 32767.0 : q);
-                out[i] = (TOut)q;
-            } else {
-                out[i] = (TOut)v;
+                if constexpr (std::is_same<TOut, vbx_mulaw8>::value) out[i].code = (uint8_t)vbx_mulaw_encode((int)q);
+                else if constexpr (std::is_same<TOut, vbx_alaw8>::value) out[i].code = (uint8_t)vbx_alaw_encode((int)q);
+                else out[i] = (TOut)q;
             }
         } else {
             const double a = fabs(x);
@@ -127,7 +131,7 @@ __global__ void __launch_bounds__(64) synth_speech_kernel(TOut* out, int64_t n_u
 extern "C" int vbx_synth_speech(vbx_ctx* ctx, void* out, int32_t dtype, int64_t n_utts, int64_t n_samples, double sample_rate,
                                 uint64_t seed, int64_t first_utt) {
     if (!ctx) return VBX_ERR_BADARG;
-    VBX_REQUIRE(ctx, dtype == VBX_F32 || dtype == VBX_I16, "dtype must be VBX_F32 or VBX_I16");
+    VBX_REQUIRE(ctx, dtype == VBX_F32 || vbx_dtype_is_pcm(dtype), "dtype must be VBX_F32, VBX_I16, VBX_MULAW8 or VBX_ALAW8");
     VBX_REQUIRE(ctx, n_utts >= 0 && n_samples >= 0 && first_utt >= 0, "negative sizes");
     VBX_REQUIRE(ctx, sample_rate >= 8000.0 && sample_rate <= 192000.0, "sample_rate must be in 8000..192000");
     if (n_utts == 0 || n_samples == 0) return VBX_OK;
@@ -137,6 +141,12 @@ extern "C" int vbx_synth_speech(vbx_ctx* ctx, void* out, int32_t dtype, int64_t 
     VBX_REQUIRE(ctx, grid <= 0x7fffffffLL, "too many utterances for one launch");
     if (dtype == VBX_I16)
         synth_speech_kernel<int16_t><<<(unsigned)grid, 64, 0, ctx->stream>>>((int16_t*)out, n_utts, n_samples, sample_rate, seed, first_utt);
+    else if (dtype == VBX_MULAW8)
+        synth_speech_kernel<vbx_mulaw8><<<(unsigned)grid, 64, 0, ctx->stream>>>((vbx_mulaw8*)out, n_utts, n_samples, sample_rate, seed,
+                                                                               first_utt);
+    else if (dtype == VBX_ALAW8)
+        synth_speech_kernel<vbx_alaw8><<<(unsigned)grid, 64, 0, ctx->stream>>>((vbx_alaw8*)out, n_utts, n_samples, sample_rate, seed,
+                                                                              first_utt);
     else
         synth_speech_kernel<float><<<(unsigned)grid, 64, 0, ctx->stream>>>((float*)out, n_utts, n_samples, sample_rate, seed, first_utt);
     VBX_CHECK_LAUNCH(ctx, "synth_speech_kernel");

@@ -17,12 +17,12 @@ LIB_PATH = os.path.join(ROOT, "libvoxbox_b200.so")
 HEADER_PATH = os.path.join(os.path.dirname(ROOT), "include", "voxbox_b200.h")
 
 OK, ERR_LPC, ERR_PITCH, ERR_POLYNOMIAL, ERR_WORKSPACE, ERR_CUDA, ERR_BADARG, ERR_NOMEM = range(8)
-F32, F64, I16 = 0, 1, 2
+F32, F64, I16, MULAW8, ALAW8 = 0, 1, 2, 3, 4  # MULAW8 / ALAW8: G.711 bytes, decoded to int16 PCM on load
 WINDOW_NONE, WINDOW_HANN_SYMMETRIC, WINDOW_HANN_PERIODIC, WINDOW_HANN_LAG = 0, 1, 2, 3
 INTERP_NONE, INTERP_PARABOLIC, INTERP_SINC = 0, 1, 2
 MAX_RESONANCES = 32
 LPC_BURG, LPC_AUTOCORR = 0, 1
-_NP = {F32: np.float32, F64: np.float64, I16: np.int16}
+_NP = {F32: np.float32, F64: np.float64, I16: np.int16, MULAW8: np.uint8, ALAW8: np.uint8}
 
 
 class VoxBoxError(RuntimeError):
@@ -310,17 +310,17 @@ class Context:
         return ac, kc
 
     # -- host-pointer twins (H2D + kernels + D2H inside the call) ------------------------------
-    def autocorrelate_host(self, audio, n_frames, frame_len, stride, window, n_lags, out_dtype=F64):
+    def autocorrelate_host(self, audio, n_frames, frame_len, stride, window, n_lags, out_dtype=F64, sample_dtype=None):
         audio = np.ascontiguousarray(audio)
-        fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, I16 if audio.dtype == np.int16 else F32)
+        fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype))
         r = np.empty((n_frames, n_lags), dtype=_NP[out_dtype])
         self._check(self.lib.vbx_autocorrelate_host(self.h, C.byref(fr), n_lags, r.ctypes.data, out_dtype),
                     "vbx_autocorrelate_host")
         return r
 
-    def lpc_host(self, audio, n_frames, frame_len, stride, window, p, out_dtype=F64, out=None):
+    def lpc_host(self, audio, n_frames, frame_len, stride, window, p, out_dtype=F64, out=None, sample_dtype=None):
         audio = np.ascontiguousarray(audio)
-        fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, I16 if audio.dtype == np.int16 else F32)
+        fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype))
         if out is None:
             out = (np.empty((n_frames, p + 1), dtype=_NP[out_dtype]), np.empty((n_frames, p + 1), dtype=_NP[out_dtype]),
                    np.empty((n_frames, p), dtype=_NP[out_dtype]))
@@ -440,9 +440,9 @@ def _find_formants(self, frames, fs, p, method, estimates, dtype=F64, want_reson
 
 
 def _find_formants_host(self, audio, n_frames, frame_len, stride, window, fs, p, method, estimates, dtype=F64,
-                        frames_per_segment=0, segment_stride=0):
+                        frames_per_segment=0, segment_stride=0, sample_dtype=None):
     audio = np.ascontiguousarray(audio)
-    fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, I16 if audio.dtype == np.int16 else F32,
+    fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype),
                      frames_per_segment, segment_stride)
     J = frames_per_segment or n_frames
     segs = n_frames // J if J else 0
@@ -483,9 +483,9 @@ def _pitch(self, frames, fs, threshold, fmin, fmax, max_cand=16, out_dtype=F64):
 
 
 def _pitch_host(self, audio, n_frames, frame_len, stride, window, fs, threshold, fmin, fmax, max_cand=16, out_dtype=F64,
-                frames_per_segment=0, segment_stride=0):
+                frames_per_segment=0, segment_stride=0, sample_dtype=None):
     audio = np.ascontiguousarray(audio)
-    fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, I16 if audio.dtype == np.int16 else F32,
+    fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype),
                      frames_per_segment, segment_stride)
     cand = np.zeros((n_frames, max_cand, 2), dtype=_NP[out_dtype])
     n = np.zeros(n_frames, dtype=np.int32)
@@ -535,9 +535,32 @@ def _n_segments(n_frames, frames_per_segment):
     return n_frames // frames_per_segment if frames_per_segment else 1
 
 
-def _host_audio(audio):
-    """Host samples and their vbx dtype: int16 PCM, float64, or anything else as float32."""
+def _g711_law(audio, sample_dtype):
+    """sample_dtype of uint8 host samples: G.711 codes carry no mark of their law, so the caller names it (MULAW8 / ALAW8);
+    None for other samples, which must then not claim a law."""
+    if audio.dtype == np.uint8:
+        if sample_dtype not in (MULAW8, ALAW8):
+            raise ValueError("uint8 samples are G.711 codes of an unknown law: pass sample_dtype=MULAW8 or sample_dtype=ALAW8")
+        return sample_dtype
+    if sample_dtype in (MULAW8, ALAW8):
+        raise ValueError(f"sample_dtype {sample_dtype} (G.711) needs uint8 samples, not {audio.dtype}")
+    return None
+
+
+def _sample_dtype(audio, sample_dtype=None):
+    """vbx dtype of the host samples of the int16 / float32 `_host` wrappers: int16 PCM, uint8 G.711 codes, anything else
+    float32."""
+    law = _g711_law(audio, sample_dtype)
+    return law if law is not None else (I16 if audio.dtype == np.int16 else F32)
+
+
+def _host_audio(audio, sample_dtype=None):
+    """Host samples and their vbx dtype: int16 PCM, uint8 G.711 codes (sample_dtype MULAW8 / ALAW8), float64, or anything
+    else as float32."""
     audio = np.asarray(audio)
+    law = _g711_law(audio, sample_dtype)
+    if law is not None:
+        return np.ascontiguousarray(audio), law
     if audio.dtype == np.int16:
         return np.ascontiguousarray(audio), I16
     if audio.dtype == np.float64:
@@ -580,9 +603,10 @@ def _pitch_with_peaks(self, frames, fs, threshold, silence_threshold, fmin, fmax
 
 def _pitch_with_peaks_host(self, audio, n_frames, frame_len, stride, window, fs, threshold, silence_threshold, fmin, fmax,
                            max_cand=16, out_dtype=F64, frames_per_segment=0, segment_stride=0, local_peaks=None,
-                           global_peaks=None):
-    """Host twin of pitch_with_peaks: audio int16 / float32 / float64 samples, peaks host arrays or None."""
-    audio, dt = _host_audio(audio)
+                           global_peaks=None, sample_dtype=None):
+    """Host twin of pitch_with_peaks: audio int16 / float32 / float64 samples (or uint8 G.711 codes with sample_dtype), peaks
+    host arrays or None."""
+    audio, dt = _host_audio(audio, sample_dtype)
     fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, dt, frames_per_segment, segment_stride)
     lp = _host_peaks(local_peaks, n_frames)
     gp = _host_peaks(global_peaks, _n_segments(n_frames, frames_per_segment))
@@ -628,10 +652,10 @@ def _mfcc(self, frames, num_coeffs, f_lo, f_hi, fs, n_keep=None, out_dtype=F64, 
 
 
 def _mfcc_host(self, audio, n_frames, frame_len, stride, window, num_coeffs, f_lo, f_hi, fs, n_keep=None, out_dtype=F64,
-               frames_per_segment=0, segment_stride=0):
+               frames_per_segment=0, segment_stride=0, sample_dtype=None):
     audio = np.ascontiguousarray(audio)
     n_keep = num_coeffs if n_keep is None else n_keep
-    fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, I16 if audio.dtype == np.int16 else F32,
+    fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype),
                      frames_per_segment, segment_stride)
     out = np.zeros((n_frames, n_keep), dtype=_NP[out_dtype])
     self._check(self.lib.vbx_mfcc_host(self.h, C.byref(fr), num_coeffs, n_keep, f_lo, f_hi, fs, out.ctypes.data, out_dtype),
@@ -751,7 +775,8 @@ def _find_formants_buffered(self, frames, fs, ratio, resampled_buf_len, p, estim
 
 
 def _synth_speech(self, n_utts, n_samples, fs, seed=0x5EED, first_utt=0, dtype=F32, out=None):
-    """Synthetic speech-like corpus generated on the device → DeviceArray [n_utts][n_samples] (csrc/vbx_synth.cu)."""
+    """Synthetic speech-like corpus generated on the device → DeviceArray [n_utts][n_samples] (csrc/vbx_synth.cu): dtype F32,
+    I16, or MULAW8 / ALAW8 (the I16 samples G.711-encoded, uint8)."""
     d = out if out is not None else self.empty((n_utts, n_samples), _NP[dtype])
     self._check(self.lib.vbx_synth_speech(self.h, d.ptr, dtype, n_utts, n_samples, float(fs), seed, first_utt), "vbx_synth_speech")
     return d
@@ -819,13 +844,14 @@ class Multi:
         return list(out)
 
     @staticmethod
-    def _view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride):
+    def _view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride, sample_dtype=None):
         audio = np.ascontiguousarray(audio)
-        return audio, Context.frames(audio.ctypes.data, n_frames, frame_len, stride, window, I16 if audio.dtype == np.int16 else F32,
+        return audio, Context.frames(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype),
                                      frames_per_segment, segment_stride)
 
-    def lpc_host(self, audio, n_frames, frame_len, stride, window, p, out_dtype=F64, frames_per_segment=0, segment_stride=0):
-        audio, fr = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride)
+    def lpc_host(self, audio, n_frames, frame_len, stride, window, p, out_dtype=F64, frames_per_segment=0, segment_stride=0,
+                 sample_dtype=None):
+        audio, fr = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride, sample_dtype)
         r = np.zeros((n_frames, p + 1), dtype=_NP[out_dtype])
         ac = np.zeros((n_frames, p + 1), dtype=_NP[out_dtype])
         kc = np.zeros((n_frames, p), dtype=_NP[out_dtype])
@@ -834,8 +860,8 @@ class Multi:
         return r, ac, kc
 
     def find_formants_host(self, audio, n_frames, frame_len, stride, window, fs, p, method, estimates, dtype=F64,
-                           frames_per_segment=0, segment_stride=0):
-        audio, fr = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride)
+                           frames_per_segment=0, segment_stride=0, sample_dtype=None):
+        audio, fr = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride, sample_dtype)
         J = frames_per_segment or n_frames
         segs = n_frames // J if J else 0
         est = np.ascontiguousarray(estimates, dtype=_NP[dtype]).reshape(segs, -1, 2).copy()
@@ -850,8 +876,8 @@ class Multi:
         return dict(tracks=tracks, estimates=est, resonances=res, n_res=nres, status=st)
 
     def pitch_host(self, audio, n_frames, frame_len, stride, window, fs, threshold, fmin, fmax, max_cand=16, out_dtype=F64,
-                   frames_per_segment=0, segment_stride=0):
-        audio, fr = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride)
+                   frames_per_segment=0, segment_stride=0, sample_dtype=None):
+        audio, fr = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride, sample_dtype)
         cand = np.zeros((n_frames, max_cand, 2), dtype=_NP[out_dtype])
         n = np.zeros(n_frames, dtype=np.int32)
         st = np.zeros(n_frames, dtype=np.uint8)
@@ -861,9 +887,9 @@ class Multi:
 
     def pitch_with_peaks_host(self, audio, n_frames, frame_len, stride, window, fs, threshold, silence_threshold, fmin, fmax,
                               max_cand=16, out_dtype=F64, frames_per_segment=0, segment_stride=0, local_peaks=None,
-                              global_peaks=None):
+                              global_peaks=None, sample_dtype=None):
         """Context.pitch_with_peaks_host sharded over the devices (vbx_multi_pitch_with_peaks_host)."""
-        audio, dt = _host_audio(audio)
+        audio, dt = _host_audio(audio, sample_dtype)
         fr = Context.frames(audio.ctypes.data, n_frames, frame_len, stride, window, dt, frames_per_segment, segment_stride)
         lp = _host_peaks(local_peaks, n_frames)
         gp = _host_peaks(global_peaks, _n_segments(n_frames, frames_per_segment))
@@ -878,8 +904,8 @@ class Multi:
         return dict(candidates=cand, n_cand=n, status=st)
 
     def mfcc_host(self, audio, n_frames, frame_len, stride, window, num_coeffs, f_lo, f_hi, fs, n_keep=None, out_dtype=F64,
-                  frames_per_segment=0, segment_stride=0):
-        audio, fr = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride)
+                  frames_per_segment=0, segment_stride=0, sample_dtype=None):
+        audio, fr = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride, sample_dtype)
         n_keep = num_coeffs if n_keep is None else n_keep
         out = np.zeros((n_frames, n_keep), dtype=_NP[out_dtype])
         self._check(self.lib.vbx_multi_mfcc_host(self.h, C.byref(fr), num_coeffs, n_keep, f_lo, f_hi, fs, out.ctypes.data, out_dtype),
