@@ -226,7 +226,7 @@ VBX_API int vbx_roots_to_resonances(vbx_ctx* ctx, const void* roots, int32_t dty
 /* LPC coefficients -> roots -> resonances in one kernel (the K3+K4 stage of find_formants).
  * lpc: [F][lpc_stride], either [1, a1..ap] (lpc_has_leading_one = 1, Levinson's `ac`) or [a1..ap] (Burg).
  * precision: 0 = fp32 Laguerre/deflation + fp64 Newton polish on the original polynomial (default), 1 = fp64
- * Laguerre/deflation as the reference's f64 instantiation, -1 = library default (env VBX_ROOTS_F64=1 selects 1).
+ * Laguerre/deflation as the reference's f64 instantiation, -1 = library default (0).
  * roots_out (optional): [F][p] complex roots in find_roots order; without it the fp32 path divides conjugate pairs
  * out of the (real) polynomial instead of one root at a time — same resonances, no root list.  status_in
  * (optional): frames whose LPC stage failed are passed through with zero resonances. */

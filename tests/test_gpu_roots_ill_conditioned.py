@@ -17,7 +17,7 @@ pytestmark = pytest.mark.gpu
 TOL_HZ = 0.5
 MALE = np.array([[320., 1.], [1440., 1.], [2760., 1.], [3200., 1.]])
 CLASSES = ("close_pair", "double_root", "close_real", "narrow_bw", "guard_band")
-N_PER_CLASS = 200  # 1000 frames: a ragged last CTA for 128 (1000 % 128 = 104) and for 96 threads (1000 % 96 = 40)
+N_PER_CLASS = 200  # 1000 frames: a ragged last 128-thread CTA (1000 % 128 = 104)
 
 
 def _root(f, bw, fs):
@@ -182,28 +182,7 @@ def test_want_roots_fp32_matches_oracle_on_ill_conditioned_polynomials(oracle, P
     _compare_with_oracle(oracle, P, fs, "want_roots")
 
 
-@pytest.mark.parametrize("fs", [16000, 44100])
-@pytest.mark.parametrize("P", [2, 3, 4, 8, 12, 13, 16, 24])
-def test_pair_kernel_cta_sizes_agree_on_ill_conditioned_polynomials(monkeypatch, P, fs):
-    """The pair-deflation kernel gives the same rows with 96- and 128-thread CTAs (both with a ragged last CTA: 1000 frames),
-    including the frames it hands to the f64 fix-up, for both layouts, f64 and f32 coefficients and both `im` filters."""
-    c = ctx()
-    lpc = _batch(P, fs)
-    assert lpc.shape[0] % 128 and lpc.shape[0] % 96
-    for npdt in (np.float64, np.float32):
-        for strict in (True, False):
-            for has_one in (True, False):
-                d = c.to_device(np.ascontiguousarray((lpc if has_one else lpc[:, 1:]).astype(npdt)))
-                out = {}
-                for threads in ("128", "96"):
-                    monkeypatch.setenv("VBX_ROOTS_THREADS", threads)
-                    out[threads] = c.lpc_to_resonances(d, P, has_one, float(fs), strict_im=strict)
-                for k in ("resonances", "n_res", "status"):
-                    assert np.array_equal(out["96"][k].to_host(), out["128"][k].to_host()), (npdt.__name__, strict, has_one, k)
-
-
-@pytest.mark.parametrize("threads", ["128", "96"])
-def test_fixup_takes_more_frames_than_one_grid(monkeypatch, threads):
+def test_fixup_takes_more_frames_than_one_grid(monkeypatch):
     """VBX_ROOTS_FORCE_HARD=1 hands every frame of the pair kernel to the fix-up launch: 3·4096 + 5 of them, more than one pass
     of the fix-up's grid.  None may be dropped, and every row must be the precision = 1 result bit for bit."""
     c = ctx()
@@ -213,7 +192,6 @@ def test_fixup_takes_more_frames_than_one_grid(monkeypatch, threads):
     _, ac, _ = c.lpc(c.frames(d.ptr, F, N, hop, vb.WINDOW_HANN_SYMMETRIC), p)
     ref = c.lpc_to_resonances(ac, p, True, float(fs), precision=1)
     monkeypatch.setenv("VBX_ROOTS_FORCE_HARD", "1")
-    monkeypatch.setenv("VBX_ROOTS_THREADS", threads)
     c.profile_begin()
     got = c.lpc_to_resonances(ac, p, True, float(fs))
     names = c.profile_end()
@@ -224,10 +202,11 @@ def test_fixup_takes_more_frames_than_one_grid(monkeypatch, threads):
 
 
 @pytest.mark.parametrize("method,window", [(vb.LPC_AUTOCORR, vb.WINDOW_HANN_SYMMETRIC), (vb.LPC_BURG, vb.WINDOW_HANN_PERIODIC)])
-def test_chunked_fixup_finishes_before_its_inputs_are_reused(monkeypatch, method, window):
+def test_chunked_fixup_matches_the_single_chunk_fixup(monkeypatch, method, window):
     """find_formants runs chunk c's fix-up on its side stream while the main stream goes on with the next chunks, which write
-    chunk-local LPC coefficients, LPC status and fix-up lists.  With every frame forced through the fix-up (each chunk well
-    below 4096 frames), any chunk count must give the single f64 pass bit for bit."""
+    chunk-local LPC coefficients, LPC status and fix-up lists, so the fix-up must finish before its inputs are reused.  With
+    every frame forced through the fix-up (each chunk well below 4096 frames), any chunk count must give the single-chunk pass
+    bit for bit — and a fix-up gives the f64 path bit for bit (test_fixup_takes_more_frames_than_one_grid)."""
     c = ctx()
     fs, N, hop, U = 16000, 400, 160, 16
     ns = fs * 2
@@ -235,11 +214,9 @@ def test_chunked_fixup_finishes_before_its_inputs_are_reused(monkeypatch, method
     J = c.n_frames_of(ns, N, hop)
     fr = c.frames(d.ptr, U * J, N, hop, window, frames_per_segment=J, segment_stride=ns)
     est = np.tile(MALE, (U, 1, 1))
-    monkeypatch.setenv("VBX_FORMANT_CHUNKS", "1")
-    monkeypatch.setenv("VBX_ROOTS_F64", "1")
-    ref = c.find_formants(fr, float(fs), 12, method, est)
-    monkeypatch.delenv("VBX_ROOTS_F64")
     monkeypatch.setenv("VBX_ROOTS_FORCE_HARD", "1")
+    monkeypatch.setenv("VBX_FORMANT_CHUNKS", "1")
+    ref = c.find_formants(fr, float(fs), 12, method, est)
     for k in ("3", "5"):
         monkeypatch.setenv("VBX_FORMANT_CHUNKS", k)
         assert U * J / int(k) < 4096

@@ -31,8 +31,8 @@ void vbx_prof_mark(vbx_ctx* ctx, const char* name) {
     ctx->prof_used++;
 }
 
-int vbx_prof_range_begin(vbx_ctx* ctx, const char* name, cudaStream_t stream) {
-    if (!ctx->prof_on || ctx->prof_ranges.size() >= 65536) return -1;
+int vbx_launch_begin(vbx_ctx* ctx, const char* name, cudaStream_t stream) {
+    if (stream == ctx->stream || !ctx->prof_on || ctx->prof_ranges.size() >= 65536) return -1;
     vbx_ctx::ProfRange r;
     r.name = name;
     if (cudaEventCreate(&r.e0) != cudaSuccess) { cudaGetLastError(); return -1; }
@@ -41,8 +41,13 @@ int vbx_prof_range_begin(vbx_ctx* ctx, const char* name, cudaStream_t stream) {
     ctx->prof_ranges.push_back(r);
     return (int)ctx->prof_ranges.size() - 1;
 }
-void vbx_prof_range_end(vbx_ctx* ctx, int slot, cudaStream_t stream) {
+int vbx_launch_end(vbx_ctx* ctx, int slot, const char* name, cudaStream_t stream) {
     if (slot >= 0 && slot < (int)ctx->prof_ranges.size()) cudaEventRecord(ctx->prof_ranges[slot].e1, stream);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return vbx_fail(ctx, VBX_ERR_CUDA, "launch of %s failed: %s", name, cudaGetErrorString(e));
+    ctx->launches++;
+    if (stream == ctx->stream && ctx->prof_on) vbx_prof_mark(ctx, name);
+    return VBX_OK;
 }
 
 int vbx_arena_reserve(vbx_ctx* ctx, size_t bytes) {

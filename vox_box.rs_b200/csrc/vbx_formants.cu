@@ -254,80 +254,45 @@ int launch_burg(vbx_ctx* ctx, const vbx_frames* fr, int p, void* coeffs_out, uin
 // =============================================================================================
 using namespace vbx_roots;
 
+// The fp32 path without a request for the roots themselves runs lpc_roots_pair_kernel (conjugate-pair deflation,
+// vbx_roots_kernel.cuh).  Its caller then launches launch_roots_fixup for the frames the kernel listed.
+bool roots_use_pair_kernel(int precision, const void* roots_out) { return precision != 1 && !roots_out; }
+
 // The f64 fix-up launch behind lpc_roots_pair_kernel (see there): redoes the frames of the pair kernel's list (Q.hard_list /
-// Q.hard_count if the caller chose one, else ctx->hard_list) with the reference's own algorithm.  One CTA per SM at most walks
-// the list (an empty list costs a few µs, a flagged frame ~0.25 ms of single-thread latency — which is why vbx_find_formants puts
-// this launch on its side stream).
+// Q.hard_count) with the reference's own algorithm, on `stream` once the pair kernel's results are visible there.  One CTA per
+// SM at most walks the list (an empty list costs a few µs, a flagged frame ~0.25 ms of single-thread latency — which is why
+// vbx_find_formants puts this launch on its side stream).
 int launch_roots_fixup(vbx_ctx* ctx, const RootsParams& Q, int p, cudaStream_t stream) {
     RootsParams Q2 = Q;
-    Q2.frame_list = Q.hard_list ? Q.hard_list : ctx->hard_list;
-    Q2.frame_count = Q.hard_list ? Q.hard_count : ctx->tile_counter + 1;
-    Q2.hard_cap = Q.hard_list ? Q.hard_cap : (int)ctx->hard_cap;
+    Q2.frame_list = Q.hard_list;
+    Q2.frame_count = Q.hard_count;
     Q2.hard_list = nullptr;
     Q2.hard_count = nullptr;
     Q2.work = nullptr;
     const size_t smem_fix = roots_rt_smem_bytes(p, false);
     VBX_CUDA(ctx, cudaFuncSetAttribute(lpc_roots_rt_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_fix));
-    const bool side = (stream != ctx->stream);
-    const int slot = side ? vbx_prof_range_begin(ctx, "lpc_roots_rt_kernel<double> (fix-up launch)", stream) : -1;
+    const char* name = "lpc_roots_rt_kernel<double> (fix-up launch)";
+    const int slot = vbx_launch_begin(ctx, name, stream);
     // one CTA per SM at most: enough for the few frames speech flags; a batch that flags most of its frames (tonal input) walks
     // the list at low occupancy, a latency not measured (DESIGN.md K3+K4)
     const int64_t grid = std::min<int64_t>((Q.n_frames + kRootsThreads - 1) / kRootsThreads, ctx->sm_count);
     lpc_roots_rt_kernel<double><<<(unsigned)grid, kRootsThreads, smem_fix, stream>>>(Q2, p);
-    if (side) {
-        vbx_prof_range_end(ctx, slot, stream);
-        const cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) return vbx_fail(ctx, VBX_ERR_CUDA, "launch of lpc_roots_rt_kernel<double> (fix-up) failed: %s", cudaGetErrorString(e));
-        ctx->launches++;
-    } else {
-        VBX_CHECK_LAUNCH(ctx, "lpc_roots_rt_kernel<double> (fix-up launch)");
-    }
-    return VBX_OK;
+    return vbx_launch_end(ctx, slot, name, stream);
 }
 
-// defer_fixup (out, optional): when given, the pair path does NOT launch its fix-up; *defer_fixup tells the caller to do so
-// (launch_roots_fixup with the same parameters) once the pair kernel's results are visible to the stream of its choice.
-int launch_lpc_roots(vbx_ctx* ctx, const RootsParams& Q, int p, int precision /*0 fast f32+polish, 1 f64*/, bool* defer_fixup = nullptr) {
-    if (defer_fixup) *defer_fixup = false;
-    VBX_REQUIRE(ctx, p >= 2 && p <= kMaxRootsOrder, "LPC order for root finding must be in 2..%d", kMaxRootsOrder);
-    VBX_REQUIRE(ctx, Q.n_frames <= 0x7fffffffLL, "too many frames for one launch");  // frame indices of the fix-up list are int
+// Launches the roots kernel only: after lpc_roots_pair_kernel (roots_use_pair_kernel), the caller launches the fix-up.
+int launch_lpc_roots(vbx_ctx* ctx, const RootsParams& Q, int p, int precision /*-1 or 0 fast f32+polish, 1 f64*/) {
     const int64_t grid = (Q.n_frames + kRootsThreads - 1) / kRootsThreads;
     const bool f32 = (precision != 1);
-    // fp32 path without a request for the roots themselves: conjugate-pair deflation (vbx_roots_kernel.cuh)
-    if (f32 && !Q.roots_out) {
-        // 96-thread CTAs (24 KB at order 12) fit next to the persistent LPC kernel's CTA on an SM: ctx->roots_small
-        int rthreads = ctx->roots_small ? 96 : kRootsThreads;
-        if (const char* e = getenv("VBX_ROOTS_THREADS")) rthreads = atoi(e) == 96 ? 96 : kRootsThreads;
-        const size_t smem_pair = roots_pair_smem_bytes(p, rthreads);
-        if (rthreads == 96) {
-            VBX_CUDA(ctx, cudaFuncSetAttribute(lpc_roots_pair_kernel<96>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_pair));
-            // the same (maximum) shared-memory carve-out as the persistent LPC kernel's SMs: CTAs of kernels that want
-            // different carve-outs do not share an SM
-            VBX_CUDA(ctx, cudaFuncSetAttribute(lpc_roots_pair_kernel<96>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-        }
-        else VBX_CUDA(ctx, cudaFuncSetAttribute(lpc_roots_pair_kernel<kRootsThreads>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_pair));
-        const int64_t grid_pair = (Q.n_frames + rthreads - 1) / rthreads;
+    if (roots_use_pair_kernel(precision, Q.roots_out)) {
+        const size_t smem_pair = roots_pair_smem_bytes(p);
+        VBX_CUDA(ctx, cudaFuncSetAttribute(lpc_roots_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_pair));
         RootsParams Q1 = Q;
-        Q1.work = vbx_work_ptr(ctx);
-        if (!Q.hard_list) {  // the caller's own list holds at least n_frames entries (vbx_find_formants), else the context's
-            const int st = vbx_hard_list_reserve(ctx, Q.n_frames);
-            if (st != VBX_OK) return st;
-            Q1.hard_list = ctx->hard_list;
-            Q1.hard_count = ctx->tile_counter + 1;
-            Q1.hard_cap = (int)ctx->hard_cap;
-        }
         if (const char* e = getenv("VBX_ROOTS_FORCE_HARD")) Q1.hard_mod = atoi(e);
         VBX_CUDA(ctx, cudaMemsetAsync(Q1.hard_count, 0, sizeof(unsigned), ctx->stream));
-        if (rthreads == 96) lpc_roots_pair_kernel<96><<<(unsigned)grid_pair, 96, smem_pair, ctx->stream>>>(Q1, p);
-        else lpc_roots_pair_kernel<kRootsThreads><<<(unsigned)grid_pair, kRootsThreads, smem_pair, ctx->stream>>>(Q1, p);
+        lpc_roots_pair_kernel<<<(unsigned)grid, kRootsThreads, smem_pair, ctx->stream>>>(Q1, p);
         VBX_CHECK_LAUNCH(ctx, "lpc_roots_pair_kernel");
-        // fix-up: frames on which a solve hit the 20-iteration cap twice (two start points) without converging go to the f64
-        // reference-order kernel
-        if (defer_fixup) {
-            *defer_fixup = true;
-            return VBX_OK;
-        }
-        return launch_roots_fixup(ctx, Q, p, ctx->stream);
+        return VBX_OK;
     }
     const size_t smem = roots_rt_smem_bytes(p, f32);
     if (f32) {
@@ -491,7 +456,7 @@ __global__ void __launch_bounds__(128) roots_to_resonances_kernel(const T* __res
 // =============================================================================================
 struct TrackParams {
     const void* res;        // [F][R] resonance pairs
-    const int32_t* nres;    // unused by the step (zeros take part), kept for debugging
+    const int32_t* nres;    // [F] count of real resonances, zero padding behind them (read by tracker_idx_kernel only)
     const uint8_t* status;  // per-frame status (frames with an error leave the estimates untouched) or null
     void* est_inout;        // [n_segments][n_est]
     void* tracks_out;       // [F][n_est] or null
@@ -903,11 +868,6 @@ __global__ void __launch_bounds__(256) resample_kernel(const TIn* __restrict__ b
     out[e] = win ? v * __ldg(win + k) : v;
 }
 
-int root_precision_default() {
-    const char* e = getenv("VBX_ROOTS_F64");
-    return (e && e[0] == '1') ? 1 : 0;
-}
-
 }  // namespace
 
 size_t vbx_burg_scratch_bytes(vbx_ctx* ctx, const vbx_frames* fr) {
@@ -939,12 +899,12 @@ int vbx_lpc_burg(vbx_ctx* ctx, const vbx_frames* frames, int32_t p, void* coeffs
     return launch_burg<float>(ctx, frames, p, coeffs_out, status_out, out_dtype);
 }
 
-static int lpc_to_resonances_impl(vbx_ctx* ctx, const void* lpc, int32_t lpc_dtype, int64_t n_frames, int32_t lpc_stride, int32_t p,
-                                  int32_t lpc_has_leading_one, double sample_rate, int32_t strict_im, const uint8_t* status_in,
-                                  void* res_out, int32_t res_slots, int32_t* nres_out, void* roots_out, uint8_t* status_out,
-                                  int32_t out_dtype, int32_t precision, int64_t in_J, int64_t out_J, int64_t out_j0,
-                                  RootsParams* q_out = nullptr, bool* defer_fixup = nullptr, int* hard_list = nullptr,
-                                  unsigned* hard_count = nullptr, int hard_cap = 0) {
+// Checks the arguments of a roots -> resonances call and fills *Q (nothing to launch when n_frames == 0).  The fix-up list of
+// the pair kernel (hard_list, hard_count, hard_cap) is left for the caller to set.
+static int lpc_roots_params(vbx_ctx* ctx, const void* lpc, int32_t lpc_dtype, int64_t n_frames, int32_t lpc_stride, int32_t p,
+                            int32_t lpc_has_leading_one, double sample_rate, int32_t strict_im, const uint8_t* status_in,
+                            void* res_out, int32_t res_slots, int32_t* nres_out, void* roots_out, uint8_t* status_out,
+                            int32_t out_dtype, int32_t precision, int64_t in_J, int64_t out_J, int64_t out_j0, RootsParams* Q) {
     if (!ctx) return VBX_ERR_BADARG;
     VBX_REQUIRE(ctx, lpc_dtype == VBX_F32 || lpc_dtype == VBX_F64, "lpc_dtype must be VBX_F32 or VBX_F64");
     VBX_REQUIRE(ctx, out_dtype == VBX_F32 || out_dtype == VBX_F64, "out_dtype must be VBX_F32 or VBX_F64");
@@ -955,24 +915,36 @@ static int lpc_to_resonances_impl(vbx_ctx* ctx, const void* lpc, int32_t lpc_dty
     if (n_frames == 0) return VBX_OK;
     VBX_REQUIRE(ctx, lpc != nullptr, "lpc is NULL");
     cudaSetDevice(ctx->device);
-    RootsParams Q;
-    Q.lpc = lpc; Q.status_in = status_in; Q.res_out = res_out; Q.nres_out = nres_out; Q.roots_out = roots_out;
-    Q.status_out = status_out; Q.n_frames = n_frames; Q.fs = sample_rate; Q.lpc_stride = lpc_stride;
-    Q.lpc_has_one = lpc_has_leading_one ? 1 : 0; Q.lpc_f64 = (lpc_dtype == VBX_F64); Q.out_f64 = (out_dtype == VBX_F64);
-    Q.R = res_slots; Q.strict_im = strict_im ? 1 : 0; Q.polish_steps = 2;
-    Q.work = vbx_work_ptr(ctx);
-    Q.in_J = in_J; Q.out_J = out_J; Q.out_j0 = out_j0;
-    Q.hard_list = hard_list; Q.hard_count = hard_count; Q.hard_cap = hard_cap; Q.hard_mod = 0; Q.frame_list = nullptr; Q.frame_count = nullptr;
-    if (q_out) *q_out = Q;
-    return launch_lpc_roots(ctx, Q, p, precision < 0 ? root_precision_default() : precision, defer_fixup);
+    VBX_REQUIRE(ctx, p >= 2 && p <= kMaxRootsOrder, "LPC order for root finding must be in 2..%d", kMaxRootsOrder);
+    VBX_REQUIRE(ctx, n_frames <= 0x7fffffffLL, "too many frames for one launch");  // frame indices of the fix-up list are int
+    Q->lpc = lpc; Q->status_in = status_in; Q->res_out = res_out; Q->nres_out = nres_out; Q->roots_out = roots_out;
+    Q->status_out = status_out; Q->n_frames = n_frames; Q->fs = sample_rate; Q->lpc_stride = lpc_stride;
+    Q->lpc_has_one = lpc_has_leading_one ? 1 : 0; Q->lpc_f64 = (lpc_dtype == VBX_F64); Q->out_f64 = (out_dtype == VBX_F64);
+    Q->R = res_slots; Q->strict_im = strict_im ? 1 : 0; Q->polish_steps = 2;
+    Q->work = vbx_work_ptr(ctx);
+    Q->in_J = in_J; Q->out_J = out_J; Q->out_j0 = out_j0;
+    Q->hard_list = nullptr; Q->hard_count = nullptr; Q->hard_cap = 0; Q->hard_mod = 0; Q->frame_list = nullptr; Q->frame_count = nullptr;
+    return VBX_OK;
 }
 
 int vbx_lpc_to_resonances(vbx_ctx* ctx, const void* lpc, int32_t lpc_dtype, int64_t n_frames, int32_t lpc_stride, int32_t p,
                           int32_t lpc_has_leading_one, double sample_rate, int32_t strict_im, const uint8_t* status_in,
                           void* res_out, int32_t res_slots, int32_t* nres_out, void* roots_out, uint8_t* status_out,
                           int32_t out_dtype, int32_t precision) {
-    return lpc_to_resonances_impl(ctx, lpc, lpc_dtype, n_frames, lpc_stride, p, lpc_has_leading_one, sample_rate, strict_im, status_in,
-                                  res_out, res_slots, nres_out, roots_out, status_out, out_dtype, precision, 0, 0, 0);
+    RootsParams Q;
+    int st = lpc_roots_params(ctx, lpc, lpc_dtype, n_frames, lpc_stride, p, lpc_has_leading_one, sample_rate, strict_im, status_in,
+                              res_out, res_slots, nres_out, roots_out, status_out, out_dtype, precision, 0, 0, 0, &Q);
+    if (st != VBX_OK || n_frames == 0) return st;
+    if (!roots_use_pair_kernel(precision, roots_out)) return launch_lpc_roots(ctx, Q, p, precision);
+    // the pair kernel's fix-up list: set 0 of the context's lists, its length in tile_counter[1]
+    st = vbx_hard_list_reserve(ctx, n_frames);
+    if (st != VBX_OK) return st;
+    Q.hard_list = ctx->hard_list;
+    Q.hard_count = ctx->tile_counter + 1;
+    Q.hard_cap = (int)ctx->hard_cap;
+    st = launch_lpc_roots(ctx, Q, p, precision);
+    if (st != VBX_OK) return st;
+    return launch_roots_fixup(ctx, Q, p, ctx->stream);
 }
 
 int vbx_find_roots(vbx_ctx* ctx, const void* coeffs, int32_t dtype, int64_t n_polys, int32_t len, void* roots_out,
@@ -1075,7 +1047,6 @@ static int estimate_formants_impl(vbx_ctx* ctx, const void* resonances, int32_t 
     T.n_segments = n_segments; T.seg_frames = frames_per_segment; T.R = res_slots; T.n_res_eff = n_resonances;
     T.n_est = n_estimates; T.res_f64 = (res_dtype == VBX_F64); T.out_f64 = (dtype == VBX_F64);
     T.j_begin = j_begin; T.j_count = j_count;
-    const bool side = (stream != ctx->stream);  // side-stream launches are timed as explicit event pairs
     // fused path (per-frame counts known, rows sorted and zero padded): the index-based thread-per-utterance kernel,
     // when the rows can be staged with 16-byte cp.async chunks.  Arbitrary caller resonances (vbx_estimate_formants) or
     // odd fp32 row lengths: the value-based warp-per-utterance kernel.
@@ -1091,50 +1062,22 @@ static int estimate_formants_impl(vbx_ctx* ctx, const void* resonances, int32_t 
     // leaves exactly that many SMs free (ctx->reserve_sms).  Whichever kernel the block scheduler places first, the tracker ends
     // up alone on its SMs (0.69 ms per chunk, hidden); with small CTAs the outcome depended on the launch race.
     int trk_threads = packed ? kTrkThreadsPacked : kTrkThreads;
-    if (const char* e = getenv("VBX_TRACKER_THREADS")) {
-        const int v = atoi(e);
-        if (v >= 32 && v <= kTrkThreadsPacked && v % 32 == 0) trk_threads = v;
-    }
     while (trk_threads > 32 && (size_t)2 * chunks * trk_threads * 16 > ctx->smem_optin) trk_threads >>= 1;
     const size_t smem = (size_t)2 * chunks * trk_threads * 16;
     if (nres && aligned && smem <= ctx->smem_optin) {
         const int64_t grid = (n_segments + trk_threads - 1) / trk_threads;
         VBX_REQUIRE(ctx, grid <= 0x7fffffffLL, "too many segments for one launch");
-        if (res_dtype == VBX_F64) {
-            VBX_CUDA(ctx, cudaFuncSetAttribute(tracker_idx_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            const int slot = side ? vbx_prof_range_begin(ctx, "tracker_idx_kernel", stream) : -1;
-            tracker_idx_kernel<true><<<(unsigned)grid, trk_threads, smem, stream>>>(T, chunks);
-            if (side) vbx_prof_range_end(ctx, slot, stream);
-        } else {
-            VBX_CUDA(ctx, cudaFuncSetAttribute(tracker_idx_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            const int slot = side ? vbx_prof_range_begin(ctx, "tracker_idx_kernel", stream) : -1;
-            tracker_idx_kernel<false><<<(unsigned)grid, trk_threads, smem, stream>>>(T, chunks);
-            if (side) vbx_prof_range_end(ctx, slot, stream);
-        }
-        if (side) {
-            const cudaError_t e = cudaGetLastError();
-            if (e != cudaSuccess) return vbx_fail(ctx, VBX_ERR_CUDA, "launch of tracker_idx_kernel failed: %s", cudaGetErrorString(e));
-            ctx->launches++;
-        } else {
-            VBX_CHECK_LAUNCH(ctx, "tracker_idx_kernel");
-        }
-        return VBX_OK;
+        void (*kern)(const TrackParams, const int) = (res_dtype == VBX_F64) ? tracker_idx_kernel<true> : tracker_idx_kernel<false>;
+        VBX_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        const int slot = vbx_launch_begin(ctx, "tracker_idx_kernel", stream);
+        kern<<<(unsigned)grid, trk_threads, smem, stream>>>(T, chunks);
+        return vbx_launch_end(ctx, slot, "tracker_idx_kernel", stream);
     }
     const int64_t grid = (n_segments + 3) / 4;  // one warp per segment
     VBX_REQUIRE(ctx, grid <= 0x7fffffffLL, "too many segments for one launch");
-    {
-        const int slot = side ? vbx_prof_range_begin(ctx, "tracker_kernel", stream) : -1;
-        tracker_kernel<<<(unsigned)grid, 128, 0, stream>>>(T);
-        if (side) vbx_prof_range_end(ctx, slot, stream);
-    }
-    if (side) {
-        const cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) return vbx_fail(ctx, VBX_ERR_CUDA, "launch of tracker_kernel failed: %s", cudaGetErrorString(e));
-        ctx->launches++;
-    } else {
-        VBX_CHECK_LAUNCH(ctx, "tracker_kernel");
-    }
-    return VBX_OK;
+    const int slot = vbx_launch_begin(ctx, "tracker_kernel", stream);
+    tracker_kernel<<<(unsigned)grid, 128, 0, stream>>>(T);
+    return vbx_launch_end(ctx, slot, "tracker_kernel", stream);
 }
 
 int vbx_estimate_formants(vbx_ctx* ctx, const void* resonances, int32_t res_dtype, int32_t res_slots, int32_t n_resonances,
@@ -1270,7 +1213,6 @@ int vbx_find_formants(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
             } else {
                 // the persistent LPC kernel leaves SMs for the co-running tracker: 16 of its warps (512 utterances) per SM
                 ctx->reserve_sms = overlap ? (int)((segs + kTrkThreadsPacked - 1) / kTrkThreadsPacked) : 0;
-                if (const char* e = getenv("VBX_FORMANT_RESERVE_SMS")) ctx->reserve_sms = atoi(e);
                 st = vbx_lpc(ctx, &sub, p, nullptr, d_lpc, nullptr, VBX_F64);
                 ctx->reserve_sms = 0;
                 lpc_stride = p + 1;
@@ -1278,13 +1220,20 @@ int vbx_find_formants(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
             }
         }
         if (st != VBX_OK) break;
+        // roots: always lpc_roots_pair_kernel here (fp32, no roots_out), with buffer set b's fix-up list
         RootsParams Qc;
-        bool fixup_pending = false;
-        st = lpc_to_resonances_impl(ctx, d_lpc, VBX_F64, sub.n_frames, lpc_stride, p, has_one, sample_rate, /*strict_im=*/1, lpc_status,
-                                    d_res, R, d_nres, nullptr, d_st, dtype, -1, K > 1 ? Jc : 0, K > 1 ? J : 0, K > 1 ? j0 : 0, &Qc,
-                                    overlap ? &fixup_pending : nullptr, ctx->hard_list + b * Fc_max, ctx->tile_counter + 1 + b,
-                                    (int)Fc_max);
+        st = lpc_roots_params(ctx, d_lpc, VBX_F64, sub.n_frames, lpc_stride, p, has_one, sample_rate, /*strict_im=*/1, lpc_status, d_res,
+                              R, d_nres, nullptr, d_st, dtype, -1, K > 1 ? Jc : 0, K > 1 ? J : 0, K > 1 ? j0 : 0, &Qc);
         if (st != VBX_OK) break;
+        Qc.hard_list = ctx->hard_list + b * Fc_max;
+        Qc.hard_count = ctx->tile_counter + 1 + b;
+        Qc.hard_cap = (int)Fc_max;
+        st = launch_lpc_roots(ctx, Qc, p, -1);
+        if (st != VBX_OK) break;
+        if (!overlap) {  // with overlap, the fix-up goes to the side stream below
+            st = launch_roots_fixup(ctx, Qc, p, ctx->stream);
+            if (st != VBX_OK) break;
+        }
         if (!track) continue;
         if (K == 1) {
             st = estimate_formants_impl(ctx, d_res, dtype, R, VBX_MAX_RESONANCES, segs, J, d_st, est_inout, n_formants, tracks_out, dtype,
@@ -1299,15 +1248,14 @@ int vbx_find_formants(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
             break;
         }
         // (the last chunk's tracker has the device to itself: small CTAs over all SMs, 0.27 ms instead of 0.69)
-        if (fixup_pending) {  // the roots fix-up (rarely any work, but ~0.25 ms of latency when there is) rides the side stream too
-            st = launch_roots_fixup(ctx, Qc, p, ctx->s_side);
-            if (st != VBX_OK) break;
-            if (cudaEventRecord(ctx->ev_side[2 + b], ctx->s_side) != cudaSuccess) {
-                st = vbx_fail(ctx, VBX_ERR_CUDA, "find_formants: fix-up event failed: %s", cudaGetErrorString(cudaGetLastError()));
-                break;
-            }
-            fixup_queued[b] = true;
+        // the roots fix-up (rarely any work, but ~0.25 ms of latency when there is) rides the side stream too
+        st = launch_roots_fixup(ctx, Qc, p, ctx->s_side);
+        if (st != VBX_OK) break;
+        if (cudaEventRecord(ctx->ev_side[2 + b], ctx->s_side) != cudaSuccess) {
+            st = vbx_fail(ctx, VBX_ERR_CUDA, "find_formants: fix-up event failed: %s", cudaGetErrorString(cudaGetLastError()));
+            break;
         }
+        fixup_queued[b] = true;
         st = estimate_formants_impl(ctx, d_res, dtype, R, VBX_MAX_RESONANCES, segs, J, d_st, est_inout, n_formants, tracks_out, dtype,
                                     d_nres, j0, Jc, ctx->s_side, /*packed=*/c + 1 < K);
         if (st != VBX_OK) break;

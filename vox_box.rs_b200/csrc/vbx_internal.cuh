@@ -60,7 +60,6 @@ struct vbx_ctx {
     // incremented only while profiling is on): see vbx_profile_counters in the header
     unsigned long long* work_counters = nullptr;
     int reserve_sms = 0;               // SMs the persistent kernels leave free for a co-running side-stream kernel
-    bool roots_small = false;          // lpc_roots_pair_kernel in 96-thread CTAs (they fit beside a persistent LPC CTA)
     unsigned* tile_counter = nullptr;  // device: [0] the persistent kernels' dynamic tile cursor, [1..2] lengths of fix-up lists
     int* hard_list = nullptr;          // device: frames the pair-deflation roots kernel hands to the f64 fix-up launch
     int64_t hard_cap = 0;              // entries of hard_list (vbx_hard_list_reserve: as many as a roots launch has frames)
@@ -74,9 +73,11 @@ static inline unsigned long long* vbx_work_ptr(vbx_ctx* ctx) { return ctx->prof_
 
 int vbx_fail(vbx_ctx* ctx, int status, const char* fmt, ...);
 void vbx_prof_mark(vbx_ctx* ctx, const char* name);        // records "launch `name` was just enqueued" (profiling on)
-// side-stream launches: begin returns a slot (or -1), end closes it; counts the launch
-int vbx_prof_range_begin(vbx_ctx* ctx, const char* name, cudaStream_t stream);
-void vbx_prof_range_end(vbx_ctx* ctx, int slot, cudaStream_t stream);
+// A launch on `stream` placed between these two.  On the context's stream, end does what VBX_CHECK_LAUNCH does; on a side
+// stream, where the begin / end markers of vbx_prof_mark do not apply, the launch is timed as its own (start, stop) event pair
+// on that stream (begin returns its slot, or -1).  end checks and counts the launch either way.
+int vbx_launch_begin(vbx_ctx* ctx, const char* name, cudaStream_t stream);
+int vbx_launch_end(vbx_ctx* ctx, int slot, const char* name, cudaStream_t stream);
 int vbx_arena_reserve(vbx_ctx* ctx, size_t bytes);         // ensures ctx->arena has >= bytes
 int vbx_pinned_reserve(vbx_ctx* ctx, size_t bytes);        // ensures ctx->pinned has >= bytes
 int vbx_hard_list_reserve(vbx_ctx* ctx, int64_t n);        // ensures ctx->hard_list has >= n entries

@@ -1,6 +1,5 @@
 // vbx_roots_kernel.cuh — LPC coefficients → roots → resonances, one thread per frame (K3 + K4).
-// Included by vbx_formants.cu (launcher) and by the vbx_roots_inst_*.cu translation units that
-// instantiate the kernel for ranges of the LPC order (split only to compile in parallel).
+// Included by vbx_formants.cu (the launcher) only: lpc_roots_pair_kernel is a plain kernel defined here.
 #pragma once
 #include "vbx_complex.cuh"
 #include "vbx_internal.cuh"
@@ -337,10 +336,9 @@ __global__ void __launch_bounds__(kRootsThreads) lpc_roots_rt_kernel(const Roots
 // (find_roots order) takes lpc_roots_rt_kernel instead.  Resonance counts and values are checked against the oracle in
 // tests/test_gpu_formants.py, tests/test_gpu_full_size.py and tools/parity_scale.py.
 // ---------------------------------------------------------------------------------------------
-template <int TT>   // threads per CTA: 128, or 96 for the launches that share their SMs with the persistent LPC kernel
-__global__ void __launch_bounds__(TT) lpc_roots_pair_kernel(const RootsParams Q, const int P) {
+__global__ void __launch_bounds__(kRootsThreads) lpc_roots_pair_kernel(const RootsParams Q, const int P) {
     extern __shared__ __align__(16) unsigned char roots_smem[];
-    constexpr int T = TT;
+    constexpr int T = kRootsThreads;
     typedef float TR;
     const unsigned FULL = 0xffffffffu;
     double* a_s = reinterpret_cast<double*>(roots_smem);                    // [P+1][T] original real coefficients
@@ -559,9 +557,9 @@ __global__ void __launch_bounds__(TT) lpc_roots_pair_kernel(const RootsParams Q,
     }
 }
 
-static inline size_t roots_pair_smem_bytes(int P, int threads = kRootsThreads) {
+static inline size_t roots_pair_smem_bytes(int P) {
     // a_s [P+1] f64, r_s [P] complex f32 (reused as the resonance staging), c_s [P+1] f32
-    return (size_t)threads * ((size_t)(P + 1) * 8 + (size_t)P * 8 + (size_t)(P + 1) * 4);
+    return (size_t)kRootsThreads * ((size_t)(P + 1) * 8 + (size_t)P * 8 + (size_t)(P + 1) * 4);
 }
 
 static inline size_t roots_rt_smem_bytes(int P, bool f32) {
