@@ -87,7 +87,26 @@ typedef enum vbx_window {
  * dtype: VBX_F32 samples, VBX_I16 PCM scaled by 1/32767 on load (tests/lib.rs:17-19), VBX_MULAW8 / VBX_ALAW8 G.711 bytes
  * (decoded to int16 PCM on load, then exactly VBX_I16), or VBX_F64 samples (what the reference's f64 callers hold, e.g. a
  * frame they windowed themselves: use VBX_WINDOW_NONE; f64 samples run the same arithmetic through the general-purpose
- * kernels, the tuned batch kernels stage fp32 / int16 / G.711).  Strides are in samples whatever the sample size. */
+ * kernels, the tuned batch kernels stage fp32 / int16 / G.711).  Strides are in samples whatever the sample size.
+ *
+ * Interleaved audio (sample_step): 0 and 1 mean contiguous frames, as above.  With s = sample_step > 1, sample i of frame
+ * f = u*J + j is base[u*segment_stride + j*frame_stride + i*s]: a recording of C interleaved channels (L0 R0 L1 R1 ...) is
+ * read in place with s = C, frame_stride = hop*C, segment_stride = 1 and one segment per channel (segment u = channel u,
+ * J frames each; or frames_per_segment = 0 and base offset by the channel for one channel).  frame_stride must be a
+ * multiple of s (every frame of a segment stays on its channel), sample_step < 0 and views whose extent overflows int64
+ * are VBX_ERR_BADARG.
+ * The rule that defines every result: let S = ((J-1)*frame_stride)/s + frame_len, the channel samples segment u spans
+ * (J = frames_per_segment, or n_frames for a single-segment view, where u = 0).  Its PLANAR EQUIVALENT is the contiguous
+ * array P[u][k] = base[u*segment_stride + k*s], k < S, laid out as rows of S' = S rounded up to a multiple of 64 samples
+ * (P[u][k] at offset u*S' + k of a 256-byte-aligned buffer of the same dtype) and viewed with frame_stride/s, segment
+ * stride S' and sample_step 1, everything else unchanged.  Every frame-view call on an interleaved view returns, bit for
+ * bit, what the same call returns on its planar equivalent: every output, status and count, and the local and global peaks
+ * of vbx_frame_peaks / vbx_pitch_with_peaks.  The library builds that planar copy on the device (a gather kernel,
+ * interleave_gather_kernel, into a grow-only buffer of the context that nothing else uses) and runs the ordinary kernels
+ * on it; a G.711 copy stays one byte per sample.  The _host twins upload the interleaved bytes once: when the segments
+ * share memory (segment_stride below a segment's extent, the channels-as-segments layout) they cut the view into time
+ * ranges of every segment rather than into whole segments.  The _multi_host twins shard such a view by segment as any
+ * other, so an interleaved recording of C channels keeps at most C devices busy. */
 typedef struct vbx_frames {
     const void* base;
     int64_t n_frames;
@@ -97,7 +116,10 @@ typedef struct vbx_frames {
     int32_t frame_len;          /* N */
     int32_t dtype;        /* vbx_dtype: VBX_F32, VBX_I16, VBX_MULAW8, VBX_ALAW8 or VBX_F64 */
     int32_t window;       /* vbx_window */
-    int32_t reserved;     /* must be 0 */
+    union {
+        int32_t reserved;    /* the field's former name: 0 is contiguous samples */
+        int32_t sample_step; /* samples between consecutive samples of a frame: 0 or 1 contiguous, s > 1 interleaved */
+    };
 } vbx_frames;
 
 /* #[repr(C)] Resonance<T> { frequency, bandwidth }  spectrum.rs:149-154 */

@@ -60,7 +60,9 @@ pub mod ffi {
         pub frame_len: i32,
         pub dtype: i32,
         pub window: i32,
-        pub reserved: i32,
+        /// samples between consecutive samples of a frame: 0 / 1 contiguous, C for C interleaved channels (the C header's
+        /// `union { reserved; sample_step; }`)
+        pub sample_step: i32,
     }
 
     pub const VBX_OK: c_int = 0;
@@ -411,7 +413,7 @@ fn one_frame<T: Elem>(x: &[T], window: i32) -> ffi::vbx_frames {
         frame_len: x.len() as i32,
         dtype: T::DTYPE,
         window,
-        reserved: 0,
+        sample_step: 0,
     }
 }
 
@@ -1179,7 +1181,7 @@ pub mod batch {
                 frame_len: bin as i32,
                 dtype: ffi::VBX_F32,
                 window,
-                reserved: 0,
+                sample_step: 0,
             }
         }
         /// Hann -> autocorrelate(p+1) -> lpc(p) for every frame: ([F][p+1] r, [F][p+1] lpc) as fp32.
@@ -1245,7 +1247,7 @@ pub mod batch {
                 frame_len: bin as i32,
                 dtype: ffi::VBX_F32,
                 window: ffi::VBX_WINDOW_HANN_SYMMETRIC,
-                reserved: 0,
+                sample_step: 0,
             };
             let mut tracks = vec![Resonance::<f32>::default(); j * n_utterances * k];
             self.check(unsafe {

@@ -202,11 +202,24 @@ int vbx_check_frames(vbx_ctx* ctx, const vbx_frames* fr, bool allow_f64) {
                 allow_f64 ? "frames dtype must be VBX_F32, VBX_I16, VBX_MULAW8, VBX_ALAW8 or VBX_F64"
                           : "frames dtype must be VBX_F32, VBX_I16, VBX_MULAW8 or VBX_ALAW8");
     VBX_REQUIRE(ctx, fr->window >= VBX_WINDOW_NONE && fr->window <= VBX_WINDOW_HANN_PERIODIC, "unknown window kind");
-    VBX_REQUIRE(ctx, fr->reserved == 0, "frames.reserved must be 0");
+    VBX_REQUIRE(ctx, fr->sample_step >= 0, "frames.sample_step < 0");
     VBX_REQUIRE(ctx, fr->frames_per_segment >= 0, "frames_per_segment < 0");
     if (fr->frames_per_segment > 0) {
         VBX_REQUIRE(ctx, fr->n_frames % fr->frames_per_segment == 0, "n_frames must be a multiple of frames_per_segment");
         VBX_REQUIRE(ctx, fr->segment_stride >= 0, "segment_stride < 0");
+    }
+    const int64_t s = vbx_sample_step(fr);
+    VBX_REQUIRE(ctx, fr->frame_stride % s == 0, "frame_stride (%lld) must be a multiple of sample_step (%lld)",
+                (long long)fr->frame_stride, (long long)s);
+    // extent = (U-1)*segment_stride + (J-1)*frame_stride + (N-1)*s + 1 samples, and its bytes, must fit int64
+    if (fr->n_frames > 0) {
+        const int64_t J = vbx_frames_per_segment(fr), U = fr->n_frames / J;
+        int64_t a = 0, b = 0, c = 0, e = 0;
+        const bool ovf = __builtin_mul_overflow(U - 1, fr->frames_per_segment > 0 ? fr->segment_stride : 0, &a) ||
+                         __builtin_mul_overflow(J - 1, fr->frame_stride, &b) ||
+                         __builtin_mul_overflow((int64_t)fr->frame_len - 1, s, &c) || __builtin_add_overflow(a, b, &e) ||
+                         __builtin_add_overflow(e, c + 1, &e) || __builtin_mul_overflow(e, (int64_t)vbx_dtype_size(fr->dtype), &e);
+        VBX_REQUIRE(ctx, !ovf, "the view's extent overflows int64");
     }
     VBX_REQUIRE(ctx, fr->n_frames == 0 || fr->base != nullptr, "frames.base is NULL");
     return VBX_OK;
@@ -321,6 +334,7 @@ int vbx_ctx_destroy(vbx_ctx* ctx) {
     if (ctx->arena) cudaFree(ctx->arena);
     if (ctx->pinned) cudaFreeHost(ctx->pinned);
     if (ctx->pipe) cudaFree(ctx->pipe);
+    if (ctx->planar) cudaFree(ctx->planar);
     for (int i = 0; i < 6; ++i) cudaEventDestroy(ctx->ev_pipe[i]);
     for (int i = 0; i < 4; ++i) cudaEventDestroy(ctx->ev_side[i]);
     for (auto& r : ctx->prof_ranges) { cudaEventDestroy(r.e0); cudaEventDestroy(r.e1); }

@@ -892,6 +892,10 @@ int vbx_lpc_burg(vbx_ctx* ctx, const vbx_frames* frames, int32_t p, void* coeffs
     if (frames->n_frames == 0) return VBX_OK;
     VBX_REQUIRE(ctx, coeffs_out != nullptr, "coeffs_out is NULL");
     cudaSetDevice(ctx->device);
+    vbx_frames pv;  // the planar equivalent of an interleaved view
+    st = vbx_planarize(ctx, frames, &pv);
+    if (st != VBX_OK) return st;
+    frames = &pv;
     if (frames->dtype == VBX_I16) return launch_burg<int16_t>(ctx, frames, p, coeffs_out, status_out, out_dtype);
     if (frames->dtype == VBX_MULAW8) return launch_burg<vbx_mulaw8>(ctx, frames, p, coeffs_out, status_out, out_dtype);
     if (frames->dtype == VBX_ALAW8) return launch_burg<vbx_alaw8>(ctx, frames, p, coeffs_out, status_out, out_dtype);
@@ -1104,6 +1108,11 @@ int vbx_find_formants(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate
     const int64_t F = frames->n_frames;
     if (F == 0) return VBX_OK;
     cudaSetDevice(ctx->device);
+    // an interleaved view is gathered into the context's planar buffer, not into the arena block reserved below
+    vbx_frames pv;
+    st = vbx_planarize(ctx, frames, &pv);
+    if (st != VBX_OK) return st;
+    frames = &pv;
     const int p = n_coeffs;
     const int64_t J = vbx_frames_per_segment(frames), segs = F / J;
     const bool track = (n_formants > 0 && est_inout);
@@ -1298,6 +1307,10 @@ extern "C" int vbx_find_formants_buffered(vbx_ctx* ctx, const vbx_frames* frames
     const int row_len = resampled_buf_len > 0 ? (int)resampled_buf_len : rlen;
     if (F == 0) return VBX_OK;
     cudaSetDevice(ctx->device);
+    vbx_frames pv;  // the planar equivalent of an interleaved view
+    st = vbx_planarize(ctx, frames, &pv);
+    if (st != VBX_OK) return st;
+    frames = &pv;
     vbx_frames rfr = *frames;
     if (resample_ratio == 1.0 && row_len == rlen) {  // lib.rs:62-64: plain copy, window over exactly the frame
         rfr.window = VBX_WINDOW_HANN_PERIODIC;
@@ -1369,7 +1382,7 @@ extern "C" int vbx_find_formants_buffered(vbx_ctx* ctx, const vbx_frames* frames
         vbx_frames pf;
         pf.base = d_out; pf.n_frames = F; pf.frame_stride = row_len; pf.frames_per_segment = frames->frames_per_segment;
         pf.segment_stride = (frames->frames_per_segment > 0) ? frames->frames_per_segment * (int64_t)row_len : 0;
-        pf.frame_len = row_len; pf.dtype = VBX_F64; pf.window = window_here ? VBX_WINDOW_NONE : VBX_WINDOW_HANN_PERIODIC; pf.reserved = 0;
+        pf.frame_len = row_len; pf.dtype = VBX_F64; pf.window = window_here ? VBX_WINDOW_NONE : VBX_WINDOW_HANN_PERIODIC; pf.sample_step = 0;
         int s2 = vbx_find_formants(ctx, &pf, sample_rate, n_coeffs, VBX_LPC_BURG, est_inout, n_formants, tracks_out, resonances_out,
                                    nres_out, status_out, dtype);
         if (s2 != VBX_OK) return s2;

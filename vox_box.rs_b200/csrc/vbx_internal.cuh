@@ -65,6 +65,9 @@ struct vbx_ctx {
     int64_t hard_cap = 0;              // entries of hard_list (vbx_hard_list_reserve: as many as a roots launch has frames)
     vbx_mfcc_cache* mfcc_cache = nullptr;
     bool mfcc_fft_f32 = false;  // MFCC transform precision (default fp64)
+    // planar copy of an interleaved view (vbx_planarize): grow-only, written and read on the context's stream only
+    void* planar = nullptr;
+    size_t planar_bytes = 0;
 };
 
 enum { VBX_WORK_ROOTS_HORNER = 0, VBX_WORK_ROOTS_ROUNDS = 1, VBX_WORK_REFINE_TERMS = 2, VBX_WORK_REFINE_EVALS = 3, VBX_N_WORK_COUNTERS = 8 };
@@ -90,7 +93,6 @@ int vbx_pipe_reserve(vbx_ctx* ctx, size_t bytes);          // ensures ctx->pipe 
 // vbx_peaks.cu: per-frame (local_out [F]) and per-segment (global_out [n_segments]) max |x| of a device view, either may be
 // null; and the same max over the whole extent of a host view (the global peak of a single-segment view)
 int vbx_launch_frame_peaks(vbx_ctx* ctx, const vbx_frames* fr, double* local_out, double* global_out);
-double vbx_host_peak(const vbx_frames* fr);
 // sample dtypes whose samples load as integer PCM values (int16, or G.711 decoded to int16): their 1/32767 scale lives in the
 // window table
 static inline bool vbx_dtype_is_pcm(int dt) { return dt == VBX_I16 || dt == VBX_MULAW8 || dt == VBX_ALAW8; }
@@ -131,11 +133,27 @@ int vbx_check_frames(vbx_ctx* ctx, const vbx_frames* fr, bool allow_f64 = false)
 static inline int64_t vbx_frames_per_segment(const vbx_frames* fr) {
     return fr->frames_per_segment > 0 ? fr->frames_per_segment : fr->n_frames;
 }
+// samples between consecutive samples of a frame (vbx_frames.sample_step: 0 and 1 are contiguous)
+static inline int64_t vbx_sample_step(const vbx_frames* fr) { return fr->sample_step > 1 ? fr->sample_step : 1; }
 static inline int64_t vbx_frames_extent(const vbx_frames* fr) {
     if (fr->n_frames <= 0) return 0;
     const int64_t J = vbx_frames_per_segment(fr), segs = fr->n_frames / J;
-    return (segs - 1) * (fr->frames_per_segment > 0 ? fr->segment_stride : 0) + (J - 1) * fr->frame_stride + fr->frame_len;
+    return (segs - 1) * (fr->frames_per_segment > 0 ? fr->segment_stride : 0) + (J - 1) * fr->frame_stride +
+           ((int64_t)fr->frame_len - 1) * vbx_sample_step(fr) + 1;
 }
+// Interleaved views (sample_step > 1, vbx_interleave.cu).  The planar equivalent of the header: segment u's channel samples
+// P[u][k] = base[u*segment_stride + k*s], k < vbx_planar_len, in rows of vbx_planar_row samples.
+static inline int64_t vbx_planar_len(const vbx_frames* fr) {
+    return ((vbx_frames_per_segment(fr) - 1) * fr->frame_stride) / vbx_sample_step(fr) + fr->frame_len;
+}
+static inline int64_t vbx_planar_row(const vbx_frames* fr) { return (vbx_planar_len(fr) + 63) & ~(int64_t)63; }
+// *out = the planar equivalent of *fr: for an interleaved view, gathered on the context's stream into ctx->planar (a grow-only
+// buffer of its own, never the scratch arena or a caller's sub-range of it); any other view is copied unchanged.  Every
+// frame-view entry point that launches kernels calls this once after its argument checks.  lead > 0 (the host pipeline) puts
+// `lead` zero samples before every row, so that the view starts at planar offset lead (rows: lead + S rounded up to 64).
+int vbx_planarize(vbx_ctx* ctx, const vbx_frames* fr, vbx_frames* out, int64_t lead = 0);
+// max |x| over segment u's channel samples (a host view; the global peak vbx_frame_peaks defines), dtype scaling included
+double vbx_host_peak(const vbx_frames* fr, int64_t u);
 
 // ------------------------------------------------------------------------------------------
 // device helpers

@@ -740,6 +740,10 @@ int lpc_dispatch(vbx_ctx* ctx, const vbx_frames* fr, int n_lags, void* r_out, vo
     int st = lpc_check(ctx, fr, n_lags, r_out, out_dtype, do_levinson);
     if (st != VBX_OK || fr->n_frames == 0) return st;
     cudaSetDevice(ctx->device);
+    vbx_frames pv;  // the planar equivalent of an interleaved view
+    st = vbx_planarize(ctx, fr, &pv);
+    if (st != VBX_OK) return st;
+    fr = &pv;
     if (fr->dtype == VBX_I16)
         return launch_lpc<int16_t>(ctx, fr, n_lags, r_out, ac_out, kc_out, out_dtype, do_levinson);
     if (fr->dtype == VBX_MULAW8)

@@ -558,6 +558,10 @@ int vbx_mfcc(vbx_ctx* ctx, const vbx_frames* frames, int32_t num_coeffs, int32_t
     if (st != VBX_OK) return st;
     if (frames->n_frames == 0) return VBX_OK;
     cudaSetDevice(ctx->device);
+    vbx_frames pv;  // the planar equivalent of an interleaved view
+    st = vbx_planarize(ctx, frames, &pv);
+    if (st != VBX_OK) return st;
+    frames = &pv;
     if (frames->dtype == VBX_I16)
         return launch_mfcc<int16_t>(ctx, frames, num_coeffs, n_keep, freq_lo, freq_hi, sample_rate, out, energies_out, out_dtype);
     if (frames->dtype == VBX_MULAW8)

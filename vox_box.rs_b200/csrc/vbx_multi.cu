@@ -278,7 +278,7 @@ int vbx_multi_pitch_with_peaks_host(vbx_multi* m, const vbx_frames* frames, doub
     const double* global = global_peaks;
     if (silence_threshold > 0.0 && !global && !segmented && frames->n_frames > 0 && frames->base && frames->frame_len >= 1 &&
         frames->frame_stride >= 1 && (frames->dtype == VBX_F32 || vbx_dtype_is_pcm(frames->dtype) || frames->dtype == VBX_F64)) {
-        whole = vbx_host_peak(frames);
+        whole = vbx_host_peak(frames, 0);
         global = &whole;
     }
     return run_all(m, [=](int i, vbx_ctx* ctx) -> int {

@@ -104,12 +104,16 @@ int vbx_launch_frame_peaks(vbx_ctx* ctx, const vbx_frames* fr, double* local_out
     return VBX_OK;
 }
 
-double vbx_host_peak(const vbx_frames* fr) {
-    const int64_t extent = vbx_frames_extent(fr);
+// segment u's samples as the planar equivalent holds them (all of a contiguous single-segment view's extent):
+// base[u*segment_stride + k*s], k < vbx_planar_len
+double vbx_host_peak(const vbx_frames* fr, int64_t u) {
+    const int64_t n = vbx_planar_len(fr), s = vbx_sample_step(fr);
+    const int64_t first = fr->frames_per_segment > 0 ? u * fr->segment_stride : 0;
     double m = 0.0;
     if (vbx_dtype_is_pcm(fr->dtype)) {
         int a = 0;
-        for (int64_t i = 0; i < extent; ++i) {
+        for (int64_t k = 0; k < n; ++k) {
+            const int64_t i = first + k * s;
             int v;
             if (fr->dtype == VBX_I16) v = ((const int16_t*)fr->base)[i];
             else if (fr->dtype == VBX_MULAW8) v = vbx_mulaw_decode(((const uint8_t*)fr->base)[i]);
@@ -120,15 +124,15 @@ double vbx_host_peak(const vbx_frames* fr) {
         m = (double)a / 32767.0;
     } else if (fr->dtype == VBX_F64) {
         const double* x = (const double*)fr->base;
-        for (int64_t i = 0; i < extent; ++i) {
-            const double a = fabs(x[i]);
+        for (int64_t k = 0; k < n; ++k) {
+            const double a = fabs(x[first + k * s]);
             if (a > m) m = a;
         }
     } else {
         const float* x = (const float*)fr->base;
         float mf = 0.f;
-        for (int64_t i = 0; i < extent; ++i) {
-            const float a = fabsf(x[i]);
+        for (int64_t k = 0; k < n; ++k) {
+            const float a = fabsf(x[first + k * s]);
             if (a > mf) mf = a;
         }
         m = (double)mf;
@@ -144,7 +148,10 @@ int vbx_frame_peaks(vbx_ctx* ctx, const vbx_frames* frames, double* local_out, d
     if (st != VBX_OK) return st;
     if (frames->n_frames == 0) return VBX_OK;
     cudaSetDevice(ctx->device);
-    return vbx_launch_frame_peaks(ctx, frames, local_out, global_out);
+    vbx_frames pv;  // the planar equivalent of an interleaved view
+    st = vbx_planarize(ctx, frames, &pv);
+    if (st != VBX_OK) return st;
+    return vbx_launch_frame_peaks(ctx, &pv, local_out, global_out);
 }
 
 }  // extern "C"

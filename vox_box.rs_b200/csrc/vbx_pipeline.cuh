@@ -7,8 +7,25 @@
 // dedicated block of the context (the kernels keep using the scratch arena, serialised on the compute
 // stream).  Pinned host memory is what makes the copies asynchronous; with pageable memory the result is
 // the same, only the overlap is lost.
+//
+// An interleaved view whose segments share memory (the channels of one recording: segment_stride below a segment's extent)
+// is cut by TIME instead: chunk k is frames [j0, j1) of every segment.  It uploads the interleaved span those frames cover,
+// once for all channels, the device call gathers the channels (vbx_planarize) and runs on the sub-view of J' = j1 − j0
+// frames per segment, and each output comes back with one cudaMemcpy2DAsync to rows u*J + j0 .. of every segment u.
+// Consecutive chunks share only the frame overlap of their boundary, (frame_len − hop) samples of every channel, exactly as
+// the frame chunks of a single-segment view do; every other interleaved byte crosses PCIe once.  The pipeline gathers each
+// interleaved chunk itself, placing the chunk's first frame at the offset (mod 64 samples) it has in the planar equivalent of
+// the whole view, so that every frame is read at the alignment the device call reads it at and the results are the device
+// call's bit for bit.
 #pragma once
 #include "vbx_internal.cuh"
+
+// the host pipeline cuts this view into time ranges of every segment (see above)
+static inline bool vbx_chunk_by_time(const vbx_frames* fr) {
+    if (fr->frames_per_segment <= 0 || vbx_sample_step(fr) <= 1) return false;
+    const int64_t seg_extent = (fr->frames_per_segment - 1) * fr->frame_stride + ((int64_t)fr->frame_len - 1) * vbx_sample_step(fr) + 1;
+    return fr->segment_stride < seg_extent;
+}
 
 struct vbx_host_out {
     void* host;              // destination (host), may be null = output not requested
@@ -16,19 +33,24 @@ struct vbx_host_out {
     void* dev;               // filled per chunk: device address of this chunk's block
 };
 
-// launch(chunk_frames_view_on_device, first_frame, first_segment, outs_with_dev_set) -> status
+// launch(chunk_frames_view_on_device, first_frame, first_segment, outs_with_dev_set) -> status.  When the view is cut by
+// time (vbx_chunk_by_time), first_frame is the chunk's first frame j0 inside every segment and first_segment is 0.
 template <class Launch>
 static int vbx_run_chunked(vbx_ctx* ctx, const vbx_frames* fr, vbx_host_out* outs, int n_outs, Launch launch,
                            int max_chunks = 0 /* 0 = no limit; paths with a latency-bound per-chunk kernel ask for few, large chunks */,
                            size_t target_bytes = (size_t)24 << 20 /* input bytes per chunk; compute-bound paths ask for more */) {
     const int64_t F = fr->n_frames;
     const size_t es = vbx_dtype_size(fr->dtype);
-    const bool segmented = fr->frames_per_segment > 0;
-    const int64_t J = vbx_frames_per_segment(fr);
-    const int64_t n_units = segmented ? F / J : F;           // chunkable units: segments or frames
-    const int64_t unit_frames = segmented ? J : 1;
+    const bool by_time = vbx_chunk_by_time(fr);
+    const bool segmented = fr->frames_per_segment > 0 && !by_time;
+    const int64_t J = vbx_frames_per_segment(fr), U = F / J;
+    const int64_t frame_extent = ((int64_t)fr->frame_len - 1) * vbx_sample_step(fr) + 1;  // samples one frame spans
+    // chunkable units: segments, frames, or (by time) the frame index j of every segment at once
+    const int64_t n_units = segmented ? U : (by_time ? J : F);
+    const int64_t unit_frames = segmented ? J : (by_time ? U : 1);
     const int64_t unit_stride = segmented ? fr->segment_stride : fr->frame_stride;  // samples between unit starts
-    const int64_t unit_extent = segmented ? (J - 1) * fr->frame_stride + fr->frame_len : fr->frame_len;
+    const int64_t unit_extent = segmented ? (J - 1) * fr->frame_stride + frame_extent
+                                          : (by_time ? (U - 1) * fr->segment_stride + frame_extent : frame_extent);
     size_t out_per_frame = 0;
     for (int i = 0; i < n_outs; ++i) out_per_frame += outs[i].host ? outs[i].bytes_per_frame : 0;
     // chunk size: `target_bytes` of input per chunk (24 MB unless the caller says otherwise; VBX_HOST_CHUNK_MB overrides)
@@ -83,9 +105,16 @@ static int vbx_run_chunked(vbx_ctx* ctx, const vbx_frames* fr, vbx_host_out* out
         // compute: needs its input, and its output buffer b free (D2H of chunk c−2 done)
         PIPE_CUDA(cudaStreamWaitEvent(ctx->stream, ev_in[b], 0));
         if (c >= 2) PIPE_CUDA(cudaStreamWaitEvent(ctx->stream, ev_out[b], 0));
-        vbx_frames dfr = *fr;
-        dfr.base = d_in;
-        dfr.n_frames = nf;
+        vbx_frames ifr = *fr;
+        ifr.base = d_in;
+        ifr.n_frames = nf;
+        if (by_time) ifr.frames_per_segment = nu;
+        // an interleaved chunk is gathered here, with its first frame at the offset (mod 64 samples) it has in the planar
+        // equivalent of the whole view: the kernels then see every frame at the alignment the device call gives it
+        vbx_frames dfr;
+        const int64_t first_frame = segmented ? 0 : u0;  // index of the chunk's first frame inside its segment(s)
+        rc = vbx_planarize(ctx, &ifr, &dfr, (first_frame * (fr->frame_stride / vbx_sample_step(fr))) % 64);
+        if (rc != VBX_OK) break;
         size_t off = 0;
         for (int i = 0; i < n_outs; ++i) {
             outs[i].dev = nullptr;
@@ -94,14 +123,19 @@ static int vbx_run_chunked(vbx_ctx* ctx, const vbx_frames* fr, vbx_host_out* out
                 off += al((size_t)units_per_chunk * unit_frames * outs[i].bytes_per_frame);
             }
         }
-        rc = launch(&dfr, u0 * unit_frames, segmented ? u0 : 0, outs);
+        rc = launch(&dfr, by_time ? u0 : u0 * unit_frames, segmented ? u0 : 0, outs);
         if (rc != VBX_OK) break;
         PIPE_CUDA(cudaEventRecord(ev_comp[b], ctx->stream));
         PIPE_CUDA(cudaStreamWaitEvent(ctx->s_d2h, ev_comp[b], 0));
         for (int i = 0; i < n_outs && rc == VBX_OK; ++i) {
             if (!outs[i].host) continue;
-            const cudaError_t ec = cudaMemcpyAsync((char*)outs[i].host + (size_t)u0 * unit_frames * outs[i].bytes_per_frame, outs[i].dev,
-                                                   (size_t)nf * outs[i].bytes_per_frame, cudaMemcpyDeviceToHost, ctx->s_d2h);
+            const size_t bpf = outs[i].bytes_per_frame;
+            // by time: the chunk's [U][nu] rows go to rows u*J + u0 of the caller's [U][J]
+            const cudaError_t ec =
+                by_time ? cudaMemcpy2DAsync((char*)outs[i].host + (size_t)u0 * bpf, (size_t)J * bpf, outs[i].dev, (size_t)nu * bpf,
+                                            (size_t)nu * bpf, (size_t)U, cudaMemcpyDeviceToHost, ctx->s_d2h)
+                        : cudaMemcpyAsync((char*)outs[i].host + (size_t)u0 * unit_frames * bpf, outs[i].dev, (size_t)nf * bpf,
+                                          cudaMemcpyDeviceToHost, ctx->s_d2h);
             if (ec != cudaSuccess) rc = vbx_fail(ctx, VBX_ERR_CUDA, "host pipeline: D2H copy failed: %s", cudaGetErrorString(ec));
         }
         if (rc != VBX_OK) break;

@@ -846,6 +846,10 @@ int pitch_check(vbx_ctx* ctx, const vbx_frames* fr, int max_cand, const void* ca
 int launch_pitch_any(vbx_ctx* ctx, const vbx_frames* fr, double fs, double threshold, double fmin, double fmax, int max_cand,
                      void* cand_out, int32_t* n_cand_out, uint8_t* status_out, int out_dtype, double* lag_out, const PitchPeaks& peaks) {
     cudaSetDevice(ctx->device);
+    vbx_frames pv;  // the planar equivalent of an interleaved view
+    const int st = vbx_planarize(ctx, fr, &pv);
+    if (st != VBX_OK) return st;
+    fr = &pv;
     if (fr->dtype == VBX_MULAW8)
         return launch_pitch<vbx_mulaw8>(ctx, fr, fs, threshold, fmin, fmax, max_cand, cand_out, n_cand_out, status_out, out_dtype,
                                         lag_out, peaks);
@@ -893,8 +897,9 @@ int vbx_pitch_with_peaks(vbx_ctx* ctx, const vbx_frames* frames, double sample_r
 }
 
 // The host pipeline cuts a segmented view into whole segments, so every chunk computes its segments' global peaks itself.  It
-// cuts a single-segment view into frame ranges, so there the global peak of the whole view is taken here, on the host, before
-// the pipeline starts.  Caller-supplied peaks are uploaded once and every chunk reads its rows.
+// cuts a single-segment view into frame ranges, and the channels of an interleaved recording into time ranges, so there the
+// global peak of every segment is taken here, on the host, over its whole channel before the pipeline starts.  Caller-supplied
+// peaks are uploaded once and every chunk reads its rows (a time chunk gathers its [U][J'] block of local peaks first).
 int vbx_pitch_with_peaks_host(vbx_ctx* ctx, const vbx_frames* frames, double sample_rate, double threshold, double silence_threshold,
                               const double* local_peaks, const double* global_peaks, double min_hz, double max_hz,
                               int32_t max_candidates, void* cand_out, int32_t* n_cand_out, uint8_t* status_out, int32_t out_dtype) {
@@ -906,18 +911,20 @@ int vbx_pitch_with_peaks_host(vbx_ctx* ctx, const vbx_frames* frames, double sam
     cudaSetDevice(ctx->device);
     const bool with_peaks = silence_threshold > 0.0;
     const bool segmented = frames->frames_per_segment > 0;
-    const int64_t F = frames->n_frames, n_segs = F / vbx_frames_per_segment(frames);
-    double whole = 0.0;
+    const bool by_time = vbx_chunk_by_time(frames);
+    const int64_t F = frames->n_frames, J = vbx_frames_per_segment(frames), n_segs = F / J;
+    std::vector<double> whole;
     const double* global_src = with_peaks ? global_peaks : nullptr;
-    if (with_peaks && !global_peaks && !segmented) {
-        whole = vbx_host_peak(frames);
-        global_src = &whole;
+    if (with_peaks && !global_peaks && (!segmented || by_time)) {
+        for (int64_t u = 0; u < n_segs; ++u) whole.push_back(vbx_host_peak(frames, u));
+        global_src = whole.data();
     }
     const double* local_src = with_peaks ? local_peaks : nullptr;
     const size_t n_local = local_src ? (size_t)F : 0, n_global = global_src ? (size_t)n_segs : 0;
+    const size_t n_chunk_local = by_time ? n_local : 0;  // a time chunk's local peaks, gathered from the [U][J] rows
     double* dev = nullptr;
     if (n_local + n_global > 0) {
-        VBX_CUDA(ctx, cudaMalloc(&dev, (n_local + n_global) * sizeof(double)));
+        VBX_CUDA(ctx, cudaMalloc(&dev, (n_local + n_global + n_chunk_local) * sizeof(double)));
         cudaError_t e = cudaSuccess;
         if (n_local) e = cudaMemcpyAsync(dev, local_src, n_local * sizeof(double), cudaMemcpyHostToDevice, ctx->stream);
         if (e == cudaSuccess && n_global)
@@ -934,7 +941,15 @@ int vbx_pitch_with_peaks_host(vbx_ctx* ctx, const vbx_frames* frames, double sam
     vbx_host_out outs[3] = {{cand_out, (size_t)max_candidates * pair, nullptr}, {n_cand_out, 4, nullptr}, {status_out, 1, nullptr}};
     // chunked H2D / kernels / D2H pipeline (vbx_pipeline.cuh); output rows are indexed from the chunk's first frame
     const int rc = vbx_run_chunked(ctx, frames, outs, 3, [&](const vbx_frames* dfr, int64_t f0, int64_t u0, vbx_host_out* o) -> int {
-        return vbx_pitch_with_peaks(ctx, dfr, sample_rate, threshold, silence_threshold, d_local ? d_local + f0 : nullptr,
+        const double* chunk_local = d_local ? d_local + f0 : nullptr;
+        if (d_local && by_time) {  // rows u*J + f0 .. of every segment u -> [U][J'] (the compute stream runs chunks in order)
+            double* dst = dev + n_local + n_global;
+            const int64_t jc = dfr->frames_per_segment;
+            VBX_CUDA(ctx, cudaMemcpy2DAsync(dst, (size_t)jc * sizeof(double), d_local + f0, (size_t)J * sizeof(double),
+                                            (size_t)jc * sizeof(double), (size_t)n_segs, cudaMemcpyDeviceToDevice, ctx->stream));
+            chunk_local = dst;
+        }
+        return vbx_pitch_with_peaks(ctx, dfr, sample_rate, threshold, silence_threshold, chunk_local,
                                     d_global ? d_global + u0 : nullptr, min_hz, max_hz, max_candidates, o[0].dev, (int32_t*)o[1].dev,
                                     (uint8_t*)o[2].dev, out_dtype);
     }, 0, (size_t)96 << 20);  // compute-bound: the copies hide behind the kernels anyway, larger chunks mean fewer kernel tails

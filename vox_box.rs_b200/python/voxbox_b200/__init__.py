@@ -34,9 +34,27 @@ class VoxBoxError(RuntimeError):
 
 
 class Frames(C.Structure):
-    """struct vbx_frames"""
+    """struct vbx_frames.  sample_step (0 / 1 contiguous, C for C interleaved channels) shares its int32 with the field's
+    former name `reserved`, which stays as an alias."""
     _fields_ = [("base", C.c_void_p), ("n_frames", C.c_int64), ("frame_stride", C.c_int64),
-                ("frames_per_segment", C.c_int64), ("segment_stride", C.c_int64), ("frame_len", C.c_int32), ("dtype", C.c_int32), ("window", C.c_int32), ("reserved", C.c_int32)]
+                ("frames_per_segment", C.c_int64), ("segment_stride", C.c_int64), ("frame_len", C.c_int32), ("dtype", C.c_int32), ("window", C.c_int32), ("sample_step", C.c_int32)]
+
+    reserved = property(lambda self: self.sample_step, lambda self, v: setattr(self, "sample_step", v))
+
+
+def channel_view(n_frames, stride, frames_per_segment=0, segment_stride=0, channels=1):
+    """(n_frames, frame_stride, frames_per_segment, segment_stride, sample_step) of the view a `_host` helper builds.
+    channels=1: the arguments as given.  channels=C > 1: the buffer holds C interleaved channels (the WAV layout, n_samples*C
+    samples), n_frames and stride count the frames and the hop of ONE channel, and the view has one segment per channel
+    (segment u = channel u, sample_step C), so the helper returns C*n_frames rows, channel-major."""
+    channels = int(channels)
+    if channels < 1:
+        raise ValueError(f"channels must be >= 1, not {channels}")
+    if channels == 1:
+        return n_frames, stride, frames_per_segment, segment_stride, 0
+    if frames_per_segment:
+        raise ValueError("channels > 1 views the buffer as one segment per channel: frames_per_segment must be 0")
+    return channels * n_frames, stride * channels, n_frames, 1, channels
 
 
 _lib = None
@@ -272,9 +290,16 @@ class Context:
 
     @staticmethod
     def frames(base_ptr, n_frames, frame_len, frame_stride, window=WINDOW_NONE, dtype=F32, frames_per_segment=0,
-               segment_stride=0):
-        """vbx_frames: frame f = u*J + j starts at base[u*segment_stride + j*frame_stride] (J = frames_per_segment)."""
-        return Frames(base_ptr, n_frames, frame_stride, frames_per_segment, segment_stride, frame_len, dtype, window, 0)
+               segment_stride=0, sample_step=0):
+        """vbx_frames: sample i of frame f = u*J + j is base[u*segment_stride + j*frame_stride + i*sample_step]
+        (J = frames_per_segment; sample_step 0 or 1 = contiguous frames)."""
+        return Frames(base_ptr, n_frames, frame_stride, frames_per_segment, segment_stride, frame_len, dtype, window, sample_step)
+
+    @staticmethod
+    def _host_view(base_ptr, n_frames, frame_len, stride, window, dtype, frames_per_segment=0, segment_stride=0, channels=1):
+        """The view of a `_host` helper (channel_view) and its number of frames."""
+        F, fst, J, seg, step = channel_view(n_frames, stride, frames_per_segment, segment_stride, channels)
+        return Context.frames(base_ptr, F, frame_len, fst, window, dtype, J, seg, step), F
 
     @staticmethod
     def n_frames_of(n_samples, frame_len, hop):
@@ -310,17 +335,19 @@ class Context:
         return ac, kc
 
     # -- host-pointer twins (H2D + kernels + D2H inside the call) ------------------------------
-    def autocorrelate_host(self, audio, n_frames, frame_len, stride, window, n_lags, out_dtype=F64, sample_dtype=None):
+    def autocorrelate_host(self, audio, n_frames, frame_len, stride, window, n_lags, out_dtype=F64, sample_dtype=None, channels=1):
         audio = np.ascontiguousarray(audio)
-        fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype))
+        fr, n_frames = self._host_view(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype),
+                                       channels=channels)
         r = np.empty((n_frames, n_lags), dtype=_NP[out_dtype])
         self._check(self.lib.vbx_autocorrelate_host(self.h, C.byref(fr), n_lags, r.ctypes.data, out_dtype),
                     "vbx_autocorrelate_host")
         return r
 
-    def lpc_host(self, audio, n_frames, frame_len, stride, window, p, out_dtype=F64, out=None, sample_dtype=None):
+    def lpc_host(self, audio, n_frames, frame_len, stride, window, p, out_dtype=F64, out=None, sample_dtype=None, channels=1):
         audio = np.ascontiguousarray(audio)
-        fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype))
+        fr, n_frames = self._host_view(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype),
+                                       channels=channels)
         if out is None:
             out = (np.empty((n_frames, p + 1), dtype=_NP[out_dtype]), np.empty((n_frames, p + 1), dtype=_NP[out_dtype]),
                    np.empty((n_frames, p), dtype=_NP[out_dtype]))
@@ -440,11 +467,12 @@ def _find_formants(self, frames, fs, p, method, estimates, dtype=F64, want_reson
 
 
 def _find_formants_host(self, audio, n_frames, frame_len, stride, window, fs, p, method, estimates, dtype=F64,
-                        frames_per_segment=0, segment_stride=0, sample_dtype=None):
+                        frames_per_segment=0, segment_stride=0, sample_dtype=None, channels=1):
+    """estimates: [n_segments][k][2] (one row per channel with channels=C)."""
     audio = np.ascontiguousarray(audio)
-    fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype),
-                     frames_per_segment, segment_stride)
-    J = frames_per_segment or n_frames
+    fr, n_frames = self._host_view(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype),
+                                   frames_per_segment, segment_stride, channels)
+    J = fr.frames_per_segment or n_frames
     segs = n_frames // J if J else 0
     est = np.ascontiguousarray(estimates, dtype=_NP[dtype]).reshape(segs, -1, 2).copy()
     k = est.shape[1]
@@ -483,10 +511,10 @@ def _pitch(self, frames, fs, threshold, fmin, fmax, max_cand=16, out_dtype=F64):
 
 
 def _pitch_host(self, audio, n_frames, frame_len, stride, window, fs, threshold, fmin, fmax, max_cand=16, out_dtype=F64,
-                frames_per_segment=0, segment_stride=0, sample_dtype=None):
+                frames_per_segment=0, segment_stride=0, sample_dtype=None, channels=1):
     audio = np.ascontiguousarray(audio)
-    fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype),
-                     frames_per_segment, segment_stride)
+    fr, n_frames = self._host_view(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype),
+                                   frames_per_segment, segment_stride, channels)
     cand = np.zeros((n_frames, max_cand, 2), dtype=_NP[out_dtype])
     n = np.zeros(n_frames, dtype=np.int32)
     st = np.zeros(n_frames, dtype=np.uint8)
@@ -603,13 +631,14 @@ def _pitch_with_peaks(self, frames, fs, threshold, silence_threshold, fmin, fmax
 
 def _pitch_with_peaks_host(self, audio, n_frames, frame_len, stride, window, fs, threshold, silence_threshold, fmin, fmax,
                            max_cand=16, out_dtype=F64, frames_per_segment=0, segment_stride=0, local_peaks=None,
-                           global_peaks=None, sample_dtype=None):
+                           global_peaks=None, sample_dtype=None, channels=1):
     """Host twin of pitch_with_peaks: audio int16 / float32 / float64 samples (or uint8 G.711 codes with sample_dtype), peaks
-    host arrays or None."""
+    host arrays or None (local [F], global [n_segments]: one per channel with channels=C)."""
     audio, dt = _host_audio(audio, sample_dtype)
-    fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, dt, frames_per_segment, segment_stride)
+    fr, n_frames = self._host_view(audio.ctypes.data, n_frames, frame_len, stride, window, dt, frames_per_segment, segment_stride,
+                                   channels)
     lp = _host_peaks(local_peaks, n_frames)
-    gp = _host_peaks(global_peaks, _n_segments(n_frames, frames_per_segment))
+    gp = _host_peaks(global_peaks, _n_segments(n_frames, fr.frames_per_segment))
     cand = np.zeros((n_frames, max_cand, 2), dtype=_NP[out_dtype])
     n = np.zeros(n_frames, dtype=np.int32)
     st = np.zeros(n_frames, dtype=np.uint8)
@@ -652,11 +681,11 @@ def _mfcc(self, frames, num_coeffs, f_lo, f_hi, fs, n_keep=None, out_dtype=F64, 
 
 
 def _mfcc_host(self, audio, n_frames, frame_len, stride, window, num_coeffs, f_lo, f_hi, fs, n_keep=None, out_dtype=F64,
-               frames_per_segment=0, segment_stride=0, sample_dtype=None):
+               frames_per_segment=0, segment_stride=0, sample_dtype=None, channels=1):
     audio = np.ascontiguousarray(audio)
     n_keep = num_coeffs if n_keep is None else n_keep
-    fr = self.frames(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype),
-                     frames_per_segment, segment_stride)
+    fr, n_frames = self._host_view(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype),
+                                   frames_per_segment, segment_stride, channels)
     out = np.zeros((n_frames, n_keep), dtype=_NP[out_dtype])
     self._check(self.lib.vbx_mfcc_host(self.h, C.byref(fr), num_coeffs, n_keep, f_lo, f_hi, fs, out.ctypes.data, out_dtype),
                 "vbx_mfcc_host")
@@ -844,14 +873,18 @@ class Multi:
         return list(out)
 
     @staticmethod
-    def _view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride, sample_dtype=None):
+    def _view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride, sample_dtype=None, channels=1):
+        """(audio, view, number of frames) of a `_host` call (channel_view); an interleaved recording shards by channel, so
+        at most `channels` devices get work."""
         audio = np.ascontiguousarray(audio)
-        return audio, Context.frames(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype),
-                                     frames_per_segment, segment_stride)
+        fr, F = Context._host_view(audio.ctypes.data, n_frames, frame_len, stride, window, _sample_dtype(audio, sample_dtype),
+                                   frames_per_segment, segment_stride, channels)
+        return audio, fr, F
 
     def lpc_host(self, audio, n_frames, frame_len, stride, window, p, out_dtype=F64, frames_per_segment=0, segment_stride=0,
-                 sample_dtype=None):
-        audio, fr = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride, sample_dtype)
+                 sample_dtype=None, channels=1):
+        audio, fr, n_frames = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride,
+                                         sample_dtype, channels)
         r = np.zeros((n_frames, p + 1), dtype=_NP[out_dtype])
         ac = np.zeros((n_frames, p + 1), dtype=_NP[out_dtype])
         kc = np.zeros((n_frames, p), dtype=_NP[out_dtype])
@@ -860,9 +893,10 @@ class Multi:
         return r, ac, kc
 
     def find_formants_host(self, audio, n_frames, frame_len, stride, window, fs, p, method, estimates, dtype=F64,
-                           frames_per_segment=0, segment_stride=0, sample_dtype=None):
-        audio, fr = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride, sample_dtype)
-        J = frames_per_segment or n_frames
+                           frames_per_segment=0, segment_stride=0, sample_dtype=None, channels=1):
+        audio, fr, n_frames = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride,
+                                         sample_dtype, channels)
+        J = fr.frames_per_segment or n_frames
         segs = n_frames // J if J else 0
         est = np.ascontiguousarray(estimates, dtype=_NP[dtype]).reshape(segs, -1, 2).copy()
         k = est.shape[1]
@@ -876,8 +910,9 @@ class Multi:
         return dict(tracks=tracks, estimates=est, resonances=res, n_res=nres, status=st)
 
     def pitch_host(self, audio, n_frames, frame_len, stride, window, fs, threshold, fmin, fmax, max_cand=16, out_dtype=F64,
-                   frames_per_segment=0, segment_stride=0, sample_dtype=None):
-        audio, fr = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride, sample_dtype)
+                   frames_per_segment=0, segment_stride=0, sample_dtype=None, channels=1):
+        audio, fr, n_frames = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride,
+                                         sample_dtype, channels)
         cand = np.zeros((n_frames, max_cand, 2), dtype=_NP[out_dtype])
         n = np.zeros(n_frames, dtype=np.int32)
         st = np.zeros(n_frames, dtype=np.uint8)
@@ -887,12 +922,13 @@ class Multi:
 
     def pitch_with_peaks_host(self, audio, n_frames, frame_len, stride, window, fs, threshold, silence_threshold, fmin, fmax,
                               max_cand=16, out_dtype=F64, frames_per_segment=0, segment_stride=0, local_peaks=None,
-                              global_peaks=None, sample_dtype=None):
+                              global_peaks=None, sample_dtype=None, channels=1):
         """Context.pitch_with_peaks_host sharded over the devices (vbx_multi_pitch_with_peaks_host)."""
         audio, dt = _host_audio(audio, sample_dtype)
-        fr = Context.frames(audio.ctypes.data, n_frames, frame_len, stride, window, dt, frames_per_segment, segment_stride)
+        fr, n_frames = Context._host_view(audio.ctypes.data, n_frames, frame_len, stride, window, dt, frames_per_segment,
+                                          segment_stride, channels)
         lp = _host_peaks(local_peaks, n_frames)
-        gp = _host_peaks(global_peaks, _n_segments(n_frames, frames_per_segment))
+        gp = _host_peaks(global_peaks, _n_segments(n_frames, fr.frames_per_segment))
         cand = np.zeros((n_frames, max_cand, 2), dtype=_NP[out_dtype])
         n = np.zeros(n_frames, dtype=np.int32)
         st = np.zeros(n_frames, dtype=np.uint8)
@@ -904,8 +940,9 @@ class Multi:
         return dict(candidates=cand, n_cand=n, status=st)
 
     def mfcc_host(self, audio, n_frames, frame_len, stride, window, num_coeffs, f_lo, f_hi, fs, n_keep=None, out_dtype=F64,
-                  frames_per_segment=0, segment_stride=0, sample_dtype=None):
-        audio, fr = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride, sample_dtype)
+                  frames_per_segment=0, segment_stride=0, sample_dtype=None, channels=1):
+        audio, fr, n_frames = self._view(audio, n_frames, frame_len, stride, window, frames_per_segment, segment_stride,
+                                         sample_dtype, channels)
         n_keep = num_coeffs if n_keep is None else n_keep
         out = np.zeros((n_frames, n_keep), dtype=_NP[out_dtype])
         self._check(self.lib.vbx_multi_mfcc_host(self.h, C.byref(fr), num_coeffs, n_keep, f_lo, f_hi, fs, out.ctypes.data, out_dtype),
